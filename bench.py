@@ -36,6 +36,24 @@ GF_PER_IMG = {"vae_encoder": 1116.66, "unet_taps": 803.18, "projections": 14.35,
 # --variant s0 (not the default bench line): the vae_decoder_loss configuration of the shipped experiment files (SURVEY §8 a-11):
 # + UNet conv_out, VAE decoder 2514.5, Bottleneck(3->128->128) at 512^2 instead of the s2 projection; SURVEY §8d total 4526.0
 GF_PER_IMG_S0 = {"vae_encoder": 1116.66, "unet": 803.27, "vae_decoder": 2514.5, "projections": 91.6, "total": 4526.0}
+DUMP_BYTES = 60_000_000  # --dump-outputs: data budget of all files together, leaves room for the .npy headers under 64 MB
+
+
+def dump_outputs(out_dir, named):
+    """--dump-outputs: writes each output as out_dir/<name>.npy in float32.  An output larger than its equal share of DUMP_BYTES is
+    written as out_dir/<name>_sample.npy instead: its flattened values at the sorted, de-duplicated flat indices
+    torch.randint(numel, (share,), generator=torch.Generator().manual_seed(0)).unique() -- the same indices in every run, so that two
+    builds can be compared output for output."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // 4 // len(named)
+    for name, t in named.items():
+        t = t.detach().float()
+        if t.numel() > share:
+            idx = torch.randint(t.numel(), (share,), generator=torch.Generator().manual_seed(0)).unique()
+            t, name = t.reshape(-1)[idx.to(t.device)], name + "_sample"
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def read_peaks():
@@ -121,7 +139,7 @@ def run_reference(args, rank, world):
     imported here: diffusers/peft/detectron2 absent).  Rank 0 alone runs it."""
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     base, dt = cpu_oracle_throughput(timed=steps, warm=1, variant=args.variant)
     line = {
         "impl": "reference", "metric": METRIC, "value": base["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
@@ -169,9 +187,10 @@ def run_product(args, rank, local_rank, world):
     # B <= engine.graph_max_batch (8): the backbone replays the step's ~555 launches as one CUDA graph (static input buffer,
     # results cloned out of the static output buffers); larger batches launch on the stream into `outs_dev`.
     graphed = 0 < B <= ldm.engine().graph_max_batch
+    last = {}  # the feature maps of the latest step_resident call (--dump-outputs)
 
     def step_resident():
-        return bb._extract(img_dev, "others", False, None, out=None if graphed else outs_dev)
+        last["features"] = bb._extract(img_dev, "others", False, None, out=None if graphed else outs_dev)["features"]
 
     def step_e2e():
         x = img_host.to(dev, non_blocking=True)               # H2D of this step's inputs from pinned memory
@@ -231,6 +250,8 @@ def run_product(args, rank, local_rank, world):
         for _ in range(max(3, args.warmup)):
             step_resident()
         ms, clocks = timed(step_resident, args.steps, ClockSampler(local_rank) if rank == 0 else None)
+        if args.dump_outputs and rank == 0:  # before the runs below reuse the output buffers
+            dump_outputs(args.dump_outputs, dict(zip(bb._out_features, last["features"])))
         for _ in range(2):
             step_e2e()
         ms_e2e_serial, _ = timed(step_e2e, args.steps)
@@ -506,10 +527,17 @@ def run_slide(args, rank, local_rank, world):
         barrier()
         return ms.item(), clocks
 
+    last = []  # what the latest timed step returned (--dump-outputs)
+
+    def step_resident():
+        last[:] = step(img_dev)
+
     with torch.no_grad():
         for _ in range(max(3, args.warmup)):
             step(img_dev)
-        ms, clocks = timed(lambda: step(img_dev), args.steps, ClockSampler(local_rank) if rank == 0 else None)
+        ms, clocks = timed(step_resident, args.steps, ClockSampler(local_rank) if rank == 0 else None)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dict(zip(["label", "weight"] if teacher else bb._out_features, last)))
         for _ in range(2):
             step_e2e()
         ms_e2e, _ = timed(step_e2e, args.steps)
@@ -665,12 +693,14 @@ def run_train(args, rank, local_rank, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step(src_dev, tgt_dev, lab_dev, timed=True)
+        loss = step(src_dev, tgt_dev, lab_dev, timed=True)
     e1.record()
     torch.cuda.synchronize()
     if prof:
         torch.cuda.cudart().cudaProfilerStop()
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:  # the step's loss and the trainable parameters it updated
+        dump_outputs(args.dump_outputs, {"loss": loss, **{n: p for n, p in bb.named_parameters() if p.requires_grad}})
     for k in ev:  # (events of the LAST step: a per-phase picture, not the timed total)
         acc_ms[k] = ev[k][0].elapsed_time(ev[k][1])
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -749,7 +779,14 @@ def main():
     ap.add_argument("--images", type=int, default=8, help="full-resolution images per GPU per step (slide1024 / teacher2048)")
     ap.add_argument("--variant", default="base", choices=["base", "s0"],
                     help="base = BASELINE configs[1] (the bench line); s0 = vae_decoder_loss configuration of the shipped experiment files")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy in float32, "
+                         "under 64 MB in all: outputs larger than their share are written as a fixed, seeded sample, DIR/<name>_sample.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the product arm (--impl madm_b200)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

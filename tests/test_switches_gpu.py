@@ -30,7 +30,7 @@ def _run(tmp_path, variant, env_kv, tag):
 
 
 @pytest.fixture(scope="module")
-def defaults(tmp_path_factory):
+def defaults(tmp_path_factory, cuda_device):
     d = tmp_path_factory.mktemp("switch_default")
     return {v: _run(d, v, None, "default_" + v) for v in ("base", "s0")}
 

@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, '/root/repo')
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from madm_b200 import ops
 dev = torch.device('cuda:0')
 def timed(fn, n=10):
