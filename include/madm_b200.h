@@ -120,7 +120,8 @@ size_t madm_workspace_bytes(madm_ctx* ctx, int32_t B);
 size_t madm_workspace_bytes_head(madm_ctx* ctx, int32_t B, int32_t head_h, int32_t head_w);
 
 #define MADM_FLAG_IMG_NORMALISED 1
-/* out[0..3] are fp16 [B,C,H,W] tensors instead of fp32 (base variant, MADM_STAGE_PROJ): an opt-in for host-bound consumers -- the
+/* out[0..3] are fp16 [B,C,H,W] tensors instead of fp32 (base variant, MADM_STAGE_PROJ; not with MADM_FLAG_TRAIN, whose madm_backward
+ * reads the fp32 maps): an opt-in for host-bound consumers -- the
  * reference returns fp32 maps (GroupNorm runs in fp32 under autocast), so fp32 stays the default.  Halves the 357 MB per 8 images that
  * a caller who downloads the feature dict moves over PCIe. */
 #define MADM_FLAG_OUT_FP16 4

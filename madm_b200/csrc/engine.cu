@@ -185,7 +185,6 @@ struct Builder {
   int cur_branch = 0;            // branch tag of the ops being emitted (build_proj)
   bool defer_free = false;       // concurrent branches must not recycle each other's buffers: frees are collected and released at the join
   std::vector<std::pair<size_t, size_t>> deferred;
-  int n_ops = 0;
   int head_h = 0, head_w = 0;  // grid of the head's first feature map (0 = the 512 x 512 crop's: 128 x 128, s0 variant 512 x 512)
   // ---- training plans (SURVEY §8 row f-3): the forward keeps what the backward needs; every builder function records its backward on
   // the tape, which build_all() replays in reverse into plan->bops
@@ -195,9 +194,9 @@ struct Builder {
   float loss_scale = 1.0f;
   std::string adapter;         // active LoRA adapter of this training plan ("" = none)
   float lora_scale = 0.f;
-  int n_bops = 0;
   std::vector<std::function<void()>> tape;
-  bool keep() const { return train && !bwd && cur_stage != MADM_STAGE_VAE; }  // forward tensors of the differentiated stages stay allocated
+  // forward of a stage the training plan differentiates (not the VAE): its tensors stay allocated and each block records its backward
+  bool recording() const { return train && !bwd && cur_stage != MADM_STAGE_VAE; }
 
   // ---- workspace allocator (first-fit free list, 1 KB granularity); identical sequence in SIZE and PLAN modes
   struct Blk { size_t off, bytes; };
@@ -260,8 +259,8 @@ struct Builder {
   }
   void release_or_defer(size_t off, size_t bytes) { if (defer_free) deferred.push_back({off, bytes}); else release(off, bytes); }
   void flush_deferred() { for (auto& d : deferred) release(d.first, d.second); deferred.clear(); }
-  void free(F32T& t) { if (keep()) return; if (!is_pinned(t.off, t.bytes)) release_or_defer(t.off, t.bytes); t.bytes = 0; t.p = nullptr; }
-  void free(B16T& t) { if (keep()) return; if (!is_pinned(t.off, t.bytes)) release_or_defer(t.off, t.bytes); t.bytes = 0; t.p = nullptr; }
+  void free(F32T& t) { if (recording()) return; if (!is_pinned(t.off, t.bytes)) release_or_defer(t.off, t.bytes); t.bytes = 0; t.p = nullptr; }
+  void free(B16T& t) { if (recording()) return; if (!is_pinned(t.off, t.bytes)) release_or_defer(t.off, t.bytes); t.bytes = 0; t.p = nullptr; }
   void free(Act& a) { free(a.f); free(a.h); }
   Act act(int B_, int H, int W, int C, bool with_f32, bool with_b16) {
     Act a; a.B = B_; a.H = H; a.W = W; a.C = C;
@@ -445,11 +444,9 @@ struct Builder {
   // ---- op emission
   void emit(Op op, bool optional = false, int kind = MADM_KIND_ELEMENTWISE, double flops = 0.0, double bytes = 0.0, double exec_flops = -1.0) {
     if (bwd) {
-      ++n_bops;
       if (mode == PLAN) plan->bops.push_back(std::move(op));
       return;
     }
-    ++n_ops;
     if (mode == PLAN) {
       plan->ops.push_back(std::move(op));
       plan->stage_of.push_back(cur_stage);
@@ -515,13 +512,11 @@ struct Builder {
           return splitk_reduce(pp, splits, ss, e0.M, e0.N, e0.bias, e0.rowbias, e0.rows_per_img, e0.ld_rowbias, e0.residual, e0.ldr, e0.out_f32,
                                e0.ldo32, e0.out_bf16, e0.ldo16, e0.act, f16, st, e0.res16);
         }, false, MADM_KIND_ELEMENTWISE, 0.0, double(splits + 2) * e0.M * e0.N * 4);
-      } else {
-        (bwd ? n_bops : n_ops) += 2;
       }
       free(part);
       return;
     }
-    if (mode != PLAN) { ++(bwd ? n_bops : n_ops); return; }
+    if (mode != PLAN) return;
     GemmDesc d = d0;
     d.fp16 = ctx->fp16;
     GemmLaunch L;
@@ -548,7 +543,7 @@ struct Builder {
   void attention(const bf16* q, int ldq, const bf16* k, int ldk, const bf16* v, int ldv, bf16* o, int ldo, int Bn, int heads, int d, int Nq,
                  int Nk, long q_bs, long kv_bs, long o_bs, float scale, float* lse = nullptr) {
     const double flops = 4.0 * double(Bn) * Nq * Nk * heads * d;
-    if (mode != PLAN) { ++(bwd ? n_bops : n_ops); return; }
+    if (mode != PLAN) return;
     const int h16 = ctx->fp16;
     FaLaunch L;
     if (const char* e = flash_attention_tc_prepare(q, ldq, k, ldk, v, ldv, o, ldo, Bn, heads, d, Nq, Nk, q_bs, kv_bs, o_bs, scale, h16, &L, lse))
@@ -756,7 +751,7 @@ struct Model {
     if (in16 && (x1 || x0.h_s2d)) b.fail(MADM_EINVAL, "resblock: a 16-bit stream input must be a single linear tensor");
     B16T n1 = b.b16(size_t(x0.M()) * Cin);
     B16T raw; if (shortcut && !in16) raw = b.b16(size_t(x0.M()) * Cin);
-    b.groupnorm(x0, x1, p + ".norm1", eps, ACT_SILU, n1.p, (shortcut && !in16) ? raw.p : nullptr, in16);
+    const Builder::GnSaved s1 = b.groupnorm(x0, x1, p + ".norm1", eps, ACT_SILU, n1.p, (shortcut && !in16) ? raw.p : nullptr, in16);
     // conv1 (+ bias + time embedding row bias) -> 16-bit intermediate (it only feeds norm2)
     Act h1 = b.act(Bn, H, W, Cout, false, true);
     {
@@ -771,7 +766,7 @@ struct Model {
     }
     b.free(n1);
     B16T n2 = b.b16(size_t(x0.M()) * Cout);
-    b.groupnorm(h1, nullptr, p + ".norm2", eps, ACT_SILU, n2.p, nullptr, /*in16=*/true);
+    const Builder::GnSaved s2 = b.groupnorm(h1, nullptr, p + ".norm2", eps, ACT_SILU, n2.p, nullptr, /*in16=*/true);
     b.free(h1);
     Act out = b.act(Bn, H, W, Cout, !out16_only, want_b16 || want_s2d || out16_only);
     out.h_s2d = want_s2d;
@@ -796,105 +791,235 @@ struct Model {
     }
     b.free(n2);
     if (shortcut && !in16) b.free(raw);
+    if (!b.recording()) return out;
+    // ---- backward
+    const Act xa = x0, xb = x1 ? *x1 : Act();
+    const bool has_b = x1 != nullptr;
+    b.tape.push_back([=]() {
+      // dgrad operands are registered whether or not this block ends up on the gradient path (the layout must not depend on it)
+      const size_t w2 = b.dconv_w(p + ".conv2", Cout, Cout, 9), w1 = b.dconv_w(p + ".conv1", Cout, Cin, 9);
+      const size_t wsc = shortcut ? b.dconv_w(p + ".conv_shortcut", Cout, Cin, 1) : 0;
+      if (!out.gr->written) return;
+      const long M = xa.M();
+      B16T g16 = b.b16(size_t(M) * Cout);
+      to16(out.gr->f.p, M * Cout, g16.p);
+      B16T dn2 = b.b16(size_t(M) * Cout);
+      { GemmDesc d; d.seg[0] = Builder::seg_3x3(g16.p, Bn, H, W, Cout); d.M = int(M); d.N = Cout; d.Nw = Cout; d.w = b.dpw(w2);
+        d.out_bf16 = dn2.p; d.ldo16 = Cout; b.gemm(d); }
+      B16T dh1 = b.b16(size_t(M) * Cout);
+      b.groupnorm_bwd(h1, nullptr, true, s2, nullptr, p + ".norm2", eps, ACT_SILU, dn2.p, nullptr, dh1.p, nullptr, 0, nullptr, 0, nullptr, nullptr);
+      b.free(dn2);
+      { const bf16* src = dh1.p; float* dst = d_temb_all.p ? d_temb_all.p + temb_off.at(p) : nullptr; const int tt = temb_total, h16 = f16(), HWi = H * W;
+        b.emit([=](cudaStream_t st) { return colsum_per_image(src, Bn, HWi, Cout, h16, dst, tt, st); }); }
+      const bool need_a = Builder::wants_grad(xa), need_b = has_b && Builder::wants_grad(xb);
+      if (need_a || need_b) {
+        B16T dn1 = b.b16(size_t(M) * Cin);
+        { GemmDesc d; d.seg[0] = Builder::seg_3x3(dh1.p, Bn, H, W, Cout); d.M = int(M); d.N = Cin; d.Nw = Cin; d.w = b.dpw(w1);
+          d.out_bf16 = dn1.p; d.ldo16 = Cin; b.gemm(d); }
+        F32T T;
+        const float* extra = out.gr->f.p;  // identity residual: d(x) += d(out)
+        if (shortcut) {
+          T = b.f32(size_t(M) * Cin);
+          GemmDesc d; d.seg[0] = Builder::seg_1x1(g16.p, Bn, H, W, Cout); d.M = int(M); d.N = Cin; d.Nw = Cin; d.w = b.dpw(wsc);
+          d.out_f32 = T.p; d.ldo32 = Cin; b.gemm(d);
+          extra = T.p;
+        }
+        int acc_a = 0, acc_b = 0;
+        float* da = need_a ? b.grad(xa, &acc_a) : nullptr;
+        float* db = need_b ? b.grad(xb, &acc_b) : nullptr;
+        b.groupnorm_bwd(xa, has_b ? &xb : nullptr, false, s1, nullptr, p + ".norm1", eps, ACT_SILU, dn1.p, extra, nullptr, da, acc_a, db, acc_b, nullptr, nullptr);
+        if (shortcut) b.free(T);
+        b.free(dn1);
+      }
+      b.free(dh1); b.free(g16);
+    });
     return out;
   }
 
   // ---- Transformer2DModel (one BasicTransformerBlock): returns fp32 (+bf16) output; x is NOT freed
   Act transformer(const std::string& p, const Act& x, bool want_b16, bool want_s2d = false) {
     if (getenv("MADM_NO_S2D_FUSE")) want_s2d = false;
+    const bool train = b.recording();
     const int Bn = x.B, H = x.H, W = x.W, C = x.C;
     const long M = x.M();
-    const int heads = 8, d_head = C / heads;
+    const int heads = 8, d_head = C / heads, n_tok = H * W;
+    const float sc = 1.0f / sqrtf(float(d_head));
     const std::string tb = p + ".transformer_blocks.0";
+    const int h16 = f16(), Mi = int(M);
     B16T n = b.b16(size_t(M) * C);
-    b.groupnorm(x, nullptr, p + ".norm", 1e-6f, ACT_NONE, n.p, nullptr);
-    // The block's internal hidden-state stream (proj_in output, updated in place by the two attention out-projections, consumed by
-    // the feed-forward) is kept in fp16 with fp16 operands, as under the reference's fp16 autocast: its three residual GEMMs are
-    // bound by that stream's HBM traffic.  It is re-based on the fp32 UNet stream by proj_out, so rounding does not accumulate
-    // across blocks.
-    // Measured: NOT a win at these sizes -- the 42 MB stream of a 64x64 block lives in the 126 MB L2, so the residual GEMMs are
-    // bound by epilogue latency rather than HBM bytes, and the conversions cost more than the bytes save (step 23.7 -> 24.5 ms,
-    // LayerNorm 0.71 -> 0.81 ms).  Off by default; MADM_TF_STREAM16=1 enables it (tested at op level and end to end).
-    const bool hs16 = f16() && getenv("MADM_TF_STREAM16");
-    F32T hs; B16T hsh;
-    if (hs16) hsh = b.b16(size_t(M) * C); else hs = b.f32(size_t(M) * C);
-    auto residual_inplace = [&](GemmDesc& d) {  // hs += GEMM
-      if (hs16) { d.residual = reinterpret_cast<const float*>(hsh.p); d.res16 = 1; d.ldr = C; d.out_bf16 = hsh.p; d.ldo16 = C; }
-      else { d.residual = hs.p; d.ldr = C; d.out_f32 = hs.p; d.ldo32 = C; }
-    };
-    { GemmDesc d; d.seg[0] = Builder::seg_1x1(n.p, Bn, H, W, C); d.M = int(M); d.N = C; d.Nw = C;
-      d.w = b.pw(b.conv_w(p + ".proj_in", C, C, 1)); d.bias = P(p + ".proj_in.bias", C);
-      if (hs16) { d.out_bf16 = hsh.p; d.ldo16 = C; } else { d.out_f32 = hs.p; d.ldo32 = C; }
-      b.gemm(d); }
+    const Builder::GnSaved sn = b.groupnorm(x, nullptr, p + ".norm", 1e-6f, ACT_NONE, n.p, nullptr);
+    // The block's fp32 hidden state in its three versions: proj_in's output and the results of the two attention out-projections.
+    // Inference updates one buffer in place (hs += GEMM); a training plan keeps every version for the LayerNorm backward.
+    F32T hs0 = b.f32(size_t(M) * C), hs1 = train ? b.f32(size_t(M) * C) : hs0, hs2 = train ? b.f32(size_t(M) * C) : hs0;
+    { GemmDesc d; d.seg[0] = Builder::seg_1x1(n.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C;
+      d.w = b.pw(b.conv_w(p + ".proj_in", C, C, 1)); d.bias = P(p + ".proj_in.bias", C); d.out_f32 = hs0.p; d.ldo32 = C; b.gemm(d); }
     b.free(n);
-    auto ln = [&](const std::string& name, bf16* y) {
+    auto ln = [&](const std::string& name, const float* src, bf16* y) {
       const float* g = P(name + ".weight", C); const float* be = P(name + ".bias", C);
-      const void* src = hs16 ? static_cast<const void*>(hsh.p) : static_cast<const void*>(hs.p); const int Mi = int(M);
-      const int h16 = f16(), i16 = hs16 ? 1 : 0;
-      b.emit([=](cudaStream_t st) { return layernorm(src, i16, Mi, C, g, be, 1e-5f, y, h16, st); }, false, MADM_KIND_LAYERNORM, 0.0,
-             double(Mi) * C * (hs16 ? 4 : 6));
+      b.emit([=](cudaStream_t st) { return layernorm(src, 0, Mi, C, g, be, 1e-5f, y, h16, st); }, false, MADM_KIND_LAYERNORM, 0.0, double(Mi) * C * 6);
     };
     // --- self attention
     B16T l1 = b.b16(size_t(M) * C);
-    ln(tb + ".norm1", l1.p);
+    ln(tb + ".norm1", hs0.p, l1.p);
     B16T qkv = b.b16(size_t(M) * 3 * C);
     { const size_t reg = b.region("qkv:" + tb, size_t(3) * C * C * 2);
       b.linear_part(tb + ".attn1.to_q", reg, 0, C, C, true);
       b.linear_part(tb + ".attn1.to_k", reg, C, C, C, true);
       b.linear_part(tb + ".attn1.to_v", reg, 2 * C, C, C, true);
-      GemmDesc d; d.seg[0] = Builder::seg_plain(l1.p, M, C); d.M = int(M); d.N = 3 * C; d.Nw = 3 * C; d.w = b.pw(reg);
+      GemmDesc d; d.seg[0] = Builder::seg_plain(l1.p, M, C); d.M = Mi; d.N = 3 * C; d.Nw = 3 * C; d.w = b.pw(reg);
       d.out_bf16 = qkv.p; d.ldo16 = 3 * C; b.gemm(d); }
     b.free(l1);
     B16T att = b.b16(size_t(M) * C);
-    { const bf16* q = qkv.p; bf16* o = att.p; const int n_tok = H * W; const float sc = 1.0f / sqrtf(float(d_head));
-      b.attention(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, o, C, Bn, heads, d_head, n_tok, n_tok, long(n_tok) * 3 * C, long(n_tok) * 3 * C,
-                  long(n_tok) * C, sc); }
+    F32T lse1, lse2;  // training: log-sum-exp rows of both attentions (for the backward)
+    if (train) { lse1 = b.f32(size_t(Bn) * heads * n_tok); lse2 = b.f32(size_t(Bn) * heads * n_tok); }
+    { const bf16* q = qkv.p;
+      b.attention(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, att.p, C, Bn, heads, d_head, n_tok, n_tok, long(n_tok) * 3 * C, long(n_tok) * 3 * C,
+                  long(n_tok) * C, sc, lse1.p); }
     b.free(qkv);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(att.p, M, C); d.M = int(M); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_plain(att.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
       d.w = b.pw(b.linear_w(tb + ".attn1.to_out.0", C, C, true)); d.bias = lora_bias(tb + ".attn1.to_out.0", C);
-      residual_inplace(d); b.gemm(d); }
+      d.residual = hs0.p; d.ldr = C; d.out_f32 = hs1.p; d.ldo32 = C; b.gemm(d); }
     // --- cross attention (K/V precomputed for all layers in kv_all)
     B16T l2 = b.b16(size_t(M) * C);
-    ln(tb + ".norm2", l2.p);
+    ln(tb + ".norm2", hs1.p, l2.p);
     B16T q2 = b.b16(size_t(M) * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(l2.p, M, C); d.M = int(M); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_plain(l2.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
       d.w = b.pw(b.linear_w(tb + ".attn2.to_q", C, C, true)); d.out_bf16 = q2.p; d.ldo16 = C; b.gemm(d); }
     b.free(l2);
-    { const bf16* q = q2.p; bf16* o = att.p; const int n_tok = H * W; const float sc = 1.0f / sqrtf(float(d_head));
-      const int off = kv_off[tb + ".attn2"]; const bf16* kv = kv_all.p; const int ldkv = kv_total;
-      b.attention(q, C, kv ? kv + off : nullptr, ldkv, kv ? kv + off + C : nullptr, ldkv, o, C, Bn, heads, d_head, n_tok, 77, long(n_tok) * C,
-                  long(77) * ldkv, long(n_tok) * C, sc); }
+    const B16T att2 = train ? b.b16(size_t(M) * C) : att;  // inference reuses the self-attention's output buffer (freed once, as att)
+    const int kvo = kv_off[tb + ".attn2"], ldkv = kv_total;
+    { const bf16* kv = kv_all.p;
+      b.attention(q2.p, C, kv ? kv + kvo : nullptr, ldkv, kv ? kv + kvo + C : nullptr, ldkv, att2.p, C, Bn, heads, d_head, n_tok, 77, long(n_tok) * C,
+                  long(77) * ldkv, long(n_tok) * C, sc, lse2.p); }
     b.free(q2);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(att.p, M, C); d.M = int(M); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_plain(att2.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
       d.w = b.pw(b.linear_w(tb + ".attn2.to_out.0", C, C, true)); d.bias = lora_bias(tb + ".attn2.to_out.0", C);
-      residual_inplace(d); b.gemm(d); }
+      d.residual = hs1.p; d.ldr = C; d.out_f32 = hs2.p; d.ldo32 = C; b.gemm(d); }
     b.free(att);
-    // --- feed-forward (GEGLU fused in the first GEMM's epilogue)
+    // --- feed-forward.  Inference: GEGLU fused in the first GEMM's epilogue.  Training keeps the pre-activation: raw = l3 W1^T + b1 in
+    // natural column order (hidden | gate; weight from the dgrad arena), then the GEGLU pass.
     B16T l3 = b.b16(size_t(M) * C);
-    ln(tb + ".norm3", l3.p);
+    ln(tb + ".norm3", hs2.p, l3.p);
+    B16T rawff; if (train) rawff = b.b16(size_t(M) * 8 * C);
     B16T ff = b.b16(size_t(M) * 4 * C);
-    { const PackEntry& e = b.entry("geglu:" + tb, [&] {
+    if (train) {
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(l3.p, M, C); d.M = Mi; d.N = 8 * C; d.Nw = 8 * C;
+        d.w = b.dpw(b.dlinear_fwd(tb + ".ff.net.0.proj", 8 * C, C)); d.bias = P(tb + ".ff.net.0.proj.bias", 8 * C);
+        d.out_bf16 = rawff.p; d.ldo16 = 8 * C; b.gemm(d); }
+      const bf16* src = rawff.p; bf16* dst = ff.p; const int Hh = 4 * C;
+      b.emit([=](cudaStream_t st) { return geglu_fwd(src, M, Hh, dst, h16, st); }, false, MADM_KIND_ELEMENTWISE, 0.0, double(M) * C * 24);
+    } else {
+      const PackEntry& e = b.entry("geglu:" + tb, [&] {
         PackEntry pe; pe.kind = PK_GEGLU; pe.src = tb + ".ff.net.0.proj.weight"; pe.src2 = tb + ".ff.net.0.proj.bias"; pe.N = 4 * C; pe.C = C;
         pe.off = b.pack_reserve(size_t(8) * C * C * 2); pe.bias_off = b.pack_reserve(size_t(8) * C * 4);
         return pe; });
-      GemmDesc d; d.seg[0] = Builder::seg_plain(l3.p, M, C); d.M = int(M); d.N = 4 * C; d.Nw = 8 * C; d.w = b.pw(e.off);
-      d.bias = b.pf(e.bias_off); d.act = ACT_GEGLU; d.out_bf16 = ff.p; d.ldo16 = 4 * C; b.gemm(d); }
+      GemmDesc d; d.seg[0] = Builder::seg_plain(l3.p, M, C); d.M = Mi; d.N = 4 * C; d.Nw = 8 * C; d.w = b.pw(e.off);
+      d.bias = b.pf(e.bias_off); d.act = ACT_GEGLU; d.out_bf16 = ff.p; d.ldo16 = 4 * C; b.gemm(d);
+    }
     b.free(l3);
     B16T hsb = b.b16(size_t(M) * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(ff.p, M, 4 * C); d.M = int(M); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_plain(ff.p, M, 4 * C); d.M = Mi; d.N = C; d.Nw = C;
       d.w = b.pw(b.linear_w(tb + ".ff.net.2", C, 4 * C, false)); d.bias = P(tb + ".ff.net.2.bias", C);
-      if (hs16) { d.residual = reinterpret_cast<const float*>(hsh.p); d.res16 = 1; } else d.residual = hs.p;
-      d.ldr = C; d.out_bf16 = hsb.p; d.ldo16 = C; b.gemm(d); }
+      d.residual = hs2.p; d.ldr = C; d.out_bf16 = hsb.p; d.ldo16 = C; b.gemm(d); }
     b.free(ff);
-    if (hs16) b.free(hsh); else b.free(hs);
+    b.free(hs0);
     Act out = b.act(Bn, H, W, C, true, want_b16 || want_s2d);
     out.h_s2d = want_s2d;
-    { GemmDesc d; d.seg[0] = Builder::seg_1x1(hsb.p, Bn, H, W, C); d.M = int(M); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_1x1(hsb.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C;
       if (want_s2d) { d.s2d_H = H; d.s2d_W = W; }
       d.w = b.pw(b.conv_w(p + ".proj_out", C, C, 1)); d.bias = P(p + ".proj_out.bias", C);
       d.residual = x.f.p; d.ldr = C; d.out_f32 = out.f.p; d.ldo32 = C; d.out_bf16 = out.h.p; d.ldo16 = C;
       b.attach_colstats(out, d); b.gemm(d); }
     b.free(hsb);
+    if (!train) return out;
+    // ---- backward
+    const Act xin = x;
+    b.tape.push_back([=]() {
+      const size_t w_po = b.dconv_w(p + ".proj_out", C, C, 1), w_pi = b.dconv_w(p + ".proj_in", C, C, 1);
+      const size_t w_ff2 = b.dlinear_w(tb + ".ff.net.2", C, 4 * C, false), w_ff1 = b.dlinear_w(tb + ".ff.net.0.proj", 8 * C, C, false);
+      const size_t w_o2 = b.dlinear_w(tb + ".attn2.to_out.0", C, C, true), w_q2 = b.dlinear_w(tb + ".attn2.to_q", C, C, true);
+      const size_t w_o1 = b.dlinear_w(tb + ".attn1.to_out.0", C, C, true);
+      const size_t w_qkv = b.dregion("qkv:" + tb, size_t(3) * C * C * 2);
+      b.dlinear_part(tb + ".attn1.to_q", w_qkv, 0, C, C, 3 * C, true);
+      b.dlinear_part(tb + ".attn1.to_k", w_qkv, C, C, C, 3 * C, true);
+      b.dlinear_part(tb + ".attn1.to_v", w_qkv, 2 * C, C, C, 3 * C, true);
+      if (b.mode == LAYOUT) {  // the LoRA factor operands of this block
+        for (const char* m : {".attn1.to_q", ".attn1.to_k", ".attn1.to_v", ".attn1.to_out.0", ".attn2.to_q", ".attn2.to_out.0"}) { b.dlora_a(tb + m, C); b.dlora_bt(tb + m, C); }
+        b.dlora_a(tb + ".attn2.to_k", 768); b.dlora_bt(tb + ".attn2.to_k", C);
+        b.dlora_a(tb + ".attn2.to_v", 768); b.dlora_bt(tb + ".attn2.to_v", C);
+      }
+      if (!out.gr->written) return;
+      // dh = gradient of the block's hidden state (fp32), carried backwards through the three residual branches
+      B16T g16 = b.b16(size_t(M) * C);
+      to16(out.gr->f.p, M * C, g16.p);
+      F32T dh = b.f32(size_t(M) * C);
+      B16T dh16 = b.b16(size_t(M) * C);
+      { GemmDesc d; d.seg[0] = Builder::seg_1x1(g16.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_po);
+        d.out_f32 = dh.p; d.ldo32 = C; d.out_bf16 = dh16.p; d.ldo16 = C; b.gemm(d); }
+      b.free(g16);
+      // --- feed-forward
+      B16T dff = b.b16(size_t(M) * 4 * C);
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = 4 * C; d.Nw = 4 * C; d.w = b.dpw(w_ff2); d.out_bf16 = dff.p; d.ldo16 = 4 * C; b.gemm(d); }
+      B16T draw = b.b16(size_t(M) * 8 * C);
+      { const bf16* r = rawff.p; const bf16* dy = dff.p; bf16* dst = draw.p; const int Hh = 4 * C;
+        b.emit([=](cudaStream_t st) { return geglu_bwd(r, dy, M, Hh, dst, h16, st); }); }
+      b.free(dff);
+      B16T dl = b.b16(size_t(M) * C);
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(draw.p, M, 8 * C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_ff1); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
+      b.free(draw);
+      auto ln_bwd = [&](const std::string& name, const float* xs) {  // dh += LayerNorm'(xs) dl ; dh16 = 16-bit(dh)
+        const float* g = P(name + ".weight", C); const bf16* dy = dl.p; float* dst = dh.p; bf16* d16 = dh16.p;
+        b.emit([=](cudaStream_t st) -> const char* {
+          return layernorm_bwd(xs, Mi, C, g, 1e-5f, dy, h16, dst, 1, st, d16);  // (writes the 16-bit copy of dh as well)
+        });
+      };
+      ln_bwd(tb + ".norm3", hs2.p);
+      F32T ascr = b.f32(attention_bwd_scratch_floats(Bn, heads, d_head, n_tok, n_tok > 77 ? n_tok : 77) + attention_bwd_scratch_floats(Bn, heads, d_head, n_tok, 77));
+      // --- cross attention
+      B16T datt = b.b16(size_t(M) * C);
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o2); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
+      lora_wgrad(tb + ".attn2.to_out.0", att2.p, C, dh16.p, C, M, C, C);
+      B16T dq2 = b.b16(size_t(M) * C);
+      { const bf16* q = q2.p; const bf16* kv = kv_all.p; const bf16* o = att2.p; const bf16* dop = datt.p; bf16* dqp = dq2.p; bf16* dkv = dkv_all.p; float* sp = ascr.p;
+        const float* lse = lse2.p;
+        b.emit([=](cudaStream_t st) {
+          return attention_bwd(q, C, kv + kvo, ldkv, kv + kvo + C, ldkv, o, C, dop, C, dqp, C, dkv + kvo, ldkv, dkv + kvo + C, ldkv, Bn, heads, d_head, n_tok, 77,
+                               long(n_tok) * C, long(77) * ldkv, long(77) * ldkv, long(n_tok) * C, long(n_tok) * C, long(n_tok) * C, long(77) * ldkv,
+                               long(77) * ldkv, sc, sp, h16, st, lse); }); }
+      lora_wgrad(tb + ".attn2.to_q", l2.p, C, dq2.p, C, M, C, C);
+      lora_wgrad(tb + ".attn2.to_k", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo : nullptr, ldkv, long(Bn) * 77, C, 768);
+      lora_wgrad(tb + ".attn2.to_v", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo + C : nullptr, ldkv, long(Bn) * 77, C, 768);
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(dq2.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_q2); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
+      b.free(dq2);
+      ln_bwd(tb + ".norm2", hs1.p);
+      // --- self attention
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o1); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
+      lora_wgrad(tb + ".attn1.to_out.0", att.p, C, dh16.p, C, M, C, C);
+      B16T dqkv = b.b16(size_t(M) * 3 * C);
+      { const bf16* q = qkv.p; const bf16* o = att.p; const bf16* dop = datt.p; bf16* dq = dqkv.p; float* sp = ascr.p;
+        const float* lse = lse1.p;
+        b.emit([=](cudaStream_t st) {
+          return attention_bwd(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, o, C, dop, C, dq, 3 * C, dq + C, 3 * C, dq + 2 * C, 3 * C, Bn, heads, d_head, n_tok, n_tok,
+                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * C, long(n_tok) * C, long(n_tok) * 3 * C,
+                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, sc, sp, h16, st, lse); }); }
+      b.free(datt);
+      lora_wgrad(tb + ".attn1.to_q", l1.p, C, dqkv.p, 3 * C, M, C, C);
+      lora_wgrad(tb + ".attn1.to_k", l1.p, C, dqkv.p ? dqkv.p + C : nullptr, 3 * C, M, C, C);
+      lora_wgrad(tb + ".attn1.to_v", l1.p, C, dqkv.p ? dqkv.p + 2 * C : nullptr, 3 * C, M, C, C);
+      { GemmDesc d; d.seg[0] = Builder::seg_plain(dqkv.p, M, 3 * C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_qkv); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
+      b.free(dqkv); b.free(ascr);
+      ln_bwd(tb + ".norm1", hs0.p);
+      // --- proj_in, GroupNorm; the block's residual adds d(out) to d(x)
+      if (Builder::wants_grad(xin)) {
+        B16T dn = b.b16(size_t(M) * C);
+        { GemmDesc d; d.seg[0] = Builder::seg_1x1(dh16.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_pi); d.out_bf16 = dn.p; d.ldo16 = C; b.gemm(d); }
+        int acc = 0;
+        float* dx = b.grad(xin, &acc);
+        b.groupnorm_bwd(xin, nullptr, false, sn, nullptr, p + ".norm", 1e-6f, ACT_NONE, dn.p, out.gr->f.p, nullptr, dx, acc, nullptr, 0, nullptr, nullptr);
+        b.free(dn);
+      }
+      b.free(dl); b.free(dh16); b.free(dh);
+    });
     return out;
   }
 
@@ -926,6 +1051,24 @@ struct Model {
       if (out16_only) { d.out_bf16 = out.h.p; d.ldo16 = C; } else { d.out_f32 = out.f.p; d.ldo32 = C; }
       b.attach_colstats(out, d); b.gemm(d); }
     if (!x.h_s2d) b.free(s2d);
+    if (!b.recording()) return out;
+    const Act xin = x;
+    b.tape.push_back([=]() {
+      const size_t w = b.dconv_w(p + ".conv", C, C, 9);
+      if (!out.gr->written || !Builder::wants_grad(xin)) return;
+      // input gradient of the stride-2 conv: zero-stuff d(out) onto the input grid, then the stride-1 dgrad GEMM with mirrored taps
+      const long Mo = out.M(), Mx = xin.M();
+      B16T g16 = b.b16(size_t(Mo) * C);
+      to16(out.gr->f.p, Mo * C, g16.p);
+      B16T z = b.b16(size_t(Mx) * C);
+      { const bf16* src = g16.p; bf16* dst = z.p; b.emit([=](cudaStream_t st) { return zero_stuff2x(src, Bn, H / 2, W / 2, C, dst, st); }); }
+      int acc = 0;
+      float* dx = b.grad(xin, &acc);
+      { GemmDesc d; d.seg[0] = Builder::seg_3x3(z.p, Bn, H, W, C); d.M = int(Mx); d.N = C; d.Nw = C; d.w = b.dpw(w);
+        if (acc) { d.residual = dx; d.ldr = C; }
+        d.out_f32 = dx; d.ldo32 = C; b.gemm(d); }
+      b.free(z); b.free(g16);
+    });
     return out;
   }
 
@@ -947,6 +1090,22 @@ struct Model {
       if (out16_only) { d.out_bf16 = out.h.p; d.ldo16 = C; } else { d.out_f32 = out.f.p; d.ldo32 = C; }
       b.attach_colstats(out, d); b.gemm(d); }
     b.free(up);
+    if (!b.recording()) return out;
+    const Act xin = x;
+    b.tape.push_back([=]() {
+      const size_t w = b.dconv_w(p + ".conv", C, C, 9);
+      if (!out.gr->written || !Builder::wants_grad(xin)) return;
+      const long Mo = out.M();
+      B16T g16 = b.b16(size_t(Mo) * C);
+      to16(out.gr->f.p, Mo * C, g16.p);
+      F32T dup = b.f32(size_t(Mo) * C);
+      { GemmDesc d; d.seg[0] = Builder::seg_3x3(g16.p, Bn, 2 * H, 2 * W, C); d.M = int(Mo); d.N = C; d.Nw = C; d.w = b.dpw(w);
+        d.out_f32 = dup.p; d.ldo32 = C; b.gemm(d); }
+      int acc = 0;
+      float* dx = b.grad(xin, &acc);
+      { const float* src = dup.p; b.emit([=](cudaStream_t st) { return sum2x2(src, Bn, H, W, C, dx, acc, st); }); }
+      b.free(dup); b.free(g16);
+    });
     return out;
   }
 
@@ -1013,9 +1172,10 @@ struct Model {
 
 
   // ============================================================================================== training path (SURVEY §8 row f-3)
-  // The training forward runs the same kernels as inference with three differences: nothing is freed in the differentiated stages,
-  // the transformer's hidden state is not updated in place (LayerNorm backward needs every version), and GEGLU keeps its pre-activation
-  // (natural-order feed-forward weight from the dgrad arena + one elementwise pass).  Every piece records its backward on the tape.
+  // A block's forward is the same builder function for inference and training; in a training plan (Builder::recording()) it also records
+  // its backward on the tape.  The training forward differs in three data choices: nothing is freed in the differentiated stages, the
+  // transformer's hidden state is not updated in place (LayerNorm backward needs every version), and GEGLU keeps its pre-activation
+  // (natural-order feed-forward weight from the dgrad arena + one elementwise pass).
   F32T d_temb_all;   // [B, temb_total] gradient of all 22 time_emb_proj outputs
   B16T dkv_all;      // [B*77, kv_total] gradient of all cross-attention K / V
   F32T emb_saved;    // [B,1280] time_embedding output before (+ cond_emb, SiLU)
@@ -1064,560 +1224,6 @@ struct Model {
       const bf16* vp = V.p; float* sp = scr.p;
       b.emit([=](cudaStream_t st) { return wgrad(X, ldx, vp, 16, Mi, K, 16, 1, 0, 0, 0, alpha, gA, 1, K, 0, sp, h16, st); });  // (X^T V)^T -> [16,K]
       b.free(scr); b.free(V);
-    }
-  }
-
-  // ---- ResnetBlock2D of the UNet, training forward + tape
-  Act resblock_train(const std::string& p, const Act& x0, const Act* x1, int Cout, bool want_b16, bool want_s2d = false) {
-    const int Bn = x0.B, H = x0.H, W = x0.W, Cin = x0.C + (x1 ? x1->C : 0);
-    const bool shortcut = Cin != Cout;
-    const float eps = 1e-5f;
-    if (x1 && !shortcut) b.fail(MADM_EINVAL, "resblock: concat input without shortcut");
-    B16T n1 = b.b16(size_t(x0.M()) * Cin);
-    B16T raw; if (shortcut) raw = b.b16(size_t(x0.M()) * Cin);
-    const Builder::GnSaved s1 = b.groupnorm(x0, x1, p + ".norm1", eps, ACT_SILU, n1.p, shortcut ? raw.p : nullptr, false);
-    Act h1 = b.act(Bn, H, W, Cout, false, true);
-    { GemmDesc d; d.seg[0] = Builder::seg_3x3(n1.p, Bn, H, W, Cin); d.M = int(x0.M()); d.N = Cout;
-      d.w = b.pw(b.conv_w(p + ".conv1", Cout, Cin, 9)); d.Nw = Cout; d.bias = P(p + ".conv1.bias", Cout);
-      d.rowbias = temb_all.p ? temb_all.p + temb_off[p] : nullptr; d.ld_rowbias = temb_total; d.rows_per_img = H * W;
-      if (dry()) d.rowbias = nullptr;
-      d.out_bf16 = h1.h.p; d.ldo16 = Cout; b.attach_colstats(h1, d); b.gemm(d); }
-    B16T n2 = b.b16(size_t(x0.M()) * Cout);
-    const Builder::GnSaved s2 = b.groupnorm(h1, nullptr, p + ".norm2", eps, ACT_SILU, n2.p, nullptr, /*in16=*/true);
-    Act out = b.act(Bn, H, W, Cout, true, want_b16 || want_s2d);
-    out.h_s2d = want_s2d;
-    { GemmDesc d; d.seg[0] = Builder::seg_3x3(n2.p, Bn, H, W, Cout); d.M = int(x0.M()); d.N = Cout; d.Nw = Cout;
-      if (want_s2d) { d.s2d_H = H; d.s2d_W = W; }
-      if (shortcut) {
-        Builder::Fused f = b.conv_plus_shortcut(p + ".conv2", p + ".conv_shortcut", Cout, Cin);
-        d.nseg = 2; d.seg[1] = Builder::seg_1x1(raw.p, Bn, H, W, Cin); d.w = b.pw(f.w_off); d.bias = b.pf(f.b_off);
-      } else {
-        d.w = b.pw(b.conv_w(p + ".conv2", Cout, Cout, 9)); d.bias = P(p + ".conv2.bias", Cout); d.residual = x0.f.p; d.ldr = Cout;
-      }
-      d.out_f32 = out.f.p; d.ldo32 = Cout; d.out_bf16 = out.h.p; d.ldo16 = Cout; b.attach_colstats(out, d); b.gemm(d); }
-    // ---- backward
-    const Act xa = x0, xb = x1 ? *x1 : Act();
-    const bool has_b = x1 != nullptr;
-    b.tape.push_back([=]() {
-      // dgrad operands are registered whether or not this block ends up on the gradient path (the layout must not depend on it)
-      const size_t w2 = b.dconv_w(p + ".conv2", Cout, Cout, 9), w1 = b.dconv_w(p + ".conv1", Cout, Cin, 9);
-      const size_t wsc = shortcut ? b.dconv_w(p + ".conv_shortcut", Cout, Cin, 1) : 0;
-      if (!out.gr->written) return;
-      const long M = xa.M();
-      B16T g16 = b.b16(size_t(M) * Cout);
-      to16(out.gr->f.p, M * Cout, g16.p);
-      B16T dn2 = b.b16(size_t(M) * Cout);
-      { GemmDesc d; d.seg[0] = Builder::seg_3x3(g16.p, Bn, H, W, Cout); d.M = int(M); d.N = Cout; d.Nw = Cout; d.w = b.dpw(w2);
-        d.out_bf16 = dn2.p; d.ldo16 = Cout; b.gemm(d); }
-      B16T dh1 = b.b16(size_t(M) * Cout);
-      b.groupnorm_bwd(h1, nullptr, true, s2, nullptr, p + ".norm2", eps, ACT_SILU, dn2.p, nullptr, dh1.p, nullptr, 0, nullptr, 0, nullptr, nullptr);
-      b.free(dn2);
-      { const bf16* src = dh1.p; float* dst = d_temb_all.p ? d_temb_all.p + temb_off.at(p) : nullptr; const int tt = temb_total, h16 = f16(), HWi = H * W;
-        b.emit([=](cudaStream_t st) { return colsum_per_image(src, Bn, HWi, Cout, h16, dst, tt, st); }); }
-      const bool need_a = Builder::wants_grad(xa), need_b = has_b && Builder::wants_grad(xb);
-      if (need_a || need_b) {
-        B16T dn1 = b.b16(size_t(M) * Cin);
-        { GemmDesc d; d.seg[0] = Builder::seg_3x3(dh1.p, Bn, H, W, Cout); d.M = int(M); d.N = Cin; d.Nw = Cin; d.w = b.dpw(w1);
-          d.out_bf16 = dn1.p; d.ldo16 = Cin; b.gemm(d); }
-        F32T T;
-        const float* extra = out.gr->f.p;  // identity residual: d(x) += d(out)
-        if (shortcut) {
-          T = b.f32(size_t(M) * Cin);
-          GemmDesc d; d.seg[0] = Builder::seg_1x1(g16.p, Bn, H, W, Cout); d.M = int(M); d.N = Cin; d.Nw = Cin; d.w = b.dpw(wsc);
-          d.out_f32 = T.p; d.ldo32 = Cin; b.gemm(d);
-          extra = T.p;
-        }
-        int acc_a = 0, acc_b = 0;
-        float* da = need_a ? b.grad(xa, &acc_a) : nullptr;
-        float* db = need_b ? b.grad(xb, &acc_b) : nullptr;
-        b.groupnorm_bwd(xa, has_b ? &xb : nullptr, false, s1, nullptr, p + ".norm1", eps, ACT_SILU, dn1.p, extra, nullptr, da, acc_a, db, acc_b, nullptr, nullptr);
-        if (shortcut) b.free(T);
-        b.free(dn1);
-      }
-      b.free(dh1); b.free(g16);
-    });
-    return out;
-  }
-
-  // ---- Transformer2DModel (one BasicTransformerBlock), training forward + tape
-  Act transformer_train(const std::string& p, const Act& x, bool want_b16, bool want_s2d = false) {
-    const int Bn = x.B, H = x.H, W = x.W, C = x.C;
-    const long M = x.M();
-    const int heads = 8, d_head = C / heads, n_tok = H * W;
-    const float sc = 1.0f / sqrtf(float(d_head));
-    const std::string tb = p + ".transformer_blocks.0";
-    const int h16 = f16(), Mi = int(M);
-    B16T n = b.b16(size_t(M) * C);
-    const Builder::GnSaved sn = b.groupnorm(x, nullptr, p + ".norm", 1e-6f, ACT_NONE, n.p, nullptr);
-    F32T hs0 = b.f32(size_t(M) * C), hs1 = b.f32(size_t(M) * C), hs2 = b.f32(size_t(M) * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_1x1(n.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C;
-      d.w = b.pw(b.conv_w(p + ".proj_in", C, C, 1)); d.bias = P(p + ".proj_in.bias", C); d.out_f32 = hs0.p; d.ldo32 = C; b.gemm(d); }
-    auto ln = [&](const std::string& name, const float* src, bf16* y) {
-      const float* g = P(name + ".weight", C); const float* be = P(name + ".bias", C);
-      b.emit([=](cudaStream_t st) { return layernorm(src, 0, Mi, C, g, be, 1e-5f, y, h16, st); }, false, MADM_KIND_LAYERNORM, 0.0, double(Mi) * C * 6);
-    };
-    // --- self attention
-    B16T l1 = b.b16(size_t(M) * C);
-    ln(tb + ".norm1", hs0.p, l1.p);
-    B16T qkv = b.b16(size_t(M) * 3 * C);
-    { const size_t reg = b.region("qkv:" + tb, size_t(3) * C * C * 2);
-      b.linear_part(tb + ".attn1.to_q", reg, 0, C, C, true);
-      b.linear_part(tb + ".attn1.to_k", reg, C, C, C, true);
-      b.linear_part(tb + ".attn1.to_v", reg, 2 * C, C, C, true);
-      GemmDesc d; d.seg[0] = Builder::seg_plain(l1.p, M, C); d.M = Mi; d.N = 3 * C; d.Nw = 3 * C; d.w = b.pw(reg);
-      d.out_bf16 = qkv.p; d.ldo16 = 3 * C; b.gemm(d); }
-    B16T att1 = b.b16(size_t(M) * C);
-    F32T lse1 = b.f32(size_t(Bn) * heads * n_tok), lse2 = b.f32(size_t(Bn) * heads * n_tok);  // log-sum-exp rows of both attentions (for the backward)
-    b.attention(qkv.p, 3 * C, qkv.p ? qkv.p + C : nullptr, 3 * C, qkv.p ? qkv.p + 2 * C : nullptr, 3 * C, att1.p, C, Bn, heads, d_head, n_tok, n_tok,
-                long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * C, sc, lse1.p);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(att1.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
-      d.w = b.pw(b.linear_w(tb + ".attn1.to_out.0", C, C, true)); d.bias = lora_bias(tb + ".attn1.to_out.0", C);
-      d.residual = hs0.p; d.ldr = C; d.out_f32 = hs1.p; d.ldo32 = C; b.gemm(d); }
-    // --- cross attention
-    B16T l2 = b.b16(size_t(M) * C);
-    ln(tb + ".norm2", hs1.p, l2.p);
-    B16T q2 = b.b16(size_t(M) * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(l2.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
-      d.w = b.pw(b.linear_w(tb + ".attn2.to_q", C, C, true)); d.out_bf16 = q2.p; d.ldo16 = C; b.gemm(d); }
-    B16T att2 = b.b16(size_t(M) * C);
-    const int kvo = kv_off[tb + ".attn2"], ldkv = kv_total;
-    { const bf16* kv = kv_all.p;
-      b.attention(q2.p, C, kv ? kv + kvo : nullptr, ldkv, kv ? kv + kvo + C : nullptr, ldkv, att2.p, C, Bn, heads, d_head, n_tok, 77, long(n_tok) * C,
-                  long(77) * ldkv, long(n_tok) * C, sc, lse2.p); }
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(att2.p, M, C); d.M = Mi; d.N = C; d.Nw = C;
-      d.w = b.pw(b.linear_w(tb + ".attn2.to_out.0", C, C, true)); d.bias = lora_bias(tb + ".attn2.to_out.0", C);
-      d.residual = hs1.p; d.ldr = C; d.out_f32 = hs2.p; d.ldo32 = C; b.gemm(d); }
-    // --- feed-forward: raw = l3 W1^T + b1 in natural column order (hidden | gate), then the GEGLU pass
-    B16T l3 = b.b16(size_t(M) * C);
-    ln(tb + ".norm3", hs2.p, l3.p);
-    B16T rawff = b.b16(size_t(M) * 8 * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(l3.p, M, C); d.M = Mi; d.N = 8 * C; d.Nw = 8 * C;
-      d.w = b.dpw(b.dlinear_fwd(tb + ".ff.net.0.proj", 8 * C, C)); d.bias = P(tb + ".ff.net.0.proj.bias", 8 * C);
-      d.out_bf16 = rawff.p; d.ldo16 = 8 * C; b.gemm(d); }
-    B16T ff = b.b16(size_t(M) * 4 * C);
-    { const bf16* src = rawff.p; bf16* dst = ff.p; const int Hh = 4 * C;
-      b.emit([=](cudaStream_t st) { return geglu_fwd(src, M, Hh, dst, h16, st); }, false, MADM_KIND_ELEMENTWISE, 0.0, double(M) * C * 24); }
-    B16T hsb = b.b16(size_t(M) * C);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(ff.p, M, 4 * C); d.M = Mi; d.N = C; d.Nw = C;
-      d.w = b.pw(b.linear_w(tb + ".ff.net.2", C, 4 * C, false)); d.bias = P(tb + ".ff.net.2.bias", C);
-      d.residual = hs2.p; d.ldr = C; d.out_bf16 = hsb.p; d.ldo16 = C; b.gemm(d); }
-    Act out = b.act(Bn, H, W, C, true, want_b16 || want_s2d);
-    out.h_s2d = want_s2d;
-    { GemmDesc d; d.seg[0] = Builder::seg_1x1(hsb.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C;
-      if (want_s2d) { d.s2d_H = H; d.s2d_W = W; }
-      d.w = b.pw(b.conv_w(p + ".proj_out", C, C, 1)); d.bias = P(p + ".proj_out.bias", C);
-      d.residual = x.f.p; d.ldr = C; d.out_f32 = out.f.p; d.ldo32 = C; d.out_bf16 = out.h.p; d.ldo16 = C;
-      b.attach_colstats(out, d); b.gemm(d); }
-    // ---- backward
-    const Act xin = x;
-    b.tape.push_back([=]() {
-      const size_t w_po = b.dconv_w(p + ".proj_out", C, C, 1), w_pi = b.dconv_w(p + ".proj_in", C, C, 1);
-      const size_t w_ff2 = b.dlinear_w(tb + ".ff.net.2", C, 4 * C, false), w_ff1 = b.dlinear_w(tb + ".ff.net.0.proj", 8 * C, C, false);
-      const size_t w_o2 = b.dlinear_w(tb + ".attn2.to_out.0", C, C, true), w_q2 = b.dlinear_w(tb + ".attn2.to_q", C, C, true);
-      const size_t w_o1 = b.dlinear_w(tb + ".attn1.to_out.0", C, C, true);
-      const size_t w_qkv = b.dregion("qkv:" + tb, size_t(3) * C * C * 2);
-      b.dlinear_part(tb + ".attn1.to_q", w_qkv, 0, C, C, 3 * C, true);
-      b.dlinear_part(tb + ".attn1.to_k", w_qkv, C, C, C, 3 * C, true);
-      b.dlinear_part(tb + ".attn1.to_v", w_qkv, 2 * C, C, C, 3 * C, true);
-      if (b.mode == LAYOUT) {  // the LoRA factor operands of this block
-        for (const char* m : {".attn1.to_q", ".attn1.to_k", ".attn1.to_v", ".attn1.to_out.0", ".attn2.to_q", ".attn2.to_out.0"}) { b.dlora_a(tb + m, C); b.dlora_bt(tb + m, C); }
-        b.dlora_a(tb + ".attn2.to_k", 768); b.dlora_bt(tb + ".attn2.to_k", C);
-        b.dlora_a(tb + ".attn2.to_v", 768); b.dlora_bt(tb + ".attn2.to_v", C);
-      }
-      if (!out.gr->written) return;
-      // dh = gradient of the block's hidden state (fp32), carried backwards through the three residual branches
-      B16T g16 = b.b16(size_t(M) * C);
-      to16(out.gr->f.p, M * C, g16.p);
-      F32T dh = b.f32(size_t(M) * C);
-      B16T dh16 = b.b16(size_t(M) * C);
-      { GemmDesc d; d.seg[0] = Builder::seg_1x1(g16.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_po);
-        d.out_f32 = dh.p; d.ldo32 = C; d.out_bf16 = dh16.p; d.ldo16 = C; b.gemm(d); }
-      b.free(g16);
-      // --- feed-forward
-      B16T dff = b.b16(size_t(M) * 4 * C);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = 4 * C; d.Nw = 4 * C; d.w = b.dpw(w_ff2); d.out_bf16 = dff.p; d.ldo16 = 4 * C; b.gemm(d); }
-      B16T draw = b.b16(size_t(M) * 8 * C);
-      { const bf16* r = rawff.p; const bf16* dy = dff.p; bf16* dst = draw.p; const int Hh = 4 * C;
-        b.emit([=](cudaStream_t st) { return geglu_bwd(r, dy, M, Hh, dst, h16, st); }); }
-      b.free(dff);
-      B16T dl = b.b16(size_t(M) * C);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(draw.p, M, 8 * C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_ff1); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
-      b.free(draw);
-      auto ln_bwd = [&](const std::string& name, const float* xs) {  // dh += LayerNorm'(xs) dl ; dh16 = 16-bit(dh)
-        const float* g = P(name + ".weight", C); const bf16* dy = dl.p; float* dst = dh.p; bf16* d16 = dh16.p;
-        b.emit([=](cudaStream_t st) -> const char* {
-          return layernorm_bwd(xs, Mi, C, g, 1e-5f, dy, h16, dst, 1, st, d16);  // (writes the 16-bit copy of dh as well)
-        });
-      };
-      ln_bwd(tb + ".norm3", hs2.p);
-      F32T ascr = b.f32(attention_bwd_scratch_floats(Bn, heads, d_head, n_tok, n_tok > 77 ? n_tok : 77) + attention_bwd_scratch_floats(Bn, heads, d_head, n_tok, 77));
-      // --- cross attention
-      B16T datt = b.b16(size_t(M) * C);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o2); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
-      lora_wgrad(tb + ".attn2.to_out.0", att2.p, C, dh16.p, C, M, C, C);
-      B16T dq2 = b.b16(size_t(M) * C);
-      { const bf16* q = q2.p; const bf16* kv = kv_all.p; const bf16* o = att2.p; const bf16* dop = datt.p; bf16* dqp = dq2.p; bf16* dkv = dkv_all.p; float* sp = ascr.p;
-        const float* lse = lse2.p;
-        b.emit([=](cudaStream_t st) {
-          return attention_bwd(q, C, kv + kvo, ldkv, kv + kvo + C, ldkv, o, C, dop, C, dqp, C, dkv + kvo, ldkv, dkv + kvo + C, ldkv, Bn, heads, d_head, n_tok, 77,
-                               long(n_tok) * C, long(77) * ldkv, long(77) * ldkv, long(n_tok) * C, long(n_tok) * C, long(n_tok) * C, long(77) * ldkv,
-                               long(77) * ldkv, sc, sp, h16, st, lse); }); }
-      lora_wgrad(tb + ".attn2.to_q", l2.p, C, dq2.p, C, M, C, C);
-      lora_wgrad(tb + ".attn2.to_k", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo : nullptr, ldkv, long(Bn) * 77, C, 768);
-      lora_wgrad(tb + ".attn2.to_v", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo + C : nullptr, ldkv, long(Bn) * 77, C, 768);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dq2.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_q2); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
-      b.free(dq2);
-      ln_bwd(tb + ".norm2", hs1.p);
-      // --- self attention
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o1); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
-      lora_wgrad(tb + ".attn1.to_out.0", att1.p, C, dh16.p, C, M, C, C);
-      B16T dqkv = b.b16(size_t(M) * 3 * C);
-      { const bf16* q = qkv.p; const bf16* o = att1.p; const bf16* dop = datt.p; bf16* dq = dqkv.p; float* sp = ascr.p;
-        const float* lse = lse1.p;
-        b.emit([=](cudaStream_t st) {
-          return attention_bwd(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, o, C, dop, C, dq, 3 * C, dq + C, 3 * C, dq + 2 * C, 3 * C, Bn, heads, d_head, n_tok, n_tok,
-                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * C, long(n_tok) * C, long(n_tok) * 3 * C,
-                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, sc, sp, h16, st, lse); }); }
-      b.free(datt);
-      lora_wgrad(tb + ".attn1.to_q", l1.p, C, dqkv.p, 3 * C, M, C, C);
-      lora_wgrad(tb + ".attn1.to_k", l1.p, C, dqkv.p ? dqkv.p + C : nullptr, 3 * C, M, C, C);
-      lora_wgrad(tb + ".attn1.to_v", l1.p, C, dqkv.p ? dqkv.p + 2 * C : nullptr, 3 * C, M, C, C);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dqkv.p, M, 3 * C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_qkv); d.out_bf16 = dl.p; d.ldo16 = C; b.gemm(d); }
-      b.free(dqkv); b.free(ascr);
-      ln_bwd(tb + ".norm1", hs0.p);
-      // --- proj_in, GroupNorm; the block's residual adds d(out) to d(x)
-      if (Builder::wants_grad(xin)) {
-        B16T dn = b.b16(size_t(M) * C);
-        { GemmDesc d; d.seg[0] = Builder::seg_1x1(dh16.p, Bn, H, W, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_pi); d.out_bf16 = dn.p; d.ldo16 = C; b.gemm(d); }
-        int acc = 0;
-        float* dx = b.grad(xin, &acc);
-        b.groupnorm_bwd(xin, nullptr, false, sn, nullptr, p + ".norm", 1e-6f, ACT_NONE, dn.p, out.gr->f.p, nullptr, dx, acc, nullptr, 0, nullptr, nullptr);
-        b.free(dn);
-      }
-      b.free(dl); b.free(dh16); b.free(dh);
-    });
-    return out;
-  }
-
-  Act downsample_train(const std::string& p, const Act& x) {
-    const int Bn = x.B, H = x.H, W = x.W, C = x.C;
-    if (!x.h_s2d) b.fail(MADM_EINVAL, "downsample_train: the producer must write the space-to-depth operand");
-    Act out = b.act(Bn, H / 2, W / 2, C, true, false);
-    { GemmDesc d; d.seg[0] = Builder::seg_s2(x.h.p, Bn, H / 2, W / 2, C, /*pad1=*/true); d.M = int(out.M()); d.N = C; d.Nw = C;
-      d.w = b.pw(b.conv_w(p + ".conv", C, C, 9)); d.bias = P(p + ".conv.bias", C); d.out_f32 = out.f.p; d.ldo32 = C;
-      b.attach_colstats(out, d); b.gemm(d); }
-    const Act xin = x;
-    b.tape.push_back([=]() {
-      const size_t w = b.dconv_w(p + ".conv", C, C, 9);
-      if (!out.gr->written || !Builder::wants_grad(xin)) return;
-      // input gradient of the stride-2 conv: zero-stuff d(out) onto the input grid, then the stride-1 dgrad GEMM with mirrored taps
-      const long Mo = out.M(), Mx = xin.M();
-      B16T g16 = b.b16(size_t(Mo) * C);
-      to16(out.gr->f.p, Mo * C, g16.p);
-      B16T z = b.b16(size_t(Mx) * C);
-      { const bf16* src = g16.p; bf16* dst = z.p; b.emit([=](cudaStream_t st) { return zero_stuff2x(src, Bn, H / 2, W / 2, C, dst, st); }); }
-      int acc = 0;
-      float* dx = b.grad(xin, &acc);
-      { GemmDesc d; d.seg[0] = Builder::seg_3x3(z.p, Bn, H, W, C); d.M = int(Mx); d.N = C; d.Nw = C; d.w = b.dpw(w);
-        if (acc) { d.residual = dx; d.ldr = C; }
-        d.out_f32 = dx; d.ldo32 = C; b.gemm(d); }
-      b.free(z); b.free(g16);
-    });
-    return out;
-  }
-
-  Act upsample_train(const std::string& p, const Act& x) {
-    const int Bn = x.B, H = x.H, W = x.W, C = x.C;
-    B16T up = b.b16(size_t(x.M()) * 4 * C);
-    { const float* src = x.f.p; bf16* dst = up.p; const int h16 = f16();
-      b.emit([=](cudaStream_t st) { return upsample_nearest2x(src, Bn, H, W, C, dst, h16, st); }, false, MADM_KIND_ELEMENTWISE, 0.0, double(x.M()) * C * 12); }
-    Act out = b.act(Bn, 2 * H, 2 * W, C, true, false);
-    { GemmDesc d; d.seg[0] = Builder::seg_3x3(up.p, Bn, 2 * H, 2 * W, C); d.M = int(out.M()); d.N = C; d.Nw = C;
-      d.w = b.pw(b.conv_w(p + ".conv", C, C, 9)); d.bias = P(p + ".conv.bias", C); d.out_f32 = out.f.p; d.ldo32 = C;
-      b.attach_colstats(out, d); b.gemm(d); }
-    const Act xin = x;
-    b.tape.push_back([=]() {
-      const size_t w = b.dconv_w(p + ".conv", C, C, 9);
-      if (!out.gr->written || !Builder::wants_grad(xin)) return;
-      const long Mo = out.M();
-      B16T g16 = b.b16(size_t(Mo) * C);
-      to16(out.gr->f.p, Mo * C, g16.p);
-      F32T dup = b.f32(size_t(Mo) * C);
-      { GemmDesc d; d.seg[0] = Builder::seg_3x3(g16.p, Bn, 2 * H, 2 * W, C); d.M = int(Mo); d.N = C; d.Nw = C; d.w = b.dpw(w);
-        d.out_f32 = dup.p; d.ldo32 = C; b.gemm(d); }
-      int acc = 0;
-      float* dx = b.grad(xin, &acc);
-      { const float* src = dup.p; b.emit([=](cudaStream_t st) { return sum2x2(src, Bn, H, W, C, dx, acc, st); }); }
-      b.free(dup); b.free(g16);
-    });
-    return out;
-  }
-
-  // =========================================================================== UNet, training forward (+ tape)
-  void build_unet_train() {
-    b.cur_stage = MADM_STAGE_UNET;
-    const int Bn = b.B;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
-    const int h16 = f16();
-    F32T noisy = b.f32(size_t(Bn) * 4096 * 4);
-    B16T col = b.b16(size_t(Bn) * 4096 * 64);
-    if (dry()) { b.emit(nullptr); b.emit(nullptr); }
-    else {
-      const float* lat = latents.p; float* nz = noisy.p; bf16* cdst = col.p; const float* ac = b.ctx->alphas_cumprod;
-      b.emit([=](cudaStream_t st) -> const char* {
-        if (io->a.noisy_latents_in) return nchw_to_nhwc4(io->a.noisy_latents_in, Bn, 4096, nz, st);
-        return qsample(lat, io->a.shared_noise, io->a.timesteps, ac, Bn, 4096, nz, io->a.noisy_latents, st);
-      });
-      b.emit([=](cudaStream_t st) { return latent_im2col(nz, Bn, 64, 64, cdst, h16, st); });
-    }
-    // ---- time embedding
-    B16T sinus = b.b16(size_t(Bn) * 320);
-    if (dry()) b.emit(nullptr);
-    else { bf16* dst = sinus.p; b.emit([=](cudaStream_t st) { return timestep_sinusoid(io->a.timesteps, Bn, dst, h16, st); }); }
-    B16T e1 = b.b16(size_t(Bn) * 1280);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(sinus.p, Bn, 320); d.M = Bn; d.N = 1280; d.Nw = 1280;
-      d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_1", 1280, 320, false)); d.bias = P(kUnet + "time_embedding.linear_1.bias", 1280);
-      d.act = ACT_SILU; d.out_bf16 = e1.p; d.ldo16 = 1280; b.gemm(d); }
-    emb_saved = b.f32(size_t(Bn) * 1280);
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(e1.p, Bn, 1280); d.M = Bn; d.N = 1280; d.Nw = 1280;
-      d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_2", 1280, 1280, false)); d.bias = P(kUnet + "time_embedding.linear_2.bias", 1280);
-      d.out_f32 = emb_saved.p; d.ldo32 = 1280; b.gemm(d); }
-    B16T emb_act = b.b16(size_t(Bn) * 1280);
-    if (dry()) b.emit(nullptr);
-    else { const float* src = emb_saved.p; bf16* dst = emb_act.p;
-      b.emit([=](cudaStream_t st) { return f32_to_bf16(src, io->a.cond_emb, long(Bn) * 1280, ACT_SILU, dst, nullptr, h16, st); }); }
-    temb_all = b.f32(size_t(Bn) * temb_total);
-    { const size_t reg = b.region("temb_w", size_t(temb_total) * 1280 * 2);
-      const size_t breg = b.region("temb_b", size_t(temb_total) * 4);
-      for (auto& l : temb_layers) {
-        b.linear_part(l.first + ".time_emb_proj", reg, temb_off[l.first], l.second, 1280, false);
-        b.f32_part(l.first + ".time_emb_proj.bias", breg, temb_off[l.first], l.second);
-      }
-      GemmDesc d; d.seg[0] = Builder::seg_plain(emb_act.p, Bn, 1280); d.M = Bn; d.N = temb_total; d.Nw = temb_total; d.w = b.pw(reg);
-      d.bias = b.pf(breg); d.out_f32 = temb_all.p; d.ldo32 = temb_total; b.gemm(d); }
-    // ---- cross-attention K/V
-    ctx16_saved = b.b16(size_t(Bn) * 77 * 768);
-    if (dry()) b.emit(nullptr);
-    else { bf16* dst = ctx16_saved.p;
-      b.emit([=](cudaStream_t st) { return f32_to_bf16(io->a.cond_inputs, nullptr, long(Bn) * 77 * 768, ACT_NONE, dst, nullptr, h16, st); }); }
-    kv_all = b.b16(size_t(Bn) * 77 * kv_total);
-    { const size_t reg = b.region("xattn_kv", size_t(kv_total) * 768 * 2);
-      for (auto& l : xattn_layers) {
-        b.linear_part(l.first + ".to_k", reg, kv_off[l.first], l.second, 768, true);
-        b.linear_part(l.first + ".to_v", reg, kv_off[l.first] + l.second, l.second, 768, true);
-      }
-      GemmDesc d; d.seg[0] = Builder::seg_plain(ctx16_saved.p, long(Bn) * 77, 768); d.M = Bn * 77; d.N = kv_total; d.Nw = kv_total; d.w = b.pw(reg);
-      d.out_bf16 = kv_all.p; d.ldo16 = kv_total; b.gemm(d); }
-    d_temb_all = b.f32(size_t(Bn) * temb_total);
-    dkv_all = b.b16(size_t(Bn) * 77 * kv_total);
-    // ---- backward of the prologue (runs last): time path -> d(cond_emb), stacked K/V projections -> d(cond_inputs)
-    b.tape.push_back([=]() {
-      const size_t wt = b.dregion("temb_w", size_t(temb_total) * 1280 * 2);
-      for (auto& l : temb_layers) b.dlinear_part(l.first + ".time_emb_proj", wt, temb_off[l.first], l.second, 1280, temb_total, false);
-      const size_t wk = b.dregion("xattn_kv", size_t(kv_total) * 768 * 2);
-      for (auto& l : xattn_layers) {
-        b.dlinear_part(l.first + ".to_k", wk, kv_off[l.first], l.second, 768, kv_total, true);
-        b.dlinear_part(l.first + ".to_v", wk, kv_off[l.first] + l.second, l.second, 768, kv_total, true);
-      }
-      const float inv = 1.0f / b.loss_scale;
-      {  // d(emb + cond_emb) = (d_temb_all W_temb) * silu'(emb + cond_emb)
-        B16T dt16 = b.b16(size_t(Bn) * temb_total);
-        to16(d_temb_all.p, long(Bn) * temb_total, dt16.p);
-        F32T dact = b.f32(size_t(Bn) * 1280);
-        { GemmDesc d; d.seg[0] = Builder::seg_plain(dt16.p, Bn, temb_total); d.M = Bn; d.N = 1280; d.Nw = 1280; d.w = b.dpw(wt);
-          d.out_f32 = dact.p; d.ldo32 = 1280; b.gemm(d); }
-        if (dry()) b.emit(nullptr);
-        else { const float* da = dact.p; const float* em = emb_saved.p;
-          b.emit([=](cudaStream_t st) -> const char* {
-            if (!io->b.d_cond_emb) return nullptr;
-            if (!io->b.cond_emb) return "madm_backward: cond_emb is required for d_cond_emb";
-            return temb_silu_bwd(da, em, io->b.cond_emb, long(Bn) * 1280, inv, io->b.d_cond_emb, st); }); }
-        b.free(dact); b.free(dt16);
-      }
-      {  // d(cond_inputs) = dkv_all W_kv : fp32 [B*77, 768] into a scratch, copied out if the caller asked for it
-        F32T dc = b.f32(size_t(Bn) * 77 * 768);
-        { GemmDesc d; d.seg[0] = Builder::seg_plain(dkv_all.p, long(Bn) * 77, kv_total); d.M = Bn * 77; d.N = 768; d.Nw = 768; d.w = b.dpw(wk);
-          d.out_f32 = dc.p; d.ldo32 = 768; b.gemm(d); }
-        if (dry()) b.emit(nullptr);
-        else { const float* src = dc.p; const long n = long(Bn) * 77 * 768;
-          b.emit([=](cudaStream_t st) -> const char* {
-            if (!io->b.d_cond_inputs) return nullptr;
-            return scale_copy_f32(src, n, inv, io->b.d_cond_inputs, st); }); }
-        b.free(dc);
-      }
-    });
-    // ---- conv_in (nothing trainable upstream: its output stops the gradient)
-    Act x = b.act(Bn, 64, 64, 320, true, false);
-    x.gr->stop = true;
-    { GemmDesc d; d.seg[0] = Builder::seg_plain(col.p, long(Bn) * 4096, 64); d.M = Bn * 4096; d.N = 320; d.Nw = 320;
-      d.w = b.pw(b.conv_w(kUnet + "conv_in", 320, 4, 9, /*Cpad=*/4)); d.bias = P(kUnet + "conv_in.bias", 320); d.out_f32 = x.f.p; d.ldo32 = 320;
-      b.attach_colstats(x, d);
-      b.gemm(d, 2.0 * double(d.M) * 320 * 36); }
-    std::vector<Act> skips;
-    skips.push_back(x);
-    const int ch[4] = {320, 640, 1280, 1280};
-    for (int i = 0; i < 4; ++i) {
-      const std::string blk = kUnet + "down_blocks." + std::to_string(i);
-      for (int j = 0; j < 2; ++j) {
-        Act y = resblock_train(blk + ".resnets." + std::to_string(j), x, nullptr, ch[i], false);
-        if (i < 3) y = transformer_train(blk + ".attentions." + std::to_string(j), y, false, /*want_s2d=*/j == 1);
-        x = y;
-        skips.push_back(x);
-      }
-      if (i < 3) { x = downsample_train(blk + ".downsamplers.0", x); skips.push_back(x); }
-    }
-    {
-      Act y = resblock_train(kUnet + "mid_block.resnets.0", x, nullptr, 1280, false);
-      Act z = transformer_train(kUnet + "mid_block.attentions.0", y, false);
-      x = resblock_train(kUnet + "mid_block.resnets.1", z, nullptr, 1280, false);
-    }
-    const int rev[4] = {1280, 1280, 640, 320};
-    int idx = 0;
-    for (int i = 0; i < 4; ++i) {
-      const std::string blk = kUnet + "up_blocks." + std::to_string(i);
-      for (int j = 0; j < 3; ++j) {
-        Act skip = skips.back(); skips.pop_back();
-        const bool is_tap = (idx == 5 || idx == 8 || idx == 11);
-        Act y = resblock_train(blk + ".resnets." + std::to_string(j), x, &skip, rev[i], is_tap && i == 0);
-        if (i > 0) y = transformer_train(blk + ".attentions." + std::to_string(j), y, is_tap);
-        x = y;
-        if (is_tap) {
-          const int t = (idx == 5) ? 2 : (idx == 8 ? 1 : 0);
-          unet_tap[t] = x;
-          b.pin(x);
-          nchw_debug(x, 1 + t);
-        }
-        ++idx;
-      }
-      if (i < 3) x = upsample_train(blk + ".upsamplers.0", x);
-    }
-  }
-
-  // =========================================================================== feature projections, training forward (+ tape)
-  void build_proj_train() {
-    b.cur_stage = MADM_STAGE_PROJ;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
-    const std::string root = "feature_projections.";
-    const Act* taps[4] = {&enc_tap, &unet_tap[0], &unet_tap[1], &unet_tap[2]};
-    const int h16 = f16();
-    for (int i = 0; i < 4; ++i) {
-      const Act x = *taps[i];
-      const std::string p = root + std::to_string(i) + ".0.";
-      const ParamRef* w1 = b.find(p + "conv1.weight"); const ParamRef* w3 = b.find(p + "conv3.weight");
-      if (!w1 || !w3) b.fail(MADM_ENOTFOUND, "parameter not registered: " + p + "conv1.weight / conv3.weight");
-      const int Bn = x.B, H = x.H, W = x.W, Cin = x.C, Cb = int(w1->shape[0]), Cout = int(w3->shape[0]);
-      if (int(w1->shape[1]) != Cin || Cb % 64 != 0 || Cout % 64 != 0 || Cin % 64 != 0) b.fail(MADM_EINVAL, "feature projection " + std::to_string(i) + ": unsupported channels");
-      const long M = x.M();
-      const int HW = H * W;
-      const bool shortcut = Cin != Cout;
-      Act c1 = b.act(Bn, H, W, Cb, false, true);
-      { GemmDesc d; d.seg[0] = Builder::seg_1x1(x.h.p, Bn, H, W, Cin); d.M = int(M); d.N = Cb; d.Nw = Cb;
-        d.w = b.pw(b.conv_w(p + "conv1", Cb, Cin, 1)); d.out_bf16 = c1.h.p; d.ldo16 = Cb; b.attach_colstats(c1, d); b.gemm(d); }
-      B16T a1 = b.b16(size_t(M) * Cb);
-      const Builder::GnSaved s1 = b.groupnorm(c1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, a1.p, nullptr, true);
-      Act c2 = b.act(Bn, H, W, Cb, false, true);
-      { GemmDesc d; d.seg[0] = Builder::seg_3x3(a1.p, Bn, H, W, Cb); d.M = int(M); d.N = Cb; d.Nw = Cb;
-        d.w = b.pw(b.conv_w(p + "conv2", Cb, Cb, 9)); d.out_bf16 = c2.h.p; d.ldo16 = Cb; b.attach_colstats(c2, d); b.gemm(d); }
-      B16T a2 = b.b16(size_t(M) * Cb);
-      const Builder::GnSaved s2 = b.groupnorm(c2, nullptr, p + "conv2.norm", 1e-5f, ACT_RELU, a2.p, nullptr, true);
-      Act c3 = b.act(Bn, H, W, Cout, true, false);
-      { GemmDesc d; d.seg[0] = Builder::seg_1x1(a2.p, Bn, H, W, Cb); d.M = int(M); d.N = Cout; d.Nw = Cout;
-        d.w = b.pw(b.conv_w(p + "conv3", Cout, Cb, 1)); d.out_f32 = c3.f.p; d.ldo32 = Cout; b.attach_colstats(c3, d); b.gemm(d); }
-      Act sc;
-      if (shortcut) {
-        sc = b.act(Bn, H, W, Cout, true, false);
-        GemmDesc d; d.seg[0] = Builder::seg_1x1(x.h.p, Bn, H, W, Cin); d.M = int(M); d.N = Cout; d.Nw = Cout;
-        d.w = b.pw(b.conv_w(p + "shortcut", Cout, Cin, 1)); d.out_f32 = sc.f.p; d.ldo32 = Cout; b.attach_colstats(sc, d); b.gemm(d);
-      }
-      float* st3 = b.new_stats(1);
-      float* sts = shortcut ? b.new_stats(1) : nullptr;
-      auto tail_stats = [&](const Act& t, float* dst) {
-        if (!t.has_cs) b.fail(MADM_EINVAL, "feature projection: fused statistics expected");
-        const float* cst = t.cs; const int nb = HW / t.sr; const int S = groupnorm_colstats_chunks(nb);
-        float* part = b.new_stats(S);
-        b.emit([=](cudaStream_t st) { return groupnorm_colstats_reduce(cst, Cout, nullptr, 0, Bn, nb, part, st); }, false, MADM_KIND_GROUPNORM, 0.0,
-               double(Bn) * nb * Cout * 8);
-        b.emit([=](cudaStream_t st) { return groupnorm_finalize_slabs(part, Bn, S, dst, st); }, false, MADM_KIND_GROUPNORM, 0.0, 0.0);
-      };
-      tail_stats(c3, st3);
-      if (shortcut) tail_stats(sc, sts);
-      const float* g3 = P(p + "conv3.norm.weight", Cout); const float* b3 = P(p + "conv3.norm.bias", Cout);
-      const float* gs = shortcut ? P(p + "shortcut.norm.weight", Cout) : nullptr;
-      const float* bs = shortcut ? P(p + "shortcut.norm.bias", Cout) : nullptr;
-      const float* c3p = c3.f.p; const float* scp = shortcut ? sc.f.p : x.f.p;
-      const double pel = double(Bn) * HW * Cout;
-      if (dry()) b.emit(nullptr);
-      else b.emit([=](cudaStream_t st) -> const char* {
-        float* dst = io->a.out[i];
-        if (!dst) return "madm_extract: output pointer is null";
-        return gn_add_relu_nchw(c3p, st3, g3, b3, scp, sts, gs, bs, 1e-5f, Bn, HW, Cout, dst, st);
-      }, false, MADM_KIND_GROUPNORM, 0.0, pel * 12);
-      // ---- backward
-      b.tape.push_back([=]() {
-        const size_t wd3 = b.dconv_w(p + "conv3", Cout, Cb, 1), wd2 = b.dconv_w(p + "conv2", Cb, Cb, 9);
-        const size_t wd1 = b.dconv_w(p + "conv1", Cb, Cin, 1), wds = shortcut ? b.dconv_w(p + "shortcut", Cout, Cin, 1) : 0;
-        const float S = b.loss_scale, inv = 1.0f / b.loss_scale;
-        const int Mi = int(M);
-        // d(z) = d(out) * (out > 0), NCHW -> NHWC, scaled by the loss scale
-        B16T dz = b.b16(size_t(M) * Cout);
-        if (dry()) b.emit(nullptr);
-        else { bf16* dst = dz.p;
-          b.emit([=](cudaStream_t st) -> const char* {
-            if (!io->b.dout[i] || !io->b.out[i]) return "madm_backward: dout / out pointer is null";
-            return relu_bwd_nchw_to_nhwc16(io->b.dout[i], io->b.out[i], Bn, Cout, HW, S, dst, h16, st); }); }
-        auto wg = [&](const std::string& name, const bf16* dy, int N, const bf16* xx, int K, int taps) {  // weight gradient of one conv
-          float* g = b.grad_buf(p + name + ".weight");
-          if (!g) return;
-          F32T scr = b.f32(wgrad_scratch_floats(Mi, N, K, taps));
-          float* sp = scr.p;
-          const long so_n = taps == 9 ? long(K) * 9 : K, so_k = taps == 9 ? 9 : 1, so_t = taps == 9 ? 1 : 0;
-          b.emit([=](cudaStream_t st) { return wgrad(dy, N, xx, K, Mi, N, K, taps, Bn, H, W, inv, g, so_n, so_k, so_t, sp, h16, st); });
-          b.free(scr);
-        };
-        int acc = 0;
-        float* dtap = Builder::wants_grad(x) ? b.grad(x, &acc) : nullptr;
-        // conv3 branch
-        B16T dc3 = b.b16(size_t(M) * Cout);
-        b.groupnorm_bwd(c3, nullptr, false, Builder::GnSaved(), st3, p + "conv3.norm", 1e-5f, ACT_NONE, dz.p, nullptr, dc3.p, nullptr, 0, nullptr, 0,
-                        b.grad_buf(p + "conv3.norm.weight"), b.grad_buf(p + "conv3.norm.bias"));
-        wg("conv3", dc3.p, Cout, a2.p, Cb, 1);
-        B16T da2 = b.b16(size_t(M) * Cb);
-        { GemmDesc d; d.seg[0] = Builder::seg_1x1(dc3.p, Bn, H, W, Cout); d.M = Mi; d.N = Cb; d.Nw = Cb; d.w = b.dpw(wd3); d.out_bf16 = da2.p; d.ldo16 = Cb; b.gemm(d); }
-        b.free(dc3);
-        B16T dc2 = b.b16(size_t(M) * Cb);
-        b.groupnorm_bwd(c2, nullptr, true, s2, nullptr, p + "conv2.norm", 1e-5f, ACT_RELU, da2.p, nullptr, dc2.p, nullptr, 0, nullptr, 0,
-                        b.grad_buf(p + "conv2.norm.weight"), b.grad_buf(p + "conv2.norm.bias"));
-        b.free(da2);
-        wg("conv2", dc2.p, Cb, a1.p, Cb, 9);
-        B16T da1 = b.b16(size_t(M) * Cb);
-        { GemmDesc d; d.seg[0] = Builder::seg_3x3(dc2.p, Bn, H, W, Cb); d.M = Mi; d.N = Cb; d.Nw = Cb; d.w = b.dpw(wd2); d.out_bf16 = da1.p; d.ldo16 = Cb; b.gemm(d); }
-        b.free(dc2);
-        B16T dc1 = b.b16(size_t(M) * Cb);
-        b.groupnorm_bwd(c1, nullptr, true, s1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, da1.p, nullptr, dc1.p, nullptr, 0, nullptr, 0,
-                        b.grad_buf(p + "conv1.norm.weight"), b.grad_buf(p + "conv1.norm.bias"));
-        b.free(da1);
-        wg("conv1", dc1.p, Cb, x.h.p, Cin, 1);
-        if (dtap) {
-          GemmDesc d; d.seg[0] = Builder::seg_1x1(dc1.p, Bn, H, W, Cb); d.M = Mi; d.N = Cin; d.Nw = Cin; d.w = b.dpw(wd1);
-          if (acc) { d.residual = dtap; d.ldr = Cin; }
-          d.out_f32 = dtap; d.ldo32 = Cin; b.gemm(d);
-          acc = 1;
-        }
-        b.free(dc1);
-        if (shortcut) {
-          B16T dsc = b.b16(size_t(M) * Cout);
-          b.groupnorm_bwd(sc, nullptr, false, Builder::GnSaved(), sts, p + "shortcut.norm", 1e-5f, ACT_NONE, dz.p, nullptr, dsc.p, nullptr, 0, nullptr, 0,
-                          b.grad_buf(p + "shortcut.norm.weight"), b.grad_buf(p + "shortcut.norm.bias"));
-          wg("shortcut", dsc.p, Cout, x.h.p, Cin, 1);
-          if (dtap) {
-            GemmDesc d; d.seg[0] = Builder::seg_1x1(dsc.p, Bn, H, W, Cout); d.M = Mi; d.N = Cin; d.Nw = Cin; d.w = b.dpw(wds);
-            if (acc) { d.residual = dtap; d.ldr = Cin; }
-            d.out_f32 = dtap; d.ldo32 = Cin; b.gemm(d);
-          }
-          b.free(dsc);
-        }
-        b.free(dz);
-      });
     }
   }
 
@@ -1714,13 +1320,13 @@ struct Model {
     { GemmDesc d; d.seg[0] = Builder::seg_plain(sinus.p, Bn, 320); d.M = Bn; d.N = 1280; d.Nw = 1280;
       d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_1", 1280, 320, false)); d.bias = P(kUnet + "time_embedding.linear_1.bias", 1280);
       d.act = ACT_SILU; d.out_bf16 = e1.p; d.ldo16 = 1280; b.gemm(d); }
-    F32T emb = b.f32(size_t(Bn) * 1280);
+    emb_saved = b.f32(size_t(Bn) * 1280);
     { GemmDesc d; d.seg[0] = Builder::seg_plain(e1.p, Bn, 1280); d.M = Bn; d.N = 1280; d.Nw = 1280;
       d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_2", 1280, 1280, false)); d.bias = P(kUnet + "time_embedding.linear_2.bias", 1280);
-      d.out_f32 = emb.p; d.ldo32 = 1280; b.gemm(d); }
+      d.out_f32 = emb_saved.p; d.ldo32 = 1280; b.gemm(d); }
     B16T emb_act = b.b16(size_t(Bn) * 1280);
     if (dry()) b.emit(nullptr);
-    else { const float* src = emb.p; bf16* dst = emb_act.p; const int h16 = f16();
+    else { const float* src = emb_saved.p; bf16* dst = emb_act.p; const int h16 = f16();
       b.emit([=](cudaStream_t st) { return f32_to_bf16(src, io->a.cond_emb, long(Bn) * 1280, ACT_SILU, dst, nullptr, h16, st); }); }
     temb_all = b.f32(size_t(Bn) * temb_total);
     { const size_t reg = b.region("temb_w", size_t(temb_total) * 1280 * 2);
@@ -1731,11 +1337,11 @@ struct Model {
       }
       GemmDesc d; d.seg[0] = Builder::seg_plain(emb_act.p, Bn, 1280); d.M = Bn; d.N = temb_total; d.Nw = temb_total; d.w = b.pw(reg);
       d.bias = b.pf(breg); d.out_f32 = temb_all.p; d.ldo32 = temb_total; b.gemm(d); }
-    b.free(sinus); b.free(e1); b.free(emb); b.free(emb_act);
+    b.free(sinus); b.free(e1); b.free(emb_saved); b.free(emb_act);
     // ---- cross-attention K/V of every transformer block in one GEMM
-    B16T ctx16 = b.b16(size_t(Bn) * 77 * 768);
+    ctx16_saved = b.b16(size_t(Bn) * 77 * 768);
     if (dry()) b.emit(nullptr);
-    else { bf16* dst = ctx16.p; const int h16 = f16();
+    else { bf16* dst = ctx16_saved.p; const int h16 = f16();
       b.emit([=](cudaStream_t st) { return f32_to_bf16(io->a.cond_inputs, nullptr, long(Bn) * 77 * 768, ACT_NONE, dst, nullptr, h16, st); }); }
     kv_all = b.b16(size_t(Bn) * 77 * kv_total);
     { const size_t reg = b.region("xattn_kv", size_t(kv_total) * 768 * 2);
@@ -1743,11 +1349,52 @@ struct Model {
         b.linear_part(l.first + ".to_k", reg, kv_off[l.first], l.second, 768, true);
         b.linear_part(l.first + ".to_v", reg, kv_off[l.first] + l.second, l.second, 768, true);
       }
-      GemmDesc d; d.seg[0] = Builder::seg_plain(ctx16.p, long(Bn) * 77, 768); d.M = Bn * 77; d.N = kv_total; d.Nw = kv_total; d.w = b.pw(reg);
+      GemmDesc d; d.seg[0] = Builder::seg_plain(ctx16_saved.p, long(Bn) * 77, 768); d.M = Bn * 77; d.N = kv_total; d.Nw = kv_total; d.w = b.pw(reg);
       d.out_bf16 = kv_all.p; d.ldo16 = kv_total; b.gemm(d); }
-    b.free(ctx16);
-    // ---- conv_in
+    b.free(ctx16_saved);
+    if (b.recording()) {
+      d_temb_all = b.f32(size_t(Bn) * temb_total);
+      dkv_all = b.b16(size_t(Bn) * 77 * kv_total);
+      // ---- backward of the prologue (runs last): time path -> d(cond_emb), stacked K/V projections -> d(cond_inputs)
+      b.tape.push_back([=]() {
+        const size_t wt = b.dregion("temb_w", size_t(temb_total) * 1280 * 2);
+        for (auto& l : temb_layers) b.dlinear_part(l.first + ".time_emb_proj", wt, temb_off[l.first], l.second, 1280, temb_total, false);
+        const size_t wk = b.dregion("xattn_kv", size_t(kv_total) * 768 * 2);
+        for (auto& l : xattn_layers) {
+          b.dlinear_part(l.first + ".to_k", wk, kv_off[l.first], l.second, 768, kv_total, true);
+          b.dlinear_part(l.first + ".to_v", wk, kv_off[l.first] + l.second, l.second, 768, kv_total, true);
+        }
+        const float inv = 1.0f / b.loss_scale;
+        {  // d(emb + cond_emb) = (d_temb_all W_temb) * silu'(emb + cond_emb)
+          B16T dt16 = b.b16(size_t(Bn) * temb_total);
+          to16(d_temb_all.p, long(Bn) * temb_total, dt16.p);
+          F32T dact = b.f32(size_t(Bn) * 1280);
+          { GemmDesc d; d.seg[0] = Builder::seg_plain(dt16.p, Bn, temb_total); d.M = Bn; d.N = 1280; d.Nw = 1280; d.w = b.dpw(wt);
+            d.out_f32 = dact.p; d.ldo32 = 1280; b.gemm(d); }
+          if (dry()) b.emit(nullptr);
+          else { const float* da = dact.p; const float* em = emb_saved.p;
+            b.emit([=](cudaStream_t st) -> const char* {
+              if (!io->b.d_cond_emb) return nullptr;
+              if (!io->b.cond_emb) return "madm_backward: cond_emb is required for d_cond_emb";
+              return temb_silu_bwd(da, em, io->b.cond_emb, long(Bn) * 1280, inv, io->b.d_cond_emb, st); }); }
+          b.free(dact); b.free(dt16);
+        }
+        {  // d(cond_inputs) = dkv_all W_kv : fp32 [B*77, 768] into a scratch, copied out if the caller asked for it
+          F32T dc = b.f32(size_t(Bn) * 77 * 768);
+          { GemmDesc d; d.seg[0] = Builder::seg_plain(dkv_all.p, long(Bn) * 77, kv_total); d.M = Bn * 77; d.N = 768; d.Nw = 768; d.w = b.dpw(wk);
+            d.out_f32 = dc.p; d.ldo32 = 768; b.gemm(d); }
+          if (dry()) b.emit(nullptr);
+          else { const float* src = dc.p; const long n = long(Bn) * 77 * 768;
+            b.emit([=](cudaStream_t st) -> const char* {
+              if (!io->b.d_cond_inputs) return nullptr;
+              return scale_copy_f32(src, n, inv, io->b.d_cond_inputs, st); }); }
+          b.free(dc);
+        }
+      });
+    }
+    // ---- conv_in (nothing trainable upstream: its output stops the gradient)
     Act x = b.act(Bn, 64, 64, 320, true, false);
+    if (b.recording()) x.gr->stop = true;
     { GemmDesc d; d.seg[0] = Builder::seg_plain(col.p, long(Bn) * 4096, 64); d.M = Bn * 4096; d.N = 320; d.Nw = 320;
       d.w = b.pw(b.conv_w(kUnet + "conv_in", 320, 4, 9, /*Cpad=*/4)); d.bias = P(kUnet + "conv_in.bias", 320); d.out_f32 = x.f.p; d.ldo32 = 320;
       b.attach_colstats(x, d);
@@ -1920,6 +1567,7 @@ struct Model {
       b.cur_branch = proj_streams() ? 1 + i : 0;
       const Act& x = *taps[i];
       const std::string p = root + std::to_string(i) + ".0.";
+      const int h16 = f16();
       const ParamRef* w1 = b.find(p + "conv1.weight"); const ParamRef* w3 = b.find(p + "conv3.weight");
       if (!w1 || !w3) b.fail(MADM_ENOTFOUND, "parameter not registered: " + p + "conv1.weight / conv3.weight");
       const int Bn = x.B, H = x.H, W = x.W, Cin = x.C, Cb = int(w1->shape[0]), Cout = int(w3->shape[0]);
@@ -1929,7 +1577,7 @@ struct Model {
       // The 3-channel decoded image of the s0 variant: its K = 3 1x1 convs are not GEMMs.  conv1 -> GN -> ReLU is one elementwise pass with
       // GroupNorm statistics derived from the image's moments, and the shortcut branch is recomputed inside the final pass (norm.cu).
       const bool rgb3 = Cin == 3;
-      if (Cin < 64 && !rgb3) b.fail(MADM_EINVAL, "feature projection " + std::to_string(i) + ": input channels must be 3 or a multiple of 64");
+      if (Cin % 64 != 0 && !rgb3) b.fail(MADM_EINVAL, "feature projection " + std::to_string(i) + ": input channels must be 3 or a multiple of 64");
       F32T mom, coef1, coefs;
       const float* img4 = x.f.p;
       if (rgb3) {
@@ -1948,14 +1596,16 @@ struct Model {
       }
       // every GroupNorm of the bottleneck takes its statistics from the producing GEMM's epilogue
       B16T a1 = b.b16(size_t(M) * Cb);
+      Act c1;
+      Builder::GnSaved s1;
       if (rgb3) {
-        bf16* a1p = a1.p; const float* c1p = coef1.p; const int HWi = H * W; const int h16 = f16();
+        bf16* a1p = a1.p; const float* c1p = coef1.p; const int HWi = H * W;
         b.emit([=](cudaStream_t st) { return c3_conv_gn_relu(img4, c1p, Bn, HWi, Cb, a1p, h16, st); }, false, MADM_KIND_GROUPNORM, 0.0, double(M) * (16 + 2.0 * Cb));
       } else {
-        Act c1 = b.act(Bn, H, W, Cb, false, true);
+        c1 = b.act(Bn, H, W, Cb, false, true);
         { GemmDesc d; d.seg[0] = Builder::seg_1x1(x.h.p, Bn, H, W, Cin); d.M = int(M); d.N = Cb; d.Nw = Cb;
           d.w = b.pw(b.conv_w(p + "conv1", Cb, Cin, 1)); d.out_bf16 = c1.h.p; d.ldo16 = Cb; b.attach_colstats(c1, d); b.gemm(d); }
-        b.groupnorm(c1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, a1.p, nullptr, /*in16=*/true);
+        s1 = b.groupnorm(c1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, a1.p, nullptr, /*in16=*/true);
         b.free(c1);
       }
       Act c2 = b.act(Bn, H, W, Cb, false, true);
@@ -1963,7 +1613,7 @@ struct Model {
         d.w = b.pw(b.conv_w(p + "conv2", Cb, Cb, 9)); d.out_bf16 = c2.h.p; d.ldo16 = Cb; b.attach_colstats(c2, d); b.gemm(d); }
       b.free(a1);
       B16T a2 = b.b16(size_t(M) * Cb);
-      b.groupnorm(c2, nullptr, p + "conv2.norm", 1e-5f, ACT_RELU, a2.p, nullptr, /*in16=*/true);
+      const Builder::GnSaved s2 = b.groupnorm(c2, nullptr, p + "conv2.norm", 1e-5f, ACT_RELU, a2.p, nullptr, /*in16=*/true);
       b.free(c2);
       Act c3 = b.act(Bn, H, W, Cout, true, false);
       { GemmDesc d; d.seg[0] = Builder::seg_1x1(a2.p, Bn, H, W, Cb); d.M = int(M); d.N = Cout; d.Nw = Cout;
@@ -2015,6 +1665,74 @@ struct Model {
       b.free(c3);
       if (shortcut && !rgb3) b.free(sc);
       if (rgb3) { b.free(mom); b.free(coef1); b.free(coefs); }
+      if (b.recording()) {
+        // ---- backward
+        b.tape.push_back([=]() {
+          const size_t wd3 = b.dconv_w(p + "conv3", Cout, Cb, 1), wd2 = b.dconv_w(p + "conv2", Cb, Cb, 9);
+          const size_t wd1 = b.dconv_w(p + "conv1", Cb, Cin, 1), wds = shortcut ? b.dconv_w(p + "shortcut", Cout, Cin, 1) : 0;
+          const float S = b.loss_scale, inv = 1.0f / b.loss_scale;
+          const int Mi = int(M);
+          // d(z) = d(out) * (out > 0), NCHW -> NHWC, scaled by the loss scale
+          B16T dz = b.b16(size_t(M) * Cout);
+          if (dry()) b.emit(nullptr);
+          else { bf16* dst = dz.p;
+            b.emit([=](cudaStream_t st) -> const char* {
+              if (!io->b.dout[i] || !io->b.out[i]) return "madm_backward: dout / out pointer is null";
+              return relu_bwd_nchw_to_nhwc16(io->b.dout[i], io->b.out[i], Bn, Cout, HW, S, dst, h16, st); }); }
+          auto wg = [&](const std::string& name, const bf16* dy, int N, const bf16* xx, int K, int taps) {  // weight gradient of one conv
+            float* g = b.grad_buf(p + name + ".weight");
+            if (!g) return;
+            F32T scr = b.f32(wgrad_scratch_floats(Mi, N, K, taps));
+            float* sp = scr.p;
+            const long so_n = taps == 9 ? long(K) * 9 : K, so_k = taps == 9 ? 9 : 1, so_t = taps == 9 ? 1 : 0;
+            b.emit([=](cudaStream_t st) { return wgrad(dy, N, xx, K, Mi, N, K, taps, Bn, H, W, inv, g, so_n, so_k, so_t, sp, h16, st); });
+            b.free(scr);
+          };
+          int acc = 0;
+          float* dtap = Builder::wants_grad(x) ? b.grad(x, &acc) : nullptr;
+          // conv3 branch
+          B16T dc3 = b.b16(size_t(M) * Cout);
+          b.groupnorm_bwd(c3, nullptr, false, Builder::GnSaved(), st3, p + "conv3.norm", 1e-5f, ACT_NONE, dz.p, nullptr, dc3.p, nullptr, 0, nullptr, 0,
+                          b.grad_buf(p + "conv3.norm.weight"), b.grad_buf(p + "conv3.norm.bias"));
+          wg("conv3", dc3.p, Cout, a2.p, Cb, 1);
+          B16T da2 = b.b16(size_t(M) * Cb);
+          { GemmDesc d; d.seg[0] = Builder::seg_1x1(dc3.p, Bn, H, W, Cout); d.M = Mi; d.N = Cb; d.Nw = Cb; d.w = b.dpw(wd3); d.out_bf16 = da2.p; d.ldo16 = Cb; b.gemm(d); }
+          b.free(dc3);
+          B16T dc2 = b.b16(size_t(M) * Cb);
+          b.groupnorm_bwd(c2, nullptr, true, s2, nullptr, p + "conv2.norm", 1e-5f, ACT_RELU, da2.p, nullptr, dc2.p, nullptr, 0, nullptr, 0,
+                          b.grad_buf(p + "conv2.norm.weight"), b.grad_buf(p + "conv2.norm.bias"));
+          b.free(da2);
+          wg("conv2", dc2.p, Cb, a1.p, Cb, 9);
+          B16T da1 = b.b16(size_t(M) * Cb);
+          { GemmDesc d; d.seg[0] = Builder::seg_3x3(dc2.p, Bn, H, W, Cb); d.M = Mi; d.N = Cb; d.Nw = Cb; d.w = b.dpw(wd2); d.out_bf16 = da1.p; d.ldo16 = Cb; b.gemm(d); }
+          b.free(dc2);
+          B16T dc1 = b.b16(size_t(M) * Cb);
+          b.groupnorm_bwd(c1, nullptr, true, s1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, da1.p, nullptr, dc1.p, nullptr, 0, nullptr, 0,
+                          b.grad_buf(p + "conv1.norm.weight"), b.grad_buf(p + "conv1.norm.bias"));
+          b.free(da1);
+          wg("conv1", dc1.p, Cb, x.h.p, Cin, 1);
+          if (dtap) {
+            GemmDesc d; d.seg[0] = Builder::seg_1x1(dc1.p, Bn, H, W, Cb); d.M = Mi; d.N = Cin; d.Nw = Cin; d.w = b.dpw(wd1);
+            if (acc) { d.residual = dtap; d.ldr = Cin; }
+            d.out_f32 = dtap; d.ldo32 = Cin; b.gemm(d);
+            acc = 1;
+          }
+          b.free(dc1);
+          if (shortcut) {
+            B16T dsc = b.b16(size_t(M) * Cout);
+            b.groupnorm_bwd(sc, nullptr, false, Builder::GnSaved(), sts, p + "shortcut.norm", 1e-5f, ACT_NONE, dz.p, nullptr, dsc.p, nullptr, 0, nullptr, 0,
+                            b.grad_buf(p + "shortcut.norm.weight"), b.grad_buf(p + "shortcut.norm.bias"));
+            wg("shortcut", dsc.p, Cout, x.h.p, Cin, 1);
+            if (dtap) {
+              GemmDesc d; d.seg[0] = Builder::seg_1x1(dsc.p, Bn, H, W, Cout); d.M = Mi; d.N = Cin; d.Nw = Cin; d.w = b.dpw(wds);
+              if (acc) { d.residual = dtap; d.ldr = Cin; }
+              d.out_f32 = dtap; d.ldo32 = Cin; b.gemm(d);
+            }
+            b.free(dsc);
+          }
+          b.free(dz);
+        });
+      }
     }
     b.cur_branch = 0;
     b.defer_free = false;
@@ -2133,30 +1851,28 @@ struct Model {
     if (b.train) {  // forward that keeps its activations + the backward pass (SURVEY §8 row f-3)
       if (s0()) b.fail(MADM_EINVAL, "training path: the base variant only (the s0 / vae_decoder_loss variant has no backward yet)");
       if (!has_path()) b.fail(MADM_ESTATE, "training path: UNet / VAE parameters are not registered");
-      enumerate_unet();
-      build_vae();
-      if (enc_tap.gr) enc_tap.gr->stop = true;  // the VAE encoder runs without gradient (ldm_diffusers.py:282)
-      build_unet_train();
-      build_proj_train();
-      b.bwd = true;
-      if (dry()) b.emit(nullptr);
-      else { float* dt = d_temb_all.p; bf16* dk = dkv_all.p; const size_t nt = size_t(b.B) * temb_total * 4, nk = size_t(b.B) * 77 * kv_total * 2;
-        b.emit([=](cudaStream_t st) -> const char* {
-          if (cudaMemsetAsync(dt, 0, nt, st) != cudaSuccess || cudaMemsetAsync(dk, 0, nk, st) != cudaSuccess) return "cudaMemsetAsync failed";
-          return nullptr; }); }
-      for (auto it = b.tape.rbegin(); it != b.tape.rend(); ++it) (*it)();
-      b.bwd = false;
-      return;
     }
     if (has_path() || !has_head()) {  // a context that holds only sem_seg_head.* runs the head alone
       enumerate_unet();
       build_vae();
+      if (enc_tap.gr) enc_tap.gr->stop = true;  // training: the VAE encoder runs without gradient (ldm_diffusers.py:282)
       build_proj_early(0);  // the encoder tap's projection overlaps the whole UNet
       build_unet();
       if (s0()) build_dec();
       build_proj();
     }
-    if (has_head()) build_head();
+    if (!b.train) {
+      if (has_head()) build_head();
+      return;
+    }
+    b.bwd = true;
+    if (dry()) b.emit(nullptr);
+    else { float* dt = d_temb_all.p; bf16* dk = dkv_all.p; const size_t nt = size_t(b.B) * temb_total * 4, nk = size_t(b.B) * 77 * kv_total * 2;
+      b.emit([=](cudaStream_t st) -> const char* {
+        if (cudaMemsetAsync(dt, 0, nt, st) != cudaSuccess || cudaMemsetAsync(dk, 0, nk, st) != cudaSuccess) return "cudaMemsetAsync failed";
+        return nullptr; }); }
+    for (auto it = b.tape.rbegin(); it != b.tape.rend(); ++it) (*it)();
+    b.bwd = false;
   }
 };
 
@@ -2191,27 +1907,57 @@ int set_err(madm_ctx* ctx, int code, const std::string& m) {
   return code;
 }
 
-// Runs the traversal in a dry mode; returns workspace bytes (peak + stats region) and op count.
-int dry_run(madm_ctx* ctx, Mode mode, int B, size_t* ws_bytes, int* n_ops, int head_h = 0, int head_w = 0, bool train = false,
-            const std::string& adapter = "") {
-  Builder bld{ctx, mode, B, false};
-  bld.head_h = head_h; bld.head_w = head_w;
-  bld.train = train; bld.adapter = adapter; bld.lora_scale = 1.0f;
+// Runs the model traversal in the builder's mode.
+int traverse(madm_ctx* ctx, Builder& bld) {
   Model m(bld);
   try {
     m.build_all();
   } catch (const BuildError& e) {
     return set_err(ctx, e.code, e.msg);
   }
-  if (ws_bytes) *ws_bytes = bld.peak + ((bld.stats_used * 4 + 1023) & ~size_t(1023)) + 1024;
-  if (n_ops) *n_ops = bld.n_ops;
+  return MADM_OK;
+}
+
+// Bytes of the GroupNorm statistics slots a traversal used; they sit at the start of the workspace, the activations after them.
+size_t stats_region(const Builder& bld) { return (bld.stats_used * 4 + 1023) & ~size_t(1023); }
+
+// Runs the traversal in a dry mode; in SIZE mode returns the workspace bytes (stats region + peak).
+int dry_run(madm_ctx* ctx, Mode mode, int B, size_t* ws_bytes, int head_h = 0, int head_w = 0, bool train = false, const std::string& adapter = "") {
+  Builder bld{ctx, mode, B, false};
+  bld.head_h = head_h; bld.head_w = head_w;
+  bld.train = train; bld.adapter = adapter; bld.lora_scale = 1.0f;
+  const int rc = traverse(ctx, bld);
+  if (rc == MADM_OK && ws_bytes) *ws_bytes = stats_region(bld) + bld.peak + 1024;
+  return rc;
+}
+
+// Emits `plan` (its pointers and workspace already set) with the settings of `cfg`: a SIZE pass of the same traversal sizes the
+// statistics region, then the PLAN pass lays the launches out over the workspace.
+int build_plan(madm_ctx* ctx, const Builder& cfg, Plan* plan) {
+  Builder probe = cfg;
+  probe.mode = SIZE;
+  int rc = traverse(ctx, probe);
+  if (rc != MADM_OK) return rc;
+  plan->stats_off = 0;
+  plan->stats_bytes = stats_region(probe);
+  Builder bld = cfg;
+  bld.mode = PLAN;
+  bld.plan = plan;
+  bld.packed = static_cast<const uint8_t*>(plan->packed);
+  bld.dpacked = static_cast<const uint8_t*>(plan->dpacked);
+  bld.stats_base = reinterpret_cast<float*>(plan->ws);
+  bld.ws = static_cast<uint8_t*>(plan->ws) + plan->stats_bytes;
+  rc = traverse(ctx, bld);
+  if (rc != MADM_OK) return rc;
+  if (plan->stats_bytes + bld.peak > plan->ws_bytes)
+    return set_err(ctx, MADM_ENOMEM, plan->train ? "madm_extract: training workspace too small for plan" : "madm_extract: workspace too small for plan");
   return MADM_OK;
 }
 
 int ensure_layout(madm_ctx* ctx) {
   if (ctx->layout_done) return MADM_OK;
   ctx->pack.clear(); ctx->pack_index.clear(); ctx->packed_bytes = 0;
-  int rc = dry_run(ctx, LAYOUT, 1, nullptr, nullptr);
+  int rc = dry_run(ctx, LAYOUT, 1, nullptr);
   if (rc != MADM_OK) return rc;
   // EMA projection twins share the layout pass (registered only if the caller provided them)
   if (ctx->params.count("ema_feature_projections.0.0.conv1.weight")) {
@@ -2480,7 +2226,7 @@ size_t madm_workspace_bytes_head(madm_ctx* ctx, int32_t B, int32_t head_h, int32
   auto it = ctx->ws_bytes_cache.find(key);
   if (it != ctx->ws_bytes_cache.end()) return it->second;
   size_t bytes = 0;
-  if (dry_run(ctx, SIZE, B, &bytes, nullptr, head_h, head_w) != MADM_OK) return 0;
+  if (dry_run(ctx, SIZE, B, &bytes, head_h, head_w) != MADM_OK) return 0;
   ctx->ws_bytes_cache[key] = bytes;
   return bytes;
 }
@@ -2556,31 +2302,10 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
   if (!plan) {
     std::unique_ptr<Plan> np(new Plan());
     np->B = a->B; np->ema = a->ema != 0; np->packed = a->packed; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
-    Builder bld{ctx, PLAN, a->B, a->ema != 0};
-    bld.head_h = a->head_h; bld.head_w = a->head_w;
-    bld.plan = np.get();
-    bld.packed = static_cast<const uint8_t*>(a->packed);
-    // statistics slots live at the start of the workspace; activations after them
-    size_t total = 0; int nops = 0;
-    {
-      Builder probe{ctx, SIZE, a->B, a->ema != 0};
-      probe.head_h = a->head_h; probe.head_w = a->head_w;
-      Model pm(probe);
-      try { pm.build_all(); } catch (const BuildError& e) { return set_err(ctx, e.code, e.msg); }
-      total = probe.stats_used; nops = probe.n_ops;
-      (void)nops;
-    }
-    np->stats_off = 0;
-    np->stats_bytes = (total * 4 + 1023) & ~size_t(1023);
-    bld.stats_base = reinterpret_cast<float*>(static_cast<uint8_t*>(a->workspace));
-    bld.ws = static_cast<uint8_t*>(a->workspace) + np->stats_bytes;
-    Model m(bld);
-    try {
-      m.build_all();
-    } catch (const BuildError& e) {
-      return set_err(ctx, e.code, e.msg);
-    }
-    if (np->stats_bytes + bld.peak > a->workspace_bytes) return set_err(ctx, MADM_ENOMEM, "madm_extract: workspace too small for plan");
+    Builder cfg{ctx, PLAN, a->B, a->ema != 0};
+    cfg.head_h = a->head_h; cfg.head_w = a->head_w;
+    rc = build_plan(ctx, cfg, np.get());
+    if (rc != MADM_OK) return rc;
     plan = np.get();
     ctx->plans[key] = std::move(np);
   }
@@ -2649,6 +2374,7 @@ namespace {
 int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
   if (a->stages != MADM_STAGE_ALL) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN runs all stages (MADM_STAGE_ALL)");
   if (a->ema) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN with the EMA projections (the teacher runs without gradient)");
+  if (a->flags & MADM_FLAG_OUT_FP16) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_OUT_FP16 with MADM_FLAG_TRAIN (madm_backward reads the fp32 outputs)");
   if (!a->packed_dgrad) return set_err(ctx, MADM_ESTATE, "madm_extract: MADM_FLAG_TRAIN needs packed_dgrad (madm_pack_dgrad_weights)");
   if (!(a->train_loss_scale > 0.f)) return set_err(ctx, MADM_EINVAL, "madm_extract: train_loss_scale must be > 0");
   if (a->B > 8) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN supports B <= 8");
@@ -2671,26 +2397,10 @@ int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
     std::unique_ptr<Plan> np(new Plan());
     np->B = a->B; np->packed = a->packed; np->dpacked = a->packed_dgrad; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
     np->train = true; np->adapter = ad; np->loss_scale = a->train_loss_scale; np->lora_scale = a->train_lora_scale;
-    size_t total = 0;
-    {
-      Builder probe{ctx, SIZE, a->B, false};
-      probe.train = true; probe.adapter = ad; probe.lora_scale = a->train_lora_scale; probe.loss_scale = a->train_loss_scale;
-      Model pm(probe);
-      try { pm.build_all(); } catch (const BuildError& e) { return set_err(ctx, e.code, e.msg); }
-      total = probe.stats_used;
-    }
-    np->stats_off = 0;
-    np->stats_bytes = (total * 4 + 1023) & ~size_t(1023);
-    Builder bld{ctx, PLAN, a->B, false};
-    bld.train = true; bld.adapter = ad; bld.lora_scale = a->train_lora_scale; bld.loss_scale = a->train_loss_scale;
-    bld.plan = np.get();
-    bld.packed = static_cast<const uint8_t*>(a->packed);
-    bld.dpacked = static_cast<const uint8_t*>(a->packed_dgrad);
-    bld.stats_base = reinterpret_cast<float*>(static_cast<uint8_t*>(a->workspace));
-    bld.ws = static_cast<uint8_t*>(a->workspace) + np->stats_bytes;
-    Model m(bld);
-    try { m.build_all(); } catch (const BuildError& e) { return set_err(ctx, e.code, e.msg); }
-    if (np->stats_bytes + bld.peak > a->workspace_bytes) return set_err(ctx, MADM_ENOMEM, "madm_extract: training workspace too small for plan");
+    Builder cfg{ctx, PLAN, a->B, false};
+    cfg.train = true; cfg.adapter = ad; cfg.lora_scale = a->train_lora_scale; cfg.loss_scale = a->train_loss_scale;
+    rc = build_plan(ctx, cfg, np.get());
+    if (rc != MADM_OK) return rc;
     plan = np.get();
     ctx->train_plans[tkey] = std::move(np);
   }
@@ -2709,7 +2419,7 @@ int ensure_dlayout(madm_ctx* ctx) {
   if (rc != MADM_OK) return rc;
   if (ctx->dlayout_done) return MADM_OK;
   ctx->dpack.clear(); ctx->dpack_index.clear(); ctx->dpacked_bytes = 0;
-  rc = dry_run(ctx, LAYOUT, 1, nullptr, nullptr, 0, 0, /*train=*/true);
+  rc = dry_run(ctx, LAYOUT, 1, nullptr, 0, 0, /*train=*/true);
   if (rc != MADM_OK) return rc;
   ctx->dlayout_done = true;
   return MADM_OK;
@@ -2823,7 +2533,7 @@ size_t madm_train_workspace_bytes(madm_ctx* ctx, int32_t B, const char* adapter)
   if (!ctx || B < 1) return 0;
   if (ensure_dlayout(ctx) != MADM_OK) return 0;
   size_t bytes = 0;
-  if (dry_run(ctx, SIZE, B, &bytes, nullptr, 0, 0, /*train=*/true, adapter ? adapter : "") != MADM_OK) return 0;
+  if (dry_run(ctx, SIZE, B, &bytes, 0, 0, /*train=*/true, adapter ? adapter : "") != MADM_OK) return 0;
   return bytes;
 }
 

@@ -52,3 +52,33 @@ def cosine(a, b):
 def max_rel(a, b):
     """max|a-b| / max|b| per tensor (SURVEY §8d parity gates)."""
     return ((a.double() - b.double()).abs().max() / b.double().abs().max()).item()
+
+
+def meta_training_params():
+    """(state_dict name, meta tensor) pairs of the host-only training dry runs: UNet with the LoRA adapters 'default' and 'Depth' (r = 16),
+    VAE encoder, four GN-bottleneck projections (512 / 320 / 640 / 1280 -> 512)."""
+    from madm_b200.sd14_params import BottleneckParams, UNetParams, VAEParams, empty_init
+    with empty_init():
+        unet, vae = UNetParams(device="meta"), VAEParams(device="meta")
+        for name in ("default", "Depth"):
+            unet.add_adapter(SimpleNamespace(r=16, lora_alpha=16, init_lora_weights="gaussian",
+                                             target_modules=["to_k", "to_q", "to_v", "to_out.0"]), name)
+        projs = [BottleneckParams(c, 512, 128, device="meta") for c in (512, 320, 640, 1280)]
+    named = [("feature_extractor.ldm_extractor.unet." + n, p) for n, p in unet.named_parameters()]
+    named += [("feature_extractor.ldm_extractor.vae." + n, p) for n, p in vae.named_parameters()]
+    for i, pr in enumerate(projs):
+        named += [(f"feature_projections.{i}.0." + n, p) for n, p in pr.named_parameters()]
+    return named
+
+
+def tensor_table(items, base):
+    """madm_tensor records of (name, tensor) pairs at fake device addresses base, base + 16, ... (dry runs never dereference them).
+    Returns the array and the encoded names, which must outlive it."""
+    from madm_b200 import _lib
+    arr = (_lib.MadmTensor * len(items))()
+    keep = [n.encode() for n, _ in items]
+    for i, (n, t) in enumerate(items):
+        arr[i].name, arr[i].data, arr[i].ndim = keep[i], base + 16 * i, t.dim()
+        for k, s in enumerate(t.shape):
+            arr[i].shape[k] = s
+    return arr, keep

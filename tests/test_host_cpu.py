@@ -348,48 +348,30 @@ def test_training_plan_dry_runs_without_a_device(monkeypatch):
     on a device-less context (MADM_PLAN_ONLY test hook: nothing can be launched from it).  Checks that the layout / size / plan passes
     of the forward-with-saved-activations + backward traversal agree with each other and scale with the batch."""
     import ctypes as C
-    from types import SimpleNamespace
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from helpers import meta_training_params, tensor_table
     from madm_b200 import _lib
-    from madm_b200.sd14_params import BottleneckParams, UNetParams, VAEParams, empty_init
     monkeypatch.setenv("MADM_PLAN_ONLY", "1")
     lib = _lib.load()
     h = C.c_void_p()
     _lib.check(lib.madm_create(C.byref(h), 0), None, "madm_create")
     try:
         _lib.check(lib.madm_set_compute_dtype(h, _lib.DTYPE_BF16), h, "dtype")
-        with empty_init():
-            unet, vae = UNetParams(device="meta"), VAEParams(device="meta")
-            for name in ("default", "Depth"):
-                unet.add_adapter(SimpleNamespace(r=16, lora_alpha=16, init_lora_weights="gaussian",
-                                                 target_modules=["to_k", "to_q", "to_v", "to_out.0"]), name)
-            projs = [BottleneckParams(c, 512, 128, device="meta") for c in (512, 320, 640, 1280)]
-        named = [("feature_extractor.ldm_extractor.unet." + n, p) for n, p in unet.named_parameters()]
-        named += [("feature_extractor.ldm_extractor.vae." + n, p) for n, p in vae.named_parameters()]
-        for i, pr in enumerate(projs):
-            named += [(f"feature_projections.{i}.0." + n, p) for n, p in pr.named_parameters()]
-
-        def table(items, base):
-            arr = (_lib.MadmTensor * len(items))()
-            keep = [n.encode() for n, _ in items]
-            for i, (n, t) in enumerate(items):
-                arr[i].name, arr[i].data, arr[i].ndim = keep[i], base + 16 * i, t.dim()
-                for k, s in enumerate(t.shape):
-                    arr[i].shape[k] = s
-            return arr, keep
-        arr, keep = table(named, 0x1000)
+        named = meta_training_params()
+        arr, keep = tensor_table(named, 0x1000)
         _lib.check(lib.madm_set_tensors(h, arr, len(named)), h, "madm_set_tensors")
         fwd = lib.madm_packed_bytes(h)
         dg = lib.madm_dgrad_packed_bytes(h)
         assert fwd > 2 ** 30 and dg > 2 ** 30, (fwd, dg, lib.madm_last_error(h))
         grads = [(n, t) for n, t in named if ("lora_" in n and ".Depth." in n) or n.startswith("feature_projections.")]
-        garr, gkeep = table(grads, 0x100000)
+        garr, gkeep = tensor_table(grads, 0x100000)
         _lib.check(lib.madm_set_grad_tensors(h, garr, len(grads)), h, "madm_set_grad_tensors")
         w1, w2, w4 = (lib.madm_train_workspace_bytes(h, b, b"Depth") for b in (1, 2, 4))
         assert 0 < w1 < w2 < w4 < 16 * 2 ** 30, (w1, w2, w4, lib.madm_last_error(h))
         assert lib.madm_train_workspace_bytes(h, 2, b"Depth") == w2
         assert lib.madm_train_workspace_bytes(h, 2, b"") <= w2  # no adapter: no LoRA gradient scratch
         # a gradient buffer for a name that is not a registered parameter is rejected
-        bad, bkeep = table([("feature_projections.9.0.conv1.weight", projs[0].conv1.weight)], 0x200000)
+        bad, bkeep = tensor_table([("feature_projections.9.0.conv1.weight", dict(named)["feature_projections.0.0.conv1.weight"])], 0x200000)
         assert lib.madm_set_grad_tensors(h, bad, 1) == -2
         # nothing can be launched from a device-less context
         a = _lib.MadmExtractArgs()

@@ -11,7 +11,7 @@ import torch
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-SWITCHES = [("base", "MADM_NO_S2D_FUSE=1"), ("base", "MADM_NO_SPLITK=1"), ("base", "MADM_TF_STREAM16=1"), ("base", "MADM_VAE_STREAM32=1"),
+SWITCHES = [("base", "MADM_NO_S2D_FUSE=1"), ("base", "MADM_NO_SPLITK=1"), ("base", "MADM_VAE_STREAM32=1"),
             ("base", "MADM_FUSE_STATS_KMIN=100000"), ("base", "MADM_GEMM_PAIR=0"), ("base", "MADM_PDL=1"), ("base", "MADM_GEMM_TMA_EPI=0"), ("base", "MADM_PROJ_STREAMS=0"),
             ("s0", "MADM_GEMM_TMA_EPI=7"),
             ("s0", "MADM_VAE_STREAM32=1"), ("s0", "MADM_NO_S2D_FUSE=1")]
