@@ -355,8 +355,7 @@ const char* bt_dispatch(const BwdTcParams& p, dim3 grid, int fp16, cudaStream_t 
 }  // namespace
 
 bool attention_bwd_tc_supported(int d, int Nq, int Nk) {
-  static const bool off = getenv("MADM_ATTN_BWD_TC") && atoi(getenv("MADM_ATTN_BWD_TC")) == 0;
-  return !off && (d == 40 || d == 80) && Nq % 128 == 0 && Nk % 128 == 0 && Nq >= 128 && Nk >= 128;
+  return (d == 40 || d == 80) && Nq % 128 == 0 && Nk % 128 == 0 && Nq >= 128 && Nk >= 128;
 }
 
 // dK / dV and dQ of one attention layer on the tcgen05 kernels.  L2 = log2-domain log-sum-exp, D = rowsum(dO * O), both [B, heads, Nq].

@@ -298,13 +298,8 @@ struct Builder {
     a.sr = 32;
     if (a.HW() % a.sr != 0 || a.C % 32 != 0) return;  // shape not eligible: the consumer falls back to a statistics pass
     // The fused statistics add ~25 % to the epilogue's instruction count (separate kernel variant, gemm_tc_kernel<BN,true>):
-    // measured +0.25 ms on the GEMM family against -1.0 ms of statistics passes, at every K; MADM_FUSE_STATS_KMIN can
-    // restrict the fusion to long-K producers.
-    int K = 0;
-    for (int sgi = 0; sgi < d.nseg; ++sgi) K += d.seg[sgi].ntaps * d.seg[sgi].C;
-    static const int kmin = getenv("MADM_FUSE_STATS_KMIN") ? atoi(getenv("MADM_FUSE_STATS_KMIN")) : 0;
-    if (K < kmin) return;
-    if (!getenv("MADM_NO_SPLITK") && choose_splits(d) > 1) return;  // split-K launches leave the statistics to a separate pass
+    // measured +0.25 ms on the GEMM family against -1.0 ms of statistics passes, at every K.
+    if (choose_splits(d) > 1) return;  // split-K launches leave the statistics to a separate pass
     const size_t n = size_t((a.M() + a.sr - 1) / a.sr) * a.C * 2;
     a.cs = stats_base ? stats_base + stats_used : nullptr;
     stats_used += n;
@@ -461,8 +456,9 @@ struct Builder {
   // algo_flops < 0: 2*M*N*K from the descriptor (K counts real channels only when k_real is given)
   // split-K factor for a GEMM whose M x N tiling cannot fill the 148 SMs (8x8-resolution convs, small batches): the K range
   // is divided over `splits` CTAs per output tile; raw fp32 partials are reduced in fixed order by splitk_reduce, which
-  // also applies the fused epilogue.  Deterministic (no atomics).
+  // also applies the fused epilogue.  Deterministic (no atomics).  MADM_NO_SPLITK=1 turns it off: the reference summation order.
   static int choose_splits(const GemmDesc& d) {
+    if (getenv("MADM_NO_SPLITK")) return 1;
     if (d.act == ACT_GEGLU || d.N % 4 != 0 || d.N < 128) return 1;
     const int tiles = ((d.M + 127) / 128) * ((d.N + 127) / 128);  // the split launch uses 128-wide N tiles
     int chunks = 0;
@@ -487,7 +483,7 @@ struct Builder {
     return by;
   }
   void gemm(const GemmDesc& d0, double algo_flops = -1.0) {
-    const int splits = getenv("MADM_NO_SPLITK") ? 1 : choose_splits(d0);
+    const int splits = choose_splits(d0);
     if (splits > 1) {  // identical allocation sequence in every builder mode
       F32T part = f32(size_t(splits) * d0.M * d0.N);
       if (mode == PLAN) {
@@ -743,7 +739,6 @@ struct Model {
   // for the plain residual); out16_only then also drops the fp32 copy of the output.
   Act resblock(const std::string& p, const Act& x0, const Act* x1, int Cout, float eps, bool has_temb, bool want_b16, bool want_s2d = false,
                bool out16_only = false) {
-    if (getenv("MADM_NO_S2D_FUSE") && !out16_only) want_s2d = false;  // (debug switch; a 16-bit-only output has no fp32 copy to convert later)
     const int Bn = x0.B, H = x0.H, W = x0.W, Cin = x0.C + (x1 ? x1->C : 0);
     const bool shortcut = Cin != Cout;
     const bool in16 = x0.f.bytes == 0 && x0.h.bytes != 0;  // (valid in every builder mode: sizes, not pointers)
@@ -838,7 +833,6 @@ struct Model {
 
   // ---- Transformer2DModel (one BasicTransformerBlock): returns fp32 (+bf16) output; x is NOT freed
   Act transformer(const std::string& p, const Act& x, bool want_b16, bool want_s2d = false) {
-    if (getenv("MADM_NO_S2D_FUSE")) want_s2d = false;
     const bool train = b.recording();
     const int Bn = x.B, H = x.H, W = x.W, C = x.C;
     const long M = x.M();
@@ -1032,25 +1026,13 @@ struct Model {
 
   Act downsample(const std::string& p, const Act& x, bool pad1, bool out16_only = false) {
     const int Bn = x.B, H = x.H, W = x.W, C = x.C;
-    B16T s2d;
-    const bf16* s2dp;
-    if (x.h_s2d) {  // the producer's epilogue already wrote the space-to-depth operand
-      s2dp = x.h.p;
-    } else {
-      if (x.f.bytes == 0) b.fail(MADM_EINVAL, "downsample: the input has neither a space-to-depth operand nor an fp32 copy");
-      s2d = b.b16(size_t(x.M()) * C);
-      s2dp = s2d.p;
-      const float* src = x.f.p; bf16* dst = s2d.p;
-      const int h16 = f16();
-      b.emit([=](cudaStream_t st) { return space_to_depth(src, Bn, H, W, C, dst, h16, st); }, false, MADM_KIND_ELEMENTWISE, 0.0,
-             double(x.M()) * C * 6);
-    }
+    // the producer's epilogue writes the stride-2 conv's space-to-depth operand (resblock / transformer with want_s2d)
+    if (!x.h_s2d) b.fail(MADM_EINVAL, "downsample: the input has no space-to-depth operand");
     Act out = b.act(Bn, H / 2, W / 2, C, !out16_only, out16_only);
-    { GemmDesc d; d.seg[0] = Builder::seg_s2(s2dp, Bn, H / 2, W / 2, C, pad1); d.M = int(out.M()); d.N = C; d.Nw = C;
+    { GemmDesc d; d.seg[0] = Builder::seg_s2(x.h.p, Bn, H / 2, W / 2, C, pad1); d.M = int(out.M()); d.N = C; d.Nw = C;
       d.w = b.pw(b.conv_w(p + ".conv", C, C, 9)); d.bias = P(p + ".conv.bias", C);
       if (out16_only) { d.out_bf16 = out.h.p; d.ldo16 = C; } else { d.out_f32 = out.f.p; d.ldo32 = C; }
       b.attach_colstats(out, d); b.gemm(d); }
-    if (!x.h_s2d) b.free(s2d);
     if (!b.recording()) return out;
     const Act xin = x;
     b.tape.push_back([=]() {
@@ -1201,30 +1183,13 @@ struct Model {
     check_lora_rank(module);
     const float alpha = b.lora_scale / b.loss_scale;
     const int h16 = f16(), Mi = int(M);
-    static const bool fused_off = getenv("MADM_LORA_GRADS_FUSED") && atoi(getenv("MADM_LORA_GRADS_FUSED")) == 0;
-    if (!fused_off && lora_grads_supported(N, K)) {  // both factor gradients in one kernel + one reduce (wgrad.cu)
-      F32T scr = b.f32(lora_grads_scratch_floats(Mi, N, K));
-      const bf16* a16 = b.dpw(oa); const bf16* bt16 = b.dpw(ob); float* sp = scr.p;
-      b.emit([=](cudaStream_t st) { return lora_grads(X, ldx, dY, ldy, a16, bt16, Mi, N, K, alpha, gA, gB, sp, h16, st); });
-      b.free(scr);
-      return;
-    }
-    if (gB) {
-      B16T U = b.b16(size_t(M) * 16);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(X, M, K, ldx); d.M = Mi; d.N = 16; d.Nw = 16; d.w = b.dpw(oa); d.out_bf16 = U.p; d.ldo16 = 16; d.bn = 16; b.gemm(d); }
-      F32T scr = b.f32(wgrad_scratch_floats(Mi, N, 16, 1));
-      const bf16* up = U.p; float* sp = scr.p;
-      b.emit([=](cudaStream_t st) { return wgrad(dY, ldy, up, 16, Mi, N, 16, 1, 0, 0, 0, alpha, gB, 16, 1, 0, sp, h16, st); });
-      b.free(scr); b.free(U);
-    }
-    if (gA) {
-      B16T V = b.b16(size_t(M) * 16);
-      { GemmDesc d; d.seg[0] = Builder::seg_plain(dY, M, N, ldy); d.M = Mi; d.N = 16; d.Nw = 16; d.w = b.dpw(ob); d.out_bf16 = V.p; d.ldo16 = 16; d.bn = 16; b.gemm(d); }
-      F32T scr = b.f32(wgrad_scratch_floats(Mi, K, 16, 1));
-      const bf16* vp = V.p; float* sp = scr.p;
-      b.emit([=](cudaStream_t st) { return wgrad(X, ldx, vp, 16, Mi, K, 16, 1, 0, 0, 0, alpha, gA, 1, K, 0, sp, h16, st); });  // (X^T V)^T -> [16,K]
-      b.free(scr); b.free(V);
-    }
+    if (!lora_grads_supported(N, K))
+      b.fail(MADM_EINVAL, "training path: no LoRA gradient kernel for N = " + std::to_string(N) + ", K = " + std::to_string(K) + " (" + module + ")");
+    // both factor gradients in one kernel + one reduce (wgrad.cu)
+    F32T scr = b.f32(lora_grads_scratch_floats(Mi, N, K));
+    const bf16* a16 = b.dpw(oa); const bf16* bt16 = b.dpw(ob); float* sp = scr.p;
+    b.emit([=](cudaStream_t st) { return lora_grads(X, ldx, dY, ldy, a16, bt16, Mi, N, K, alpha, gA, gB, sp, h16, st); });
+    b.free(scr);
   }
 
   // =========================================================================== VAE encoder
@@ -1239,7 +1204,7 @@ struct Model {
       b.emit([=](cudaStream_t st) { return image_im2col(io->a.img, Bn, R, R, dst, io->a.range_flag, h16, st, io->a.flags & MADM_FLAG_IMG_NORMALISED); }); }
     // fp16 operands: the residual stream of the 512^2 and 256^2 stages (3/4 of the VAE's bytes) is kept in fp16 like the
     // reference's VAE (AutoencoderKL loaded with torch_dtype=float16, ldm_diffusers.py:246-249); bf16 keeps the fp32 stream.
-    const bool s16 = f16() && !getenv("MADM_VAE_STREAM32");
+    const bool s16 = f16();
     Act x = b.act(Bn, R, R, 128, !s16, s16);
     { GemmDesc d; d.seg[0] = Builder::seg_plain(col.p, long(Bn) * R * R, 64); d.M = Bn * R * R; d.N = 128; d.Nw = 128;
       d.w = b.pw(b.conv_w(e + "conv_in", 128, 3, 9, /*Cpad=*/3)); d.bias = P(e + "conv_in.bias", 128);
@@ -1498,7 +1463,7 @@ struct Model {
       y = resblock(dc + "mid_block.resnets.1", x, nullptr, 512, 1e-6f, false, false); b.free(x); x = y;
     }
     // fp16 operands: the 256^2 and 512^2 stages keep their residual stream in fp16, like the encoder's (and the reference's fp16 VAE)
-    const bool s16 = f16() && !getenv("MADM_VAE_STREAM32");
+    const bool s16 = f16();
     const int ch[4] = {512, 512, 256, 128};
     for (int i = 0; i < 4; ++i) {
       const bool o16 = s16 && i >= 2;
@@ -1540,15 +1505,10 @@ struct Model {
   // branch (1..4) and emitted as soon as its tap exists -- the encoder tap's right after the VAE stage, the UNet taps' after up layers 5 / 8 / 11 --
   // so madm_extract can run it on a side stream that forks there and joins at the end of the plan (inside a CUDA-graph capture: parallel graph
   // branches): the projections fill the SMs the under-filled 16x16 / 8x8 UNet levels leave idle.  A branch's buffers are not recycled before the
-  // end of the plan.  MADM_PROJ_STREAMS=0 keeps everything on the caller's stream, in the old order (after the UNet).
+  // end of the plan.
   bool proj_built[4] = {false, false, false, false};
-  static bool proj_streams() {
-    static const bool on = !(getenv("MADM_PROJ_STREAMS") && atoi(getenv("MADM_PROJ_STREAMS")) == 0);
-    return on;
-  }
   void build_proj_early(int i) {  // called where tap i has just been produced
-    static const bool early = !(getenv("MADM_PROJ_EARLY") && atoi(getenv("MADM_PROJ_EARLY")) == 0);
-    if (early && proj_streams() && !s0() && !b.train) build_proj_one(i);
+    if (!s0() && !b.train) build_proj_one(i);
   }
   void build_proj() {
     for (int i = 0; i < 4; ++i) build_proj_one(i);
@@ -1562,9 +1522,9 @@ struct Model {
     std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
     const std::string root = b.ema ? "ema_feature_projections." : "feature_projections.";
     const Act* taps[4] = {&enc_tap, &unet_tap[0], &unet_tap[1], &unet_tap[2]};
-    b.defer_free = proj_streams();
+    b.defer_free = true;
     {
-      b.cur_branch = proj_streams() ? 1 + i : 0;
+      b.cur_branch = 1 + i;
       const Act& x = *taps[i];
       const std::string p = root + std::to_string(i) + ".0.";
       const int h16 = f16();

@@ -20,6 +20,7 @@
 
 #include <mutex>
 #include <stdio.h>
+#include <string.h>
 
 namespace madm {
 
@@ -100,12 +101,10 @@ struct Cfg {
   static constexpr int BUDGET = 227 * 1024 - 1024 /*align*/ - 256 /*barriers*/ - EPI_BYTES;
   static constexpr int STAGES = (BUDGET / STAGE_BYTES) > 8 ? 8 : (BUDGET / STAGE_BYTES);
   static constexpr int ACC_STRIDE = BN <= 16 ? 16 : (BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256)));
-  // two accumulator stages (the MMAs of tile i+1 overlap the epilogue of tile i) wherever they fit the 512 TMEM columns; the 512-row pair tile of the
-  // 160-wide layers (MT = 2, stride 256) has room for one: its drain is exposed, its W traffic per MMA is halved (DESIGN section 9)
-  static constexpr int NACC = (2 * MT * ACC_STRIDE <= 512) ? 2 : 1;
+  static constexpr int NACC = 2;  // accumulator stages: the MMAs of tile i+1 overlap the epilogue of tile i
   static constexpr int TMEM_COLS = NACC * MT * ACC_STRIDE < 32 ? 32 : NACC * MT * ACC_STRIDE;
   static constexpr size_t SMEM = size_t(STAGES) * STAGE_BYTES + EPI_BYTES + 1024 + 256;
-  static_assert(TMEM_COLS <= 512, "TMEM budget");
+  static_assert(TMEM_COLS <= 512, "two accumulator stages must fit the 512 TMEM columns");
 };
 
 __device__ __forceinline__ float silu_f(float v) { return v / (1.0f + __expf(-v)); }
@@ -953,24 +952,13 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     const long tiles2 = long((d.M + 2 * BM - 1) / (2 * BM)) * n_tiles;
     if (d.mt == 2 || tiles2 >= 2L * num_sms()) L.mt = 2;
   }
-  // 160-wide layers with long K (the UNet's 64x64-level convs): 512-row pair tiles when there are at least two waves of them
-  {
-    static const int env160 = getenv("MADM_GEMM_MT160") ? atoi(getenv("MADM_GEMM_MT160")) : 0;
-    int ktot160 = 0;
-    for (int s = 0; s < d.nseg; ++s) ktot160 += d.seg[s].ntaps * d.seg[s].C;
-    const long ptiles = long((d.M + 4 * BM - 1) / (4 * BM)) * n_tiles;
-    if (L.bn == 160 && num_sms() % 2 == 0 && d.pair >= 0 && (d.mt == 2 || (env160 > 0 && d.mt != 1 && ktot160 >= 2304 && ptiles >= num_sms()))) L.mt = 2;
-  }
   int m_tiles = (d.M + BM * L.mt - 1) / (BM * L.mt);
   // CTA pairs: worthwhile when every pair still gets at least one full tile; needs an even CTA count
   L.pair = 0;
   {
-    static const int env_pair = getenv("MADM_GEMM_PAIR") ? atoi(getenv("MADM_GEMM_PAIR")) : 1;
     const bool shape_ok = L.bn >= 128 && num_sms() % 2 == 0;
     const long pair_tiles = long((m_tiles + 1) / 2) * n_tiles;
-    if (shape_ok && d.pair >= 0 && (d.pair == 1 || (env_pair > 0 && pair_tiles >= num_sms() / 2))) L.pair = 1;
-    if (L.bn == 160 && L.mt == 2 && !L.pair) L.mt = 1;  // (the one-stage 512-row tile exists as a pair kernel only)
-    if (L.bn == 160 && L.mt == 1 && m_tiles != (d.M + BM - 1) / BM) m_tiles = (d.M + BM - 1) / BM;
+    if (shape_ok && d.pair >= 0 && (d.pair == 1 || pair_tiles >= num_sms() / 2)) L.pair = 1;
   }
   if (L.pair) m_tiles = (m_tiles + 1) / 2;  // tiles of the pair
   {
@@ -998,9 +986,8 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
   // split-K, two outputs and out-of-place / 16-bit residuals keep the coalesced epilogue.  MADM_GEMM_TMA_EPI=0 disables.
   L.tma_epi = TMA_EPI_NONE;
   {
-    const char* env = getenv("MADM_GEMM_TMA_EPI");  // bit mask: 1 fp32 stores, 2 reduce-add, 4 16-bit stores, 8 with fused statistics, 16 residual load + 16-bit store
-    const int mask = env ? atoi(env) : 31;
-    const bool on = mask != 0;
+    const char* env = getenv("MADM_GEMM_TMA_EPI");
+    const bool on = !(env && strcmp(env, "0") == 0);
     auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
     const bool plain = on && L.bn >= 32 && L.splits == 1 && d.s2d_W == 0 && d.N % 32 == 0 && (!d.bias || al16(d.bias)) &&
                        (!d.rowbias || (al16(d.rowbias) && (d.ld_rowbias ? d.ld_rowbias : d.N) % 4 == 0));
@@ -1015,8 +1002,6 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
                al16(d.residual) && d.ldr % 4 == 0 && EPI_NBUF >= 2) {
       L.tma_epi = TMA_EPI_RES_H16;  // out16 = 16-bit(GEMM + fp32 residual), residual out of place: the transformer's FF out-projection
     }
-    if (L.tma_epi && !((mask >> (L.tma_epi == TMA_EPI_F32 ? 0 : (L.tma_epi == TMA_EPI_RED ? 1 : (L.tma_epi == TMA_EPI_H16 ? 2 : 4)))) & 1)) L.tma_epi = TMA_EPI_NONE;
-    if (L.tma_epi && d.colstats && !(mask & 8)) L.tma_epi = TMA_EPI_NONE;
     if (L.tma_epi == TMA_EPI_RES_H16) {
       cuuint64_t dims[2] = {cuuint64_t(d.N), cuuint64_t(d.M)};
       cuuint64_t strides[1] = {cuuint64_t(d.ldr) * 4};
@@ -1045,7 +1030,7 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     case 32: L.smem = Cfg<32, 1>::SMEM; break;
     case 64: L.smem = Cfg<64, 1>::SMEM; break;
     case 128: L.smem = L.mt == 2 ? (L.pair ? Cfg<128, 2, true>::SMEM : Cfg<128, 2>::SMEM) : (L.pair ? Cfg<128, 1, true>::SMEM : Cfg<128, 1>::SMEM); break;
-    case 160: L.smem = L.mt == 2 ? Cfg<160, 2, true>::SMEM : (L.pair ? Cfg<160, 1, true>::SMEM : Cfg<160, 1>::SMEM); break;
+    case 160: L.smem = L.pair ? Cfg<160, 1, true>::SMEM : Cfg<160, 1>::SMEM; break;
     case 192: L.smem = L.pair ? Cfg<192, 1, true>::SMEM : Cfg<192, 1>::SMEM; break;
     case 256: L.smem = L.pair ? Cfg<256, 1, true>::SMEM : Cfg<256, 1>::SMEM; break;
     default: return "gemm: unsupported N tile";
@@ -1073,7 +1058,7 @@ static const char* launch_bn_s(const GemmLaunch& L, const GemmParams& p, cudaStr
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
-    if (pdl_enabled()) {
+    if (pdl_train_scope()) {
       at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
       at[1].val.programmaticStreamSerializationAllowed = 1;
       cfg.numAttrs = 2;
@@ -1111,9 +1096,6 @@ template <int BN>
 static const char* launch_bn(const GemmLaunch& L, const GemmParams& p, cudaStream_t stream) {
   if constexpr (BN == 128) {
     if (L.mt == 2) return L.pair ? launch_epi<BN, 2, true>(L, p, stream) : launch_epi<BN, 2, false>(L, p, stream);
-  }
-  if constexpr (BN == 160) {
-    if (L.mt == 2) return launch_epi<BN, 2, true>(L, p, stream);
   }
   if constexpr (BN >= 128) {
     if (L.pair) return launch_epi<BN, 1, true>(L, p, stream);

@@ -5,34 +5,21 @@
 // Rules that keep this race-free: (1) every kernel launched through launch_k() executes pdl_wait() on every thread before its first
 // global-memory access and before any early return; (2) kernels that are not PDL-aware are launched with <<<>>> and serialise as usual
 // (griddepcontrol.* are no-ops without the launch attribute).
-// Measured on B200 (bench.py, B = 8, CUDA-graph replay, 20 steps): 24.25 -> 24.17 ms per step for the base path, 50.36 -> 50.59 ms for
-// the s0 variant, i.e. nothing: inside a graph the launch gaps are already ~1 us and the step runs at the board's power cap.  The
-// attribute is therefore OFF by default for inference plans; MADM_PDL=1 turns it on (the full GPU test suite passes either way).
+// The attribute is on inside training passes (PdlTrainScope) and off for inference.  A training pass at 2 images per GPU is ~1200
+// eager launches of 5-40 us whose prologues are a visible fraction of each kernel: 64.0 -> 60.8 ms per training step (bench.py
+// --config train, two runs each).  For inference it measured nothing (B200, bench.py, B = 8, CUDA-graph replay, 20 steps: 24.25 ->
+// 24.17 ms per step for the base path, 50.36 -> 50.59 ms for the s0 variant): inside a graph the launch gaps are already ~1 us and
+// the step runs at the board's power cap.
 #pragma once
 #include <cuda_runtime.h>
-#include <stdlib.h>
 
 namespace madm {
 
-// MADM_PDL=0 / 1 forces the attribute off / on everywhere; unset: off for inference plans (measured above), ON inside the training scope --
-// a training pass at 2 images per GPU is ~1200 eager launches of 5-40 us whose prologues (TMEM allocation, barrier init, tensor-map prefetch) are
-// a visible fraction of each kernel: 64.0 -> 60.8 ms per training step (bench.py --config train, two runs each).
-inline int pdl_env() {
-  static const int v = [] {
-    const char* e = getenv("MADM_PDL");
-    return e ? (atoi(e) != 0 ? 1 : 0) : -1;
-  }();
-  return v;
-}
 inline bool& pdl_train_scope() {
   static thread_local bool on = false;
   return on;
 }
-inline bool pdl_enabled() {
-  const int e = pdl_env();
-  return e >= 0 ? e != 0 : pdl_train_scope();
-}
-struct PdlTrainScope {  // RAII: launches issued while one is alive carry the PDL attribute (unless MADM_PDL=0)
+struct PdlTrainScope {  // RAII: launches issued while one is alive carry the PDL attribute
   bool prev;
   PdlTrainScope() : prev(pdl_train_scope()) { pdl_train_scope() = true; }
   ~PdlTrainScope() { pdl_train_scope() = prev; }
@@ -46,7 +33,7 @@ inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute at[1];
-  if (pdl_enabled()) {
+  if (pdl_train_scope()) {
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;

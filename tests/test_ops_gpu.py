@@ -406,8 +406,6 @@ def test_layernorm(ops, cuda_device, M, Cc):
     (1, 1, 1000, 256, 416, 1, 0, 0),      # ragged M and an N that is not a multiple of the tile (W rows past N are TMA zero fill)
     (2, 64, 64, 320, 320, 9, 0, 0),       # 3x3 conv, 160-wide pair tiles
     (2, 128, 128, 128, 128, 9, 128, 2),   # 512-row pair tiles (two M sub-tiles per CTA)
-    (2, 64, 64, 320, 320, 9, 160, 2),     # 512-row pair tiles of the 160-wide layers: one accumulator stage (pair = -1 falls back to 128-row tiles)
-    (1, 1, 1300, 320, 320, 1, 160, 2),    # the same with a ragged last tile
     (3, 32, 32, 640, 1280, 1, 0, 0),
 ])
 def test_gemm_cta_pairs_match_single_cta(ops, cuda_device, B, H, W, Cin, Cout, taps, bn, mt):

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Attention backward against torch.autograd on a chosen input distribution (peaky softmax, loss-scaled dO); run with MADM_ATTN_BWD_TC=0 / 1
-to compare the warp-level and the tcgen05 kernels.  Usage: check_attn_bwd.py [qk_scale] [do_scale] [dtype]"""
+"""Attention backward against torch.autograd on a chosen input distribution (peaky softmax, loss-scaled dO), at the d = 40 self-attention
+shape that runs on the tcgen05 kernels.  Usage: check_attn_bwd.py [qk_scale] [do_scale] [dtype]"""
 import math
 import os
 import sys
@@ -34,7 +34,7 @@ ops.attention_bwd(q, 3 * Cc, k, 3 * Cc, v, 3 * Cc, o, Cc, dout, Cc, dq, 3 * Cc, 
                   N * 3 * Cc, N * 3 * Cc, 1.0 / math.sqrt(d))
 torch.cuda.synchronize()
 merge = lambda t: t.transpose(1, 2).reshape(B, -1, Cc)  # noqa: E731
-print(f"MADM_ATTN_BWD_TC={os.environ.get('MADM_ATTN_BWD_TC', '(default)')} qk_scale {qk_scale} do_scale {do_scale} {dt}")
+print(f"qk_scale {qk_scale} do_scale {do_scale} {dt}")
 for name, got, ref in (("dq", dq, qr.grad), ("dk", dk, kr.grad), ("dv", dv, vr.grad)):
     r = merge(ref).double().flatten(); gg = got.double().flatten()
     cos = F.cosine_similarity(gg, r, dim=0).item()
