@@ -13,6 +13,7 @@
 #include "kernels.h"
 #include "launch.cuh"
 
+#include <algorithm>
 #include <cuda_bf16.h>
 #include <functional>
 #include <map>
@@ -43,40 +44,47 @@ struct ParamRef {
   }
 };
 
-// ---- packed arena entries
-enum PackKind { PK_CONV, PK_LINEAR, PK_GEGLU, PK_VAE_HEAD, PK_F32_COPY, PK_F32_SUM2, PK_F32_GEGLU_BIAS,
-                PK_BN_FOLD,   // eval-mode BatchNorm -> fp32 [scale | shift] (bias_off = N floats each)
-                PK_CONV_BN,   // conv weight with the BatchNorm scale (at bias_off) folded into its rows
-                PK_DW_BN,     // depthwise 3x3 weight * BatchNorm scale -> fp32 [9][C]
-                PK_IDENTITY }; // N x N identity block (16-bit) inside a wider packed row: the residual add as an extra K segment
+// ---- packed arena entries.  Two arenas use them: the forward arena (madm_pack_weights) and the training path's input-gradient
+// ("dgrad") arena (madm_pack_dgrad_weights): transposed / tap-mirrored 16-bit copies of the frozen weights (LoRA folded), the skinny
+// LoRA factor operands, and the natural-order feed-forward weight of the training forward.
+enum PackKind { PK_CONV,       // conv [N,C,k,k] -> [N, taps*Cpad] inside rows of pitch ldo
+                PK_CONV_DGRAD, // conv [Cout=N,Cin=C,k,k] -> [Cin, taps*Cpad], mirrored taps (Cpad = Cout)
+                PK_LINEAR,     // linear [N,K=C] (+ LoRA) in natural row order, rows of pitch ldo
+                PK_LINEAR_T,   // linear [N,K=C] (+ LoRA) -> its transpose, written at a column offset of a [K, ldo] region
+                PK_LORA_A,     // lora_A [r,in] -> [r,in]       (operand of U = X A^T)
+                PK_LORA_BT,    // lora_B [out,r] -> [r,out]     (operand of V = dY B)
+                PK_GEGLU, PK_VAE_HEAD, PK_F32_COPY, PK_F32_SUM2,
+                PK_BN_FOLD,    // eval-mode BatchNorm -> fp32 [scale | shift] (bias_off = N floats each)
+                PK_CONV_BN,    // conv weight with the BatchNorm scale (at bias_off) folded into its rows
+                PK_DW_BN,      // depthwise 3x3 weight * BatchNorm scale -> fp32 [9][C]
+                PK_IDENTITY,   // N x N identity block (16-bit) inside a wider packed row: the residual add as an extra K segment
+                PK_REGION };   // bytes reserved for entries registered into it
 struct PackEntry {
   PackKind kind;
-  std::string src, src2, src3, src4;  // parameter names
+  std::string src, src2, src3, src4;  // parameter names (linear / LoRA factor: the module path)
   size_t off = 0;                     // byte offset in arena
   int N = 0, C = 0, taps = 1, Cpad = 0, Kpad = 0, ldo = 0;
-  bool lora = false;                  // LoRA-targeted linear (src is the module path)
+  bool lora = false;                  // LoRA-targeted linear
+  bool trainable = false;             // an optimizer or EMA step can change it: the subset a partial repack rewrites
   size_t bias_off = 0;                // for GEGLU / VAE head: fp32 bias region
+};
+
+// An arena's layout: its entries by key, laid out by a LAYOUT pass of the traversal and looked up by the other passes
+struct Arena {
+  std::vector<PackEntry> entries;
+  std::map<std::string, size_t> index;  // key -> index in entries
+  size_t bytes = 0;
+  bool done = false;                    // laid out for the current parameter shapes, operand dtype and variant
+  size_t reserve(size_t n) {
+    const size_t off = bytes;
+    bytes += (n + 1023) & ~size_t(1023);
+    return off;
+  }
 };
 
 struct IoBind {  // per-call pointers read by the plan's first/last ops
   madm_extract_args a;
   madm_backward_args b;  // training plans: the arguments of the madm_backward call being replayed
-};
-
-// ---- input-gradient ("dgrad") arena of the training path: transposed / tap-mirrored 16-bit copies of the frozen weights (LoRA folded),
-// the skinny LoRA factor operands, and the natural-order feed-forward weight of the training forward
-enum DPackKind { DG_CONV,        // conv [Cout,Cin,k,k] -> [Cin, taps*CoPad], mirrored taps
-                 DG_LINEAR,      // linear [N,K] (+ LoRA) -> its transpose, written at a column offset of a [K, ldo] region
-                 DG_LINEAR_FWD,  // linear [N,K] -> [N,K] (forward operand in natural row order: ff.net.0.proj of the training forward)
-                 DG_LORA_A,      // lora_A [r,in] -> [r,in]       (operand of U = X A^T)
-                 DG_LORA_BT,     // lora_B [out,r] -> [r,out]     (operand of V = dY B)
-                 DG_REGION };
-struct DPackEntry {
-  DPackKind kind;
-  std::string src;   // parameter name (conv: "<m>.weight"; linear / LoRA: module path)
-  size_t off = 0;
-  int N = 0, C = 0, taps = 1, CoPad = 0, ldo = 0;
-  bool lora = false;
 };
 
 struct F32T { float* p = nullptr; size_t off = 0; size_t bytes = 0; };
@@ -135,10 +143,8 @@ struct madm_ctx {
   int variant = MADM_VARIANT_BASE;
   std::string err;
   std::unordered_map<std::string, ParamRef> params;
-  std::vector<PackEntry> pack;
-  std::map<std::string, size_t> pack_index;  // key -> index in pack
-  size_t packed_bytes = 0;
-  bool layout_done = false;
+  Arena fwd;    // forward arena (madm_pack_weights)
+  Arena dgrad;  // input-gradient arena of the training path (madm_pack_dgrad_weights)
   float* alphas_cumprod = nullptr;  // [1000] device
   bool profiling = false;
   cudaStream_t side[4] = {nullptr, nullptr, nullptr, nullptr};  // projection branches (created on first use)
@@ -149,12 +155,7 @@ struct madm_ctx {
   std::map<std::tuple<int, int, int>, size_t> ws_bytes_cache;             // (B, head_h, head_w)
   // training path
   std::unordered_map<std::string, float*> grads;     // gradient output buffers by parameter name (madm_set_grad_tensors)
-  std::vector<DPackEntry> dpack;
-  std::map<std::string, size_t> dpack_index;
-  size_t dpacked_bytes = 0;
-  bool dlayout_done = false;
   std::map<std::pair<int, uintptr_t>, std::unique_ptr<Plan>> train_plans;  // (B, training workspace) -> forward (activations kept) + backward
-  std::map<int, size_t> train_ws_cache;
 };
 
 namespace {
@@ -194,7 +195,7 @@ struct Builder {
   float loss_scale = 1.0f;
   std::string adapter;         // active LoRA adapter of this training plan ("" = none)
   float lora_scale = 0.f;
-  std::vector<std::function<void()>> tape;
+  std::vector<std::pair<int, std::function<void()>>> tape;  // (stage of the forward that recorded it, its backward)
   // forward of a stage the training plan differentiates (not the VAE): its tensors stay allocated and each block records its backward
   bool recording() const { return train && !bwd && cur_stage != MADM_STAGE_VAE; }
 
@@ -321,20 +322,19 @@ struct Builder {
     return r->p;
   }
 
-  // ---- packed arena
-  size_t pack_reserve(size_t bytes) {
-    size_t off = ctx->packed_bytes;
-    ctx->packed_bytes += (bytes + 1023) & ~size_t(1023);
-    return off;
-  }
-  // returns arena offset of an entry, registering it in LAYOUT mode
-  const PackEntry& entry(const std::string& key, const std::function<PackEntry()>& make) {
-    auto it = ctx->pack_index.find(key);
-    if (it != ctx->pack_index.end()) return ctx->pack[it->second];
+  // ---- packed arenas
+  // returns an arena's entry, registering it in a LAYOUT pass.  The training traversal's LAYOUT pass only adds to the dgrad arena: the
+  // caller has sized the forward arena already (madm_packed_bytes).
+  const PackEntry& entry(Arena& a, const std::string& key, const std::function<PackEntry()>& make) {
+    auto it = a.index.find(key);
+    if (it != a.index.end()) return a.entries[it->second];
     if (mode != LAYOUT) fail(MADM_ESTATE, "packed entry missing from layout: " + key);
-    ctx->pack.push_back(make());
-    ctx->pack_index[key] = ctx->pack.size() - 1;
-    return ctx->pack.back();
+    if (train && &a == &ctx->fwd) fail(MADM_ESTATE, "training layout reached a forward-arena entry the forward layout lacks: " + key);
+    PackEntry e = make();
+    e.trainable = e.lora || e.kind == PK_LORA_A || e.kind == PK_LORA_BT || cur_stage == MADM_STAGE_PROJ;
+    a.index[key] = a.entries.size();
+    a.entries.push_back(e);
+    return a.entries.back();
   }
   const bf16* pw(size_t off) const { return reinterpret_cast<const bf16*>(packed + off); }
   const float* pf(size_t off) const { return reinterpret_cast<const float*>(packed + off); }
@@ -343,9 +343,9 @@ struct Builder {
   size_t conv_w(const std::string& name, int N, int C, int taps, int Cpad = 0) {
     if (Cpad == 0) Cpad = (C + 63) / 64 * 64;
     const int Kpad = (taps * Cpad + 63) / 64 * 64;
-    return entry("conv:" + name, [&] {
+    return entry(ctx->fwd, "conv:" + name, [&] {
       PackEntry e; e.kind = PK_CONV; e.src = name + ".weight"; e.N = N; e.C = C; e.taps = taps; e.Cpad = Cpad; e.Kpad = Kpad; e.ldo = Kpad;
-      e.off = pack_reserve(size_t(N) * Kpad * 2);
+      e.off = ctx->fwd.reserve(size_t(N) * Kpad * 2);
       return e;
     }).off;
   }
@@ -353,20 +353,20 @@ struct Builder {
   struct Fused { size_t w_off, b_off; };
   Fused conv_plus_shortcut(const std::string& conv, const std::string& sc, int Cout, int Cin) {
     const int K0 = 9 * Cout, K = K0 + Cin;
-    const PackEntry& e0 = entry("convsc:" + conv, [&] {
+    const PackEntry& e0 = entry(ctx->fwd, "convsc:" + conv, [&] {
       PackEntry e; e.kind = PK_CONV; e.src = conv + ".weight"; e.N = Cout; e.C = Cout; e.taps = 9; e.Cpad = Cout; e.Kpad = K0; e.ldo = K;
-      e.off = pack_reserve(size_t(Cout) * K * 2);
+      e.off = ctx->fwd.reserve(size_t(Cout) * K * 2);
       return e;
     });
     const size_t w_off = e0.off;
-    entry("convsc_sc:" + conv, [&] {
+    entry(ctx->fwd, "convsc_sc:" + conv, [&] {
       PackEntry e; e.kind = PK_CONV; e.src = sc + ".weight"; e.N = Cout; e.C = Cin; e.taps = 1; e.Cpad = Cin; e.Kpad = Cin; e.ldo = K;
       e.off = w_off + size_t(K0) * 2;
       return e;
     });
-    const size_t b_off = entry("convsc_b:" + conv, [&] {
+    const size_t b_off = entry(ctx->fwd, "convsc_b:" + conv, [&] {
       PackEntry e; e.kind = PK_F32_SUM2; e.src = conv + ".bias"; e.src2 = sc + ".bias"; e.N = Cout;
-      e.off = pack_reserve(size_t(Cout) * 4);
+      e.off = ctx->fwd.reserve(size_t(Cout) * 4);
       return e;
     }).off;
     return Fused{w_off, b_off};
@@ -376,12 +376,12 @@ struct Builder {
   // needs no fp32 residual tensor.
   size_t conv_plus_identity(const std::string& conv, int C) {
     const int K0 = 9 * C, K = K0 + C;
-    const size_t w_off = entry("convid:" + conv, [&] {
+    const size_t w_off = entry(ctx->fwd, "convid:" + conv, [&] {
       PackEntry e; e.kind = PK_CONV; e.src = conv + ".weight"; e.N = C; e.C = C; e.taps = 9; e.Cpad = C; e.Kpad = K0; e.ldo = K;
-      e.off = pack_reserve(size_t(C) * K * 2);
+      e.off = ctx->fwd.reserve(size_t(C) * K * 2);
       return e;
     }).off;
-    entry("convid_i:" + conv, [&] {
+    entry(ctx->fwd, "convid_i:" + conv, [&] {
       PackEntry e; e.kind = PK_IDENTITY; e.N = C; e.ldo = K; e.off = w_off + size_t(K0) * 2;
       return e;
     });
@@ -389,51 +389,54 @@ struct Builder {
   }
   // a region holding several linears stacked along N (fused QKV, all cross-attn K/V, all time_emb_proj)
   size_t region(const std::string& key, size_t bytes) {
-    return entry("region:" + key, [&] { PackEntry e; e.kind = PK_F32_COPY; e.N = 0; e.off = pack_reserve(bytes); return e; }).off;
+    return entry(ctx->fwd, "region:" + key, [&] { PackEntry e; e.kind = PK_REGION; e.off = ctx->fwd.reserve(bytes); return e; }).off;
   }
   void linear_part(const std::string& module, size_t region_off, int row_off, int N, int K, bool lora) {
-    entry("lin:" + module, [&] {
+    entry(ctx->fwd, "lin:" + module, [&] {
       PackEntry e; e.kind = PK_LINEAR; e.src = module; e.N = N; e.C = K; e.ldo = K; e.lora = lora;
       e.off = region_off + size_t(row_off) * K * 2;
       return e;
     });
   }
   size_t linear_w(const std::string& module, int N, int K, bool lora) {
-    return entry("lin:" + module, [&] {
+    return entry(ctx->fwd, "lin:" + module, [&] {
       PackEntry e; e.kind = PK_LINEAR; e.src = module; e.N = N; e.C = K; e.ldo = K; e.lora = lora;
-      e.off = pack_reserve(size_t(N) * K * 2);
+      e.off = ctx->fwd.reserve(size_t(N) * K * 2);
       return e;
     }).off;
   }
   // mmcv ConvModule (conv without bias -> BatchNorm(eval) -> ReLU): BN scale folded into the packed weight rows, shift = epilogue bias
   struct ConvBn { size_t w_off, shift_off; };
   ConvBn conv_bn(const std::string& mod, int N, int C, int taps) {
-    const size_t fold = entry("bnfold:" + mod, [&] {
-      PackEntry e; e.kind = PK_BN_FOLD; e.src = mod + ".bn"; e.N = N; e.off = pack_reserve(size_t(2) * N * 4);
+    const size_t fold = entry(ctx->fwd, "bnfold:" + mod, [&] {
+      PackEntry e; e.kind = PK_BN_FOLD; e.src = mod + ".bn"; e.N = N; e.off = ctx->fwd.reserve(size_t(2) * N * 4);
       return e;
     }).off;
     const int Kpad = taps * C;
-    const size_t w = entry("convbn:" + mod, [&] {
+    const size_t w = entry(ctx->fwd, "convbn:" + mod, [&] {
       PackEntry e; e.kind = PK_CONV_BN; e.src = mod + ".conv.weight"; e.N = N; e.C = C; e.taps = taps; e.Cpad = C; e.Kpad = Kpad; e.ldo = Kpad;
-      e.bias_off = fold; e.off = pack_reserve(size_t(N) * Kpad * 2);
+      e.bias_off = fold; e.off = ctx->fwd.reserve(size_t(N) * Kpad * 2);
       return e;
     }).off;
     return ConvBn{w, fold + size_t(N) * 4};
   }
   // depthwise ConvModule: fp32 [9][C] weights (scale folded) + shift
   ConvBn depthwise_bn(const std::string& mod, int C) {
-    const size_t fold = entry("bnfold:" + mod, [&] {
-      PackEntry e; e.kind = PK_BN_FOLD; e.src = mod + ".bn"; e.N = C; e.off = pack_reserve(size_t(2) * C * 4);
+    const size_t fold = entry(ctx->fwd, "bnfold:" + mod, [&] {
+      PackEntry e; e.kind = PK_BN_FOLD; e.src = mod + ".bn"; e.N = C; e.off = ctx->fwd.reserve(size_t(2) * C * 4);
       return e;
     }).off;
-    const size_t w = entry("dwbn:" + mod, [&] {
-      PackEntry e; e.kind = PK_DW_BN; e.src = mod + ".conv.weight"; e.C = C; e.bias_off = fold; e.off = pack_reserve(size_t(9) * C * 4);
+    const size_t w = entry(ctx->fwd, "dwbn:" + mod, [&] {
+      PackEntry e; e.kind = PK_DW_BN; e.src = mod + ".conv.weight"; e.C = C; e.bias_off = fold; e.off = ctx->fwd.reserve(size_t(9) * C * 4);
       return e;
     }).off;
     return ConvBn{w, fold + size_t(C) * 4};
   }
   void f32_part(const std::string& name, size_t region_off, int elem_off, int n) {
-    entry("f32:" + name, [&] { PackEntry e; e.kind = PK_F32_COPY; e.src = name; e.N = n; e.off = region_off + size_t(elem_off) * 4; return e; });
+    entry(ctx->fwd, "f32:" + name, [&] {
+      PackEntry e; e.kind = PK_F32_COPY; e.src = name; e.N = n; e.off = region_off + size_t(elem_off) * 4;
+      return e;
+    });
   }
 
   // ---- op emission
@@ -636,59 +639,47 @@ struct Builder {
   }
 
   // ---- dgrad arena (training plans)
-  size_t dpack_reserve(size_t bytes) {
-    size_t off = ctx->dpacked_bytes;
-    ctx->dpacked_bytes += (bytes + 1023) & ~size_t(1023);
-    return off;
-  }
-  const DPackEntry& dentry(const std::string& key, const std::function<DPackEntry()>& make) {
-    auto it = ctx->dpack_index.find(key);
-    if (it != ctx->dpack_index.end()) return ctx->dpack[it->second];
-    if (mode != LAYOUT) fail(MADM_ESTATE, "dgrad entry missing from layout: " + key);
-    ctx->dpack.push_back(make());
-    ctx->dpack_index[key] = ctx->dpack.size() - 1;
-    return ctx->dpack.back();
-  }
   const bf16* dpw(size_t off) const { return dpacked ? reinterpret_cast<const bf16*>(dpacked + off) : nullptr; }
   // conv [Cout,Cin,k,k] -> [Cin, taps*Cout] (Cout % 64 == 0), the B operand of dX = dY (*) W^T
   size_t dconv_w(const std::string& name, int Cout, int Cin, int taps) {
-    return dentry("dconv:" + name, [&] {
-      DPackEntry e; e.kind = DG_CONV; e.src = name + ".weight"; e.N = Cout; e.C = Cin; e.taps = taps; e.CoPad = Cout; e.ldo = taps * Cout;
-      e.off = dpack_reserve(size_t(Cin) * taps * Cout * 2);
+    return entry(ctx->dgrad, "dconv:" + name, [&] {
+      PackEntry e; e.kind = PK_CONV_DGRAD; e.src = name + ".weight"; e.N = Cout; e.C = Cin; e.taps = taps; e.Cpad = Cout; e.Kpad = taps * Cout;
+      e.ldo = taps * Cout; e.off = ctx->dgrad.reserve(size_t(Cin) * taps * Cout * 2);
       return e;
     }).off;
   }
   size_t dregion(const std::string& key, size_t bytes) {
-    return dentry("dregion:" + key, [&] { DPackEntry e; e.kind = DG_REGION; e.off = dpack_reserve(bytes); return e; }).off;
+    return entry(ctx->dgrad, "dregion:" + key, [&] { PackEntry e; e.kind = PK_REGION; e.off = ctx->dgrad.reserve(bytes); return e; }).off;
   }
   // linear [N,K] (+LoRA) transposed into columns [col_off, col_off+N) of a [K, ldo] region
   void dlinear_part(const std::string& module, size_t region_off, int col_off, int N, int K, int ldo, bool lora) {
-    dentry("dlin:" + module, [&] {
-      DPackEntry e; e.kind = DG_LINEAR; e.src = module; e.N = N; e.C = K; e.ldo = ldo; e.lora = lora; e.off = region_off + size_t(col_off) * 2;
+    entry(ctx->dgrad, "dlin:" + module, [&] {
+      PackEntry e; e.kind = PK_LINEAR_T; e.src = module; e.N = N; e.C = K; e.ldo = ldo; e.lora = lora; e.off = region_off + size_t(col_off) * 2;
       return e;
     });
   }
   size_t dlinear_w(const std::string& module, int N, int K, bool lora) {
-    return dentry("dlin:" + module, [&] {
-      DPackEntry e; e.kind = DG_LINEAR; e.src = module; e.N = N; e.C = K; e.ldo = N; e.lora = lora; e.off = dpack_reserve(size_t(N) * K * 2);
+    return entry(ctx->dgrad, "dlin:" + module, [&] {
+      PackEntry e; e.kind = PK_LINEAR_T; e.src = module; e.N = N; e.C = K; e.ldo = N; e.lora = lora; e.off = ctx->dgrad.reserve(size_t(N) * K * 2);
       return e;
     }).off;
   }
+  // linear [N,K] in natural row order: the forward operand of ff.net.0.proj in the training forward
   size_t dlinear_fwd(const std::string& module, int N, int K) {
-    return dentry("dlinfwd:" + module, [&] {
-      DPackEntry e; e.kind = DG_LINEAR_FWD; e.src = module; e.N = N; e.C = K; e.ldo = K; e.off = dpack_reserve(size_t(N) * K * 2);
+    return entry(ctx->dgrad, "dlinfwd:" + module, [&] {
+      PackEntry e; e.kind = PK_LINEAR; e.src = module; e.N = N; e.C = K; e.ldo = K; e.off = ctx->dgrad.reserve(size_t(N) * K * 2);
       return e;
     }).off;
   }
   size_t dlora_a(const std::string& module, int K) {
-    return dentry("dloraA:" + module, [&] {
-      DPackEntry e; e.kind = DG_LORA_A; e.src = module; e.N = 16; e.C = K; e.ldo = K; e.off = dpack_reserve(size_t(16) * K * 2);
+    return entry(ctx->dgrad, "dloraA:" + module, [&] {
+      PackEntry e; e.kind = PK_LORA_A; e.src = module; e.N = 16; e.C = K; e.ldo = K; e.off = ctx->dgrad.reserve(size_t(16) * K * 2);
       return e;
     }).off;
   }
   size_t dlora_bt(const std::string& module, int N) {
-    return dentry("dloraB:" + module, [&] {
-      DPackEntry e; e.kind = DG_LORA_BT; e.src = module; e.N = N; e.C = 16; e.ldo = N; e.off = dpack_reserve(size_t(16) * N * 2);
+    return entry(ctx->dgrad, "dloraB:" + module, [&] {
+      PackEntry e; e.kind = PK_LORA_BT; e.src = module; e.N = N; e.C = 16; e.ldo = N; e.off = ctx->dgrad.reserve(size_t(16) * N * 2);
       return e;
     }).off;
   }
@@ -790,7 +781,7 @@ struct Model {
     // ---- backward
     const Act xa = x0, xb = x1 ? *x1 : Act();
     const bool has_b = x1 != nullptr;
-    b.tape.push_back([=]() {
+    b.tape.push_back({b.cur_stage, [=]() {
       // dgrad operands are registered whether or not this block ends up on the gradient path (the layout must not depend on it)
       const size_t w2 = b.dconv_w(p + ".conv2", Cout, Cout, 9), w1 = b.dconv_w(p + ".conv1", Cout, Cin, 9);
       const size_t wsc = shortcut ? b.dconv_w(p + ".conv_shortcut", Cout, Cin, 1) : 0;
@@ -827,7 +818,7 @@ struct Model {
         b.free(dn1);
       }
       b.free(dh1); b.free(g16);
-    });
+    }});
     return out;
   }
 
@@ -903,9 +894,9 @@ struct Model {
       const bf16* src = rawff.p; bf16* dst = ff.p; const int Hh = 4 * C;
       b.emit([=](cudaStream_t st) { return geglu_fwd(src, M, Hh, dst, h16, st); }, false, MADM_KIND_ELEMENTWISE, 0.0, double(M) * C * 24);
     } else {
-      const PackEntry& e = b.entry("geglu:" + tb, [&] {
+      const PackEntry& e = b.entry(b.ctx->fwd, "geglu:" + tb, [&] {
         PackEntry pe; pe.kind = PK_GEGLU; pe.src = tb + ".ff.net.0.proj.weight"; pe.src2 = tb + ".ff.net.0.proj.bias"; pe.N = 4 * C; pe.C = C;
-        pe.off = b.pack_reserve(size_t(8) * C * C * 2); pe.bias_off = b.pack_reserve(size_t(8) * C * 4);
+        pe.off = b.ctx->fwd.reserve(size_t(8) * C * C * 2); pe.bias_off = b.ctx->fwd.reserve(size_t(8) * C * 4);
         return pe; });
       GemmDesc d; d.seg[0] = Builder::seg_plain(l3.p, M, C); d.M = Mi; d.N = 4 * C; d.Nw = 8 * C; d.w = b.pw(e.off);
       d.bias = b.pf(e.bias_off); d.act = ACT_GEGLU; d.out_bf16 = ff.p; d.ldo16 = 4 * C; b.gemm(d);
@@ -928,7 +919,7 @@ struct Model {
     if (!train) return out;
     // ---- backward
     const Act xin = x;
-    b.tape.push_back([=]() {
+    b.tape.push_back({b.cur_stage, [=]() {
       const size_t w_po = b.dconv_w(p + ".proj_out", C, C, 1), w_pi = b.dconv_w(p + ".proj_in", C, C, 1);
       const size_t w_ff2 = b.dlinear_w(tb + ".ff.net.2", C, 4 * C, false), w_ff1 = b.dlinear_w(tb + ".ff.net.0.proj", 8 * C, C, false);
       const size_t w_o2 = b.dlinear_w(tb + ".attn2.to_out.0", C, C, true), w_q2 = b.dlinear_w(tb + ".attn2.to_q", C, C, true);
@@ -1013,7 +1004,7 @@ struct Model {
         b.free(dn);
       }
       b.free(dl); b.free(dh16); b.free(dh);
-    });
+    }});
     return out;
   }
 
@@ -1035,7 +1026,7 @@ struct Model {
       b.attach_colstats(out, d); b.gemm(d); }
     if (!b.recording()) return out;
     const Act xin = x;
-    b.tape.push_back([=]() {
+    b.tape.push_back({b.cur_stage, [=]() {
       const size_t w = b.dconv_w(p + ".conv", C, C, 9);
       if (!out.gr->written || !Builder::wants_grad(xin)) return;
       // input gradient of the stride-2 conv: zero-stuff d(out) onto the input grid, then the stride-1 dgrad GEMM with mirrored taps
@@ -1050,7 +1041,7 @@ struct Model {
         if (acc) { d.residual = dx; d.ldr = C; }
         d.out_f32 = dx; d.ldo32 = C; b.gemm(d); }
       b.free(z); b.free(g16);
-    });
+    }});
     return out;
   }
 
@@ -1074,7 +1065,7 @@ struct Model {
     b.free(up);
     if (!b.recording()) return out;
     const Act xin = x;
-    b.tape.push_back([=]() {
+    b.tape.push_back({b.cur_stage, [=]() {
       const size_t w = b.dconv_w(p + ".conv", C, C, 9);
       if (!out.gr->written || !Builder::wants_grad(xin)) return;
       const long Mo = out.M();
@@ -1087,7 +1078,7 @@ struct Model {
       float* dx = b.grad(xin, &acc);
       { const float* src = dup.p; b.emit([=](cudaStream_t st) { return sum2x2(src, Bn, H, W, C, dx, acc, st); }); }
       b.free(dup); b.free(g16);
-    });
+    }});
     return out;
   }
 
@@ -1244,9 +1235,9 @@ struct Model {
     B16T n = b.b16(size_t(x.M()) * 512);
     b.groupnorm(x, nullptr, e + "conv_norm_out", 1e-6f, ACT_SILU, n.p, nullptr);
     latents = b.f32(size_t(x.M()) * 4);
-    { const PackEntry& pe = b.entry("vae_head", [&] {
+    { const PackEntry& pe = b.entry(b.ctx->fwd, "vae_head", [&] {
         PackEntry q; q.kind = PK_VAE_HEAD; q.src = e + "conv_out.weight"; q.src2 = e + "conv_out.bias"; q.src3 = kVae + "quant_conv.weight";
-        q.src4 = kVae + "quant_conv.bias"; q.C = 512; q.off = b.pack_reserve(size_t(16) * 9 * 512 * 2); q.bias_off = b.pack_reserve(64);
+        q.src4 = kVae + "quant_conv.bias"; q.C = 512; q.off = b.ctx->fwd.reserve(size_t(16) * 9 * 512 * 2); q.bias_off = b.ctx->fwd.reserve(64);
         return q; });
       GemmDesc d; d.seg[0] = Builder::seg_3x3(n.p, Bn, x.H, x.W, 512); d.M = int(x.M()); d.N = 4; d.Nw = 16; d.w = b.pw(pe.off);
       d.bias = b.pf(pe.bias_off); d.out_f32 = latents.p; d.ldo32 = 4; d.bn = 16;
@@ -1321,7 +1312,7 @@ struct Model {
       d_temb_all = b.f32(size_t(Bn) * temb_total);
       dkv_all = b.b16(size_t(Bn) * 77 * kv_total);
       // ---- backward of the prologue (runs last): time path -> d(cond_emb), stacked K/V projections -> d(cond_inputs)
-      b.tape.push_back([=]() {
+      b.tape.push_back({b.cur_stage, [=]() {
         const size_t wt = b.dregion("temb_w", size_t(temb_total) * 1280 * 2);
         for (auto& l : temb_layers) b.dlinear_part(l.first + ".time_emb_proj", wt, temb_off[l.first], l.second, 1280, temb_total, false);
         const size_t wk = b.dregion("xattn_kv", size_t(kv_total) * 768 * 2);
@@ -1355,7 +1346,7 @@ struct Model {
               return scale_copy_f32(src, n, inv, io->b.d_cond_inputs, st); }); }
           b.free(dc);
         }
-      });
+      }});
     }
     // ---- conv_in (nothing trainable upstream: its output stops the gradient)
     Act x = b.act(Bn, 64, 64, 320, true, false);
@@ -1627,7 +1618,7 @@ struct Model {
       if (rgb3) { b.free(mom); b.free(coef1); b.free(coefs); }
       if (b.recording()) {
         // ---- backward
-        b.tape.push_back([=]() {
+        b.tape.push_back({b.cur_stage, [=]() {
           const size_t wd3 = b.dconv_w(p + "conv3", Cout, Cb, 1), wd2 = b.dconv_w(p + "conv2", Cb, Cb, 9);
           const size_t wd1 = b.dconv_w(p + "conv1", Cb, Cin, 1), wds = shortcut ? b.dconv_w(p + "shortcut", Cout, Cin, 1) : 0;
           const float S = b.loss_scale, inv = 1.0f / b.loss_scale;
@@ -1691,7 +1682,7 @@ struct Model {
             b.free(dsc);
           }
           b.free(dz);
-        });
+        }});
       }
     }
     b.cur_branch = 0;
@@ -1831,7 +1822,10 @@ struct Model {
       b.emit([=](cudaStream_t st) -> const char* {
         if (cudaMemsetAsync(dt, 0, nt, st) != cudaSuccess || cudaMemsetAsync(dk, 0, nk, st) != cudaSuccess) return "cudaMemsetAsync failed";
         return nullptr; }); }
-    for (auto it = b.tape.rbegin(); it != b.tape.rend(); ++it) (*it)();
+    for (auto it = b.tape.rbegin(); it != b.tape.rend(); ++it) {
+      b.cur_stage = it->first;  // the dgrad entries a backward registers belong to its forward's stage
+      it->second();
+    }
     b.bwd = false;
   }
 };
@@ -1847,16 +1841,6 @@ const char* Model::nchw_to_nhwc4(const float* src, int Bn, int HW, float* dst, c
   const long total = long(Bn) * HW;
   nchw_to_nhwc4_kernel<<<unsigned((total + 255) / 256), 256, 0, st>>>(src, Bn, HW, dst);
   return cudaGetLastError() == cudaSuccess ? nullptr : "nchw_to_nhwc4 launch failed";
-}
-
-__global__ void identity16_kernel(uint16_t* out, int N, int ldo, uint16_t one) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < N * N) out[size_t(i / N) * ldo + (i % N)] = (i / N == i % N) ? one : uint16_t(0);
-}
-
-__global__ void f32_sum2_kernel(const float* a, const float* b2, int n, float* out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = a[i] + b2[i];
 }
 
 int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st);
@@ -1915,8 +1899,8 @@ int build_plan(madm_ctx* ctx, const Builder& cfg, Plan* plan) {
 }
 
 int ensure_layout(madm_ctx* ctx) {
-  if (ctx->layout_done) return MADM_OK;
-  ctx->pack.clear(); ctx->pack_index.clear(); ctx->packed_bytes = 0;
+  if (ctx->fwd.done) return MADM_OK;
+  ctx->fwd = Arena();
   int rc = dry_run(ctx, LAYOUT, 1, nullptr);
   if (rc != MADM_OK) return rc;
   // EMA projection twins share the layout pass (registered only if the caller provided them)
@@ -1935,7 +1919,175 @@ int ensure_layout(madm_ctx* ctx) {
       return set_err(ctx, e.code, e.msg);
     }
   }
-  ctx->layout_done = true;
+  ctx->fwd.done = true;
+  return MADM_OK;
+}
+
+// The dgrad arena is laid out by a LAYOUT pass of the training traversal, which reads the forward arena's entries.
+int ensure_dlayout(madm_ctx* ctx) {
+  int rc = ensure_layout(ctx);
+  if (rc != MADM_OK) return rc;
+  if (ctx->dgrad.done) return MADM_OK;
+  ctx->dgrad = Arena();
+  rc = dry_run(ctx, LAYOUT, 1, nullptr, 0, 0, /*train=*/true);
+  if (rc != MADM_OK) return rc;
+  ctx->dgrad.done = true;
+  return MADM_OK;
+}
+
+// What a setter changed.  Each level drops everything the levels before it drop.
+enum Change {
+  GRAD_BUFFERS,    // training plans capture the gradient buffers
+  PARAM_POINTERS,  // every plan captures parameter pointers
+  LAYOUT_INPUTS,   // parameter shapes, operand dtype or variant: the arena layouts and the workspace sizes follow from them
+};
+void invalidate(madm_ctx* ctx, Change what) {
+  ctx->train_plans.clear();
+  if (what >= PARAM_POINTERS) {
+    ctx->plans.clear();
+    ctx->last_plan = nullptr;
+  }
+  if (what >= LAYOUT_INPUTS) {
+    ctx->fwd.done = false;
+    ctx->dgrad.done = false;
+    ctx->ws_bytes_cache.clear();
+  }
+}
+
+__global__ void identity16_kernel(uint16_t* out, int N, int ldo, uint16_t one) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < N * N) out[size_t(i / N) * ldo + (i % N)] = (i / N == i % N) ? one : uint16_t(0);
+}
+
+__global__ void f32_sum2_kernel(const float* a, const float* b2, int n, float* out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = a[i] + b2[i];
+}
+
+// Which entries of an arena a pack rewrites: all, the LoRA-targeted linears (adapter switch), or what an optimizer or EMA step can
+// change (PackEntry::trainable), in an arena that was fully packed before.
+enum Subset { PACK_ALL, PACK_LORA, PACK_TRAINABLE };
+
+// Packs the `subset` of `arena` into `base`, folding the LoRA adapter `ad` ("" = base weights) scaled by `scale`.
+int pack_arena(madm_ctx* ctx, const Arena& arena, uint8_t* base, const std::string& ad, float scale, Subset subset, cudaStream_t st) {
+  auto get = [&](const std::string& name) -> const ParamRef* {
+    auto it = ctx->params.find(name);
+    return it == ctx->params.end() ? nullptr : &it->second;
+  };
+  // a linear's weight: "<m>.base_layer.weight" if a LoRA adapter wraps it, else "<m>.weight"; folded with the active adapter's factors
+  // when wrapped (le.la = null and le.r = 0 otherwise)
+  auto linear = [&](const PackEntry& e, LoraPackEntry* le) -> int {
+    const ParamRef* w = get(e.src + ".base_layer.weight");
+    const bool wrapped = w != nullptr;
+    if (!w) w = get(e.src + ".weight");
+    if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src + ".weight");
+    if (w->numel() != int64_t(e.N) * e.C) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
+    *le = LoraPackEntry{w->p, nullptr, nullptr, base + e.off, e.N, e.C, 0, e.ldo};
+    if (wrapped && !ad.empty()) {
+      const ParamRef* A = get(e.src + ".lora_A." + ad + ".weight");
+      const ParamRef* Bm = get(e.src + ".lora_B." + ad + ".weight");
+      if (!A || !Bm) return set_err(ctx, MADM_ENOTFOUND, "LoRA adapter '" + ad + "' not registered for " + e.src);
+      le->r = int(A->shape[0]);
+      if (A->shape[1] != e.C || Bm->shape[0] != e.N || Bm->shape[1] != le->r) return set_err(ctx, MADM_EINVAL, "LoRA shape mismatch: " + e.src);
+      le->la = A->p; le->lb = Bm->p;
+    }
+    return MADM_OK;
+  };
+  std::vector<LoraPackEntry> multi[2];  // natural-order [0] / transposed [1] outputs of the multi-tensor pack kernel
+  for (const PackEntry& e : arena.entries) {
+    if ((subset == PACK_LORA && !e.lora) || (subset == PACK_TRAINABLE && !e.trainable)) continue;
+    const char* err = nullptr;
+    switch (e.kind) {
+      case PK_CONV: case PK_CONV_BN: case PK_CONV_DGRAD: {
+        const ParamRef* w = get(e.src);
+        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        if (w->numel() != int64_t(e.N) * e.C * e.taps) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
+        if (e.kind == PK_CONV_DGRAD) err = pack_conv_dgrad_weight(w->p, e.N, e.C, e.taps, e.Cpad, e.Kpad, e.ldo, base + e.off, ctx->fp16, st);
+        else err = pack_conv_weight(w->p, e.N, e.C, e.taps, e.Cpad, e.Kpad, e.ldo, base + e.off, ctx->fp16, st,
+                                    e.kind == PK_CONV_BN ? reinterpret_cast<const float*>(base + e.bias_off) : nullptr);
+        break;
+      }
+      case PK_LINEAR: case PK_LINEAR_T: {
+        LoraPackEntry le;
+        if (const int rc = linear(e, &le)) return rc;
+        const bool t = e.kind == PK_LINEAR_T;
+        if (e.lora && le.r <= 16) {  // the 128 LoRA-targeted projections: folded by the multi-tensor kernel after the loop
+          multi[t].push_back(le);
+          break;
+        }
+        err = (t ? pack_linear_dgrad_weight : pack_linear_weight)(le.w, e.N, e.C, le.la, le.lb, le.r, scale, e.ldo, base + e.off, ctx->fp16, st);
+        break;
+      }
+      case PK_LORA_A: case PK_LORA_BT: {
+        if (ad.empty()) break;
+        const ParamRef* f = get(e.src + (e.kind == PK_LORA_A ? ".lora_A." : ".lora_B.") + ad + ".weight");
+        if (!f) break;  // module not wrapped (zero-adapter configuration)
+        LoraPackEntry le{f->p, nullptr, nullptr, base + e.off, 0, 0, 0, e.ldo};
+        if (e.kind == PK_LORA_A) {
+          if (f->shape[0] != 16 || f->shape[1] != e.C) return set_err(ctx, MADM_EINVAL, "training path: lora_A must be [16, in]: " + e.src);
+          le.N = 16; le.K = e.C;
+          multi[0].push_back(le);  // [16, in] as is
+        } else {
+          if (f->shape[0] != e.N || f->shape[1] != 16) return set_err(ctx, MADM_EINVAL, "training path: lora_B must be [out, 16]: " + e.src);
+          le.N = e.N; le.K = 16;
+          multi[1].push_back(le);  // [out, 16] -> [16, out]
+        }
+        break;
+      }
+      case PK_GEGLU: {
+        const ParamRef* w = get(e.src); const ParamRef* bb = get(e.src2);
+        if (!w || !bb) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        err = pack_geglu_weight(w->p, bb->p, e.N, e.C, base + e.off, reinterpret_cast<float*>(base + e.bias_off), ctx->fp16, st);
+        break;
+      }
+      case PK_VAE_HEAD: {
+        const ParamRef *w = get(e.src), *b1 = get(e.src2), *wq = get(e.src3), *bq = get(e.src4);
+        if (!w || !b1 || !wq || !bq) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        err = pack_vae_latent_head(w->p, b1->p, wq->p, bq->p, 0.18215f, e.C, base + e.off, reinterpret_cast<float*>(base + e.bias_off),
+                                   ctx->fp16, st);
+        break;
+      }
+      case PK_F32_COPY: {
+        const ParamRef* s = get(e.src);
+        if (!s) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        if (cudaMemcpyAsync(base + e.off, s->p, size_t(e.N) * 4, cudaMemcpyDeviceToDevice, st) != cudaSuccess) err = "cudaMemcpyAsync failed";
+        break;
+      }
+      case PK_BN_FOLD: {
+        const ParamRef *g = get(e.src + ".weight"), *bt = get(e.src + ".bias"), *mu = get(e.src + ".running_mean"), *var = get(e.src + ".running_var");
+        if (!g || !bt || !mu || !var) return set_err(ctx, MADM_ENOTFOUND, "BatchNorm parameters / running statistics not registered: " + e.src);
+        if (g->numel() != e.N || bt->numel() != e.N || mu->numel() != e.N || var->numel() != e.N)
+          return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
+        err = bn_fold(g->p, bt->p, mu->p, var->p, nullptr, 1e-5f, e.N, reinterpret_cast<float*>(base + e.off), st);
+        break;
+      }
+      case PK_DW_BN: {
+        const ParamRef* w = get(e.src);
+        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        if (w->numel() != int64_t(e.C) * 9) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
+        err = pack_depthwise(w->p, reinterpret_cast<const float*>(base + e.bias_off), e.C, reinterpret_cast<float*>(base + e.off), st);
+        break;
+      }
+      case PK_IDENTITY: {
+        identity16_kernel<<<(e.N * e.N + 255) / 256, 256, 0, st>>>(reinterpret_cast<uint16_t*>(base + e.off), e.N, e.ldo,
+                                                                  ctx->fp16 ? uint16_t(0x3C00) : uint16_t(0x3F80));
+        if (cudaGetLastError() != cudaSuccess) err = "identity16 launch failed";
+        break;
+      }
+      case PK_F32_SUM2: {
+        const ParamRef *a = get(e.src), *b2 = get(e.src2);
+        if (!a || !b2) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
+        f32_sum2_kernel<<<(e.N + 255) / 256, 256, 0, st>>>(a->p, b2->p, e.N, reinterpret_cast<float*>(base + e.off));
+        if (cudaGetLastError() != cudaSuccess) err = "f32_sum2 launch failed";
+        break;
+      }
+      case PK_REGION: break;
+    }
+    if (err) return set_err(ctx, MADM_ECUDA, err);
+  }
+  for (int t = 0; t < 2; ++t)
+    if (!multi[t].empty())
+      if (const char* err = pack_lora_multi(multi[t].data(), int(multi[t].size()), scale, t, ctx->fp16, st)) return set_err(ctx, MADM_ECUDA, err);
   return MADM_OK;
 }
 
@@ -2006,12 +2158,7 @@ int madm_set_compute_dtype(madm_ctx* ctx, int32_t dtype) {
   const int f = dtype == MADM_DTYPE_FP16 ? 1 : 0;
   if (f != ctx->fp16) {
     ctx->fp16 = f;
-    ctx->plans.clear();
-    ctx->last_plan = nullptr;
-    ctx->layout_done = false;       // the packed layout depends on the operand dtype (16-bit VAE stream: identity segments)
-    ctx->dlayout_done = false;
-    ctx->train_plans.clear();
-    ctx->ws_bytes_cache.clear();
+    invalidate(ctx, LAYOUT_INPUTS);  // the packed layout depends on the operand dtype (16-bit VAE stream: identity segments)
   }
   return MADM_OK;
 }
@@ -2022,12 +2169,7 @@ int madm_set_variant(madm_ctx* ctx, int32_t variant) {
   if (!ctx || (variant != MADM_VARIANT_BASE && variant != MADM_VARIANT_S0)) return set_err(ctx, MADM_EINVAL, "madm_set_variant: bad argument");
   if (variant != ctx->variant) {
     ctx->variant = variant;
-    ctx->plans.clear();
-    ctx->train_plans.clear();
-    ctx->last_plan = nullptr;
-    ctx->layout_done = false;
-    ctx->dlayout_done = false;
-    ctx->ws_bytes_cache.clear();
+    invalidate(ctx, LAYOUT_INPUTS);
   }
   return MADM_OK;
 }
@@ -2043,138 +2185,29 @@ int madm_set_tensors(madm_ctx* ctx, const madm_tensor* named, int32_t n) {
     r.p = static_cast<const float*>(t.data);
     r.ndim = t.ndim;
     for (int k = 0; k < t.ndim; ++k) r.shape[k] = t.shape[k];
-    const bool is_new = ctx->params.find(t.name) == ctx->params.end();
+    auto it = ctx->params.find(t.name);
+    // a new name (adapters / EMA twins added) or a new shape under a known one: the model changed shape
+    if (it == ctx->params.end() || it->second.ndim != r.ndim || !std::equal(r.shape, r.shape + r.ndim, it->second.shape))
+      invalidate(ctx, LAYOUT_INPUTS);
     ctx->params[t.name] = r;
-    if (is_new && ctx->layout_done) {  // model changed shape (e.g. adapters / EMA twins added): rebuild layout and plans
-      ctx->layout_done = false;
-      ctx->dlayout_done = false;
-    }
   }
-  ctx->plans.clear();  // plans capture parameter pointers
-  ctx->train_plans.clear();
-  ctx->last_plan = nullptr;
+  invalidate(ctx, PARAM_POINTERS);
   return MADM_OK;
 }
 
 size_t madm_packed_bytes(madm_ctx* ctx) {
   if (!ctx) return 0;
   if (ensure_layout(ctx) != MADM_OK) return 0;
-  return ctx->packed_bytes;
+  return ctx->fwd.bytes;
 }
 
 int madm_pack_weights(madm_ctx* ctx, void* packed, const char* adapter, float scale, int32_t lora_only, madm_stream stream) {
   if (!ctx || !packed) return set_err(ctx, MADM_EINVAL, "madm_pack_weights: null argument");
   if (ctx->device < 0) return set_err(ctx, MADM_ECUDA, "madm_pack_weights: this context was created without a device (MADM_PLAN_ONLY)");
-  int rc = ensure_layout(ctx);
+  const int rc = ensure_layout(ctx);
   if (rc != MADM_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  uint8_t* base = static_cast<uint8_t*>(packed);
-  const std::string ad = adapter ? adapter : "";
-  auto get = [&](const std::string& name) -> const ParamRef* {
-    auto it = ctx->params.find(name);
-    return it == ctx->params.end() ? nullptr : &it->second;
-  };
-  auto is_proj = [](const std::string& s) { return s.rfind("feature_projections.", 0) == 0 || s.rfind("ema_feature_projections.", 0) == 0; };
-  std::vector<LoraPackEntry> multi;
-  for (const PackEntry& e : ctx->pack) {
-    const char* err = nullptr;
-    if (lora_only == 1 && !(e.kind == PK_LINEAR && e.lora)) continue;
-    if (lora_only == 2 && !((e.kind == PK_LINEAR && e.lora) || is_proj(e.src))) continue;  // the training step's trainable set
-    switch (e.kind) {
-      case PK_CONV: {
-        const ParamRef* w = get(e.src);
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        if (w->numel() != int64_t(e.N) * e.C * e.taps) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        err = pack_conv_weight(w->p, e.N, e.C, e.taps, e.Cpad, e.Kpad, e.ldo, base + e.off, ctx->fp16, st);
-        break;
-      }
-      case PK_LINEAR: {
-        const ParamRef* w = get(e.src + ".base_layer.weight");
-        const bool wrapped = w != nullptr;
-        if (!w) w = get(e.src + ".weight");
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src + ".weight");
-        if (w->numel() != int64_t(e.N) * e.C) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        const float *la = nullptr, *lb = nullptr;
-        int r = 0;
-        if (wrapped && !ad.empty()) {
-          const ParamRef* A = get(e.src + ".lora_A." + ad + ".weight");
-          const ParamRef* Bm = get(e.src + ".lora_B." + ad + ".weight");
-          if (!A || !Bm) return set_err(ctx, MADM_ENOTFOUND, "LoRA adapter '" + ad + "' not registered for " + e.src);
-          r = int(A->shape[0]);
-          if (A->shape[1] != e.C || Bm->shape[0] != e.N || Bm->shape[1] != r) return set_err(ctx, MADM_EINVAL, "LoRA shape mismatch: " + e.src);
-          la = A->p; lb = Bm->p;
-        }
-        if (e.lora && r <= 16) {  // the 128 LoRA-targeted projections: folded by the multi-tensor kernel after the loop
-          LoraPackEntry le; le.w = w->p; le.la = la; le.lb = lb; le.out = base + e.off; le.N = e.N; le.K = e.C; le.r = r; le.ldo = e.ldo;
-          multi.push_back(le);
-          break;
-        }
-        err = pack_linear_weight(w->p, e.N, e.C, la, lb, r, scale, e.ldo, base + e.off, ctx->fp16, st);
-        break;
-      }
-      case PK_GEGLU: {
-        const ParamRef* w = get(e.src); const ParamRef* bb = get(e.src2);
-        if (!w || !bb) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        err = pack_geglu_weight(w->p, bb->p, e.N, e.C, base + e.off, reinterpret_cast<float*>(base + e.bias_off), ctx->fp16, st);
-        break;
-      }
-      case PK_VAE_HEAD: {
-        const ParamRef *w = get(e.src), *b1 = get(e.src2), *wq = get(e.src3), *bq = get(e.src4);
-        if (!w || !b1 || !wq || !bq) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        err = pack_vae_latent_head(w->p, b1->p, wq->p, bq->p, 0.18215f, e.C, base + e.off, reinterpret_cast<float*>(base + e.bias_off),
-                                   ctx->fp16, st);
-        break;
-      }
-      case PK_F32_COPY: {
-        if (e.N == 0) break;  // pure region reservation
-        const ParamRef* s = get(e.src);
-        if (!s) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        if (cudaMemcpyAsync(base + e.off, s->p, size_t(e.N) * 4, cudaMemcpyDeviceToDevice, st) != cudaSuccess) err = "cudaMemcpyAsync failed";
-        break;
-      }
-      case PK_BN_FOLD: {
-        const ParamRef *g = get(e.src + ".weight"), *bt = get(e.src + ".bias"), *mu = get(e.src + ".running_mean"), *var = get(e.src + ".running_var");
-        if (!g || !bt || !mu || !var) return set_err(ctx, MADM_ENOTFOUND, "BatchNorm parameters / running statistics not registered: " + e.src);
-        if (g->numel() != e.N || bt->numel() != e.N || mu->numel() != e.N || var->numel() != e.N)
-          return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        err = bn_fold(g->p, bt->p, mu->p, var->p, nullptr, 1e-5f, e.N, reinterpret_cast<float*>(base + e.off), st);
-        break;
-      }
-      case PK_CONV_BN: {
-        const ParamRef* w = get(e.src);
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        if (w->numel() != int64_t(e.N) * e.C * e.taps) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        err = pack_conv_weight(w->p, e.N, e.C, e.taps, e.Cpad, e.Kpad, e.ldo, base + e.off, ctx->fp16, st,
-                               reinterpret_cast<const float*>(base + e.bias_off));
-        break;
-      }
-      case PK_DW_BN: {
-        const ParamRef* w = get(e.src);
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        if (w->numel() != int64_t(e.C) * 9) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        err = pack_depthwise(w->p, reinterpret_cast<const float*>(base + e.bias_off), e.C, reinterpret_cast<float*>(base + e.off), st);
-        break;
-      }
-      case PK_IDENTITY: {
-        identity16_kernel<<<(e.N * e.N + 255) / 256, 256, 0, st>>>(reinterpret_cast<uint16_t*>(base + e.off), e.N, e.ldo,
-                                                                  ctx->fp16 ? uint16_t(0x3C00) : uint16_t(0x3F80));
-        if (cudaGetLastError() != cudaSuccess) err = "identity16 launch failed";
-        break;
-      }
-      case PK_F32_SUM2: {
-        const ParamRef *a = get(e.src), *b2 = get(e.src2);
-        if (!a || !b2) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        f32_sum2_kernel<<<(e.N + 255) / 256, 256, 0, st>>>(a->p, b2->p, e.N, reinterpret_cast<float*>(base + e.off));
-        if (cudaGetLastError() != cudaSuccess) err = "f32_sum2 launch failed";
-        break;
-      }
-      default: break;
-    }
-    if (err) return set_err(ctx, MADM_ECUDA, err);
-  }
-  if (!multi.empty())
-    if (const char* err = pack_lora_multi(multi.data(), int(multi.size()), scale, 0, ctx->fp16, st)) return set_err(ctx, MADM_ECUDA, err);
-  return MADM_OK;
+  const Subset subset = lora_only == 1 ? PACK_LORA : lora_only == 2 ? PACK_TRAINABLE : PACK_ALL;
+  return pack_arena(ctx, ctx->fwd, static_cast<uint8_t*>(packed), adapter ? adapter : "", scale, subset, static_cast<cudaStream_t>(stream));
 }
 
 size_t madm_workspace_bytes(madm_ctx* ctx, int32_t B) { return madm_workspace_bytes_head(ctx, B, 0, 0); }
@@ -2325,9 +2358,6 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------------ training path (SURVEY §8 row f-3)
-namespace {
-int ensure_dlayout(madm_ctx* ctx);
-}
 extern "C" size_t madm_train_workspace_bytes(madm_ctx* ctx, int32_t B, const char* adapter);
 namespace {
 // madm_extract with MADM_FLAG_TRAIN: the forward of a training plan (activations kept for madm_backward)
@@ -2373,18 +2403,6 @@ int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
   return MADM_OK;
 }
 }  // namespace
-namespace {
-int ensure_dlayout(madm_ctx* ctx) {
-  int rc = ensure_layout(ctx);
-  if (rc != MADM_OK) return rc;
-  if (ctx->dlayout_done) return MADM_OK;
-  ctx->dpack.clear(); ctx->dpack_index.clear(); ctx->dpacked_bytes = 0;
-  rc = dry_run(ctx, LAYOUT, 1, nullptr, 0, 0, /*train=*/true);
-  if (rc != MADM_OK) return rc;
-  ctx->dlayout_done = true;
-  return MADM_OK;
-}
-}  // namespace
 
 extern "C" {
 
@@ -2400,93 +2418,22 @@ int madm_set_grad_tensors(madm_ctx* ctx, const madm_tensor* named, int32_t n) {
     if (numel != it->second.numel()) return set_err(ctx, MADM_EINVAL, std::string("madm_set_grad_tensors: shape mismatch: ") + named[i].name);
     ctx->grads[named[i].name] = static_cast<float*>(const_cast<void*>(named[i].data));
   }
-  ctx->train_plans.clear();  // plans capture the gradient pointers
-  ctx->train_ws_cache.clear();
+  invalidate(ctx, GRAD_BUFFERS);
   return MADM_OK;
 }
 
 size_t madm_dgrad_packed_bytes(madm_ctx* ctx) {
   if (!ctx || ensure_dlayout(ctx) != MADM_OK) return 0;
-  return ctx->dpacked_bytes;
+  return ctx->dgrad.bytes;
 }
 
 int madm_pack_dgrad_weights(madm_ctx* ctx, void* packed, const char* adapter, float scale, int32_t trainable_only, madm_stream stream) {
   if (!ctx || !packed) return set_err(ctx, MADM_EINVAL, "madm_pack_dgrad_weights: null argument");
   if (ctx->device < 0) return set_err(ctx, MADM_ECUDA, "madm_pack_dgrad_weights: this context was created without a device (MADM_PLAN_ONLY)");
-  int rc = ensure_dlayout(ctx);
+  const int rc = ensure_dlayout(ctx);
   if (rc != MADM_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  uint8_t* base = static_cast<uint8_t*>(packed);
-  const std::string ad = adapter ? adapter : "";
-  auto get = [&](const std::string& name) -> const ParamRef* {
-    auto it = ctx->params.find(name);
-    return it == ctx->params.end() ? nullptr : &it->second;
-  };
-  std::vector<LoraPackEntry> multi_t, multi_n;  // transposed / natural outputs of the multi-tensor pack kernel
-  for (const DPackEntry& e : ctx->dpack) {
-    const char* err = nullptr;
-    if (trainable_only) {  // only what an optimizer step / adapter switch can change: LoRA-folded linears, LoRA factors, projection convs
-      const bool hit = (e.kind == DG_LINEAR && e.lora) || e.kind == DG_LORA_A || e.kind == DG_LORA_BT ||
-                       (e.kind == DG_CONV && e.src.rfind("feature_projections.", 0) == 0);
-      if (!hit) continue;
-    }
-    switch (e.kind) {
-      case DG_CONV: {
-        const ParamRef* w = get(e.src);
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src);
-        if (w->numel() != int64_t(e.N) * e.C * e.taps) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        err = pack_conv_dgrad_weight(w->p, e.N, e.C, e.taps, e.CoPad, e.taps * e.CoPad, e.ldo, base + e.off, ctx->fp16, st);
-        break;
-      }
-      case DG_LINEAR: case DG_LINEAR_FWD: {
-        const ParamRef* w = get(e.src + ".base_layer.weight");
-        const bool wrapped = w != nullptr;
-        if (!w) w = get(e.src + ".weight");
-        if (!w) return set_err(ctx, MADM_ENOTFOUND, "parameter not registered: " + e.src + ".weight");
-        if (w->numel() != int64_t(e.N) * e.C) return set_err(ctx, MADM_EINVAL, "unexpected shape: " + e.src);
-        const float *la = nullptr, *lb = nullptr;
-        int r = 0;
-        if (e.lora && wrapped && !ad.empty()) {
-          const ParamRef* A = get(e.src + ".lora_A." + ad + ".weight");
-          const ParamRef* Bm = get(e.src + ".lora_B." + ad + ".weight");
-          if (!A || !Bm) return set_err(ctx, MADM_ENOTFOUND, "LoRA adapter '" + ad + "' not registered for " + e.src);
-          r = int(A->shape[0]);
-          la = A->p; lb = Bm->p;
-        }
-        if (e.kind == DG_LINEAR && e.lora && r <= 16) {
-          LoraPackEntry le; le.w = w->p; le.la = la; le.lb = lb; le.out = base + e.off; le.N = e.N; le.K = e.C; le.r = r; le.ldo = e.ldo;
-          multi_t.push_back(le);
-          break;
-        }
-        if (e.kind == DG_LINEAR) err = pack_linear_dgrad_weight(w->p, e.N, e.C, la, lb, r, scale, e.ldo, base + e.off, ctx->fp16, st);
-        else err = pack_linear_weight(w->p, e.N, e.C, nullptr, nullptr, 0, 0.f, e.ldo, base + e.off, ctx->fp16, st);
-        break;
-      }
-      case DG_LORA_A: case DG_LORA_BT: {
-        if (ad.empty()) break;
-        const ParamRef* f = get(e.src + (e.kind == DG_LORA_A ? ".lora_A." : ".lora_B.") + ad + ".weight");
-        if (!f) break;  // module not wrapped (zero-adapter configuration)
-        LoraPackEntry le; le.w = f->p; le.la = nullptr; le.lb = nullptr; le.out = base + e.off; le.r = 0; le.ldo = e.ldo;
-        if (e.kind == DG_LORA_A) {
-          if (f->shape[0] != 16 || f->shape[1] != e.C) return set_err(ctx, MADM_EINVAL, "training path: lora_A must be [16, in]: " + e.src);
-          le.N = 16; le.K = e.C;
-          multi_n.push_back(le);  // [16, in] as is
-        } else {
-          if (f->shape[0] != e.N || f->shape[1] != 16) return set_err(ctx, MADM_EINVAL, "training path: lora_B must be [out, 16]: " + e.src);
-          le.N = e.N; le.K = 16;
-          multi_t.push_back(le);  // [out, 16] -> [16, out]
-        }
-        break;
-      }
-      default: break;
-    }
-    if (err) return set_err(ctx, MADM_ECUDA, err);
-  }
-  if (!multi_t.empty())
-    if (const char* err = pack_lora_multi(multi_t.data(), int(multi_t.size()), scale, 1, ctx->fp16, st)) return set_err(ctx, MADM_ECUDA, err);
-  if (!multi_n.empty())
-    if (const char* err = pack_lora_multi(multi_n.data(), int(multi_n.size()), scale, 0, ctx->fp16, st)) return set_err(ctx, MADM_ECUDA, err);
-  return MADM_OK;
+  return pack_arena(ctx, ctx->dgrad, static_cast<uint8_t*>(packed), adapter ? adapter : "", scale, trainable_only ? PACK_TRAINABLE : PACK_ALL,
+                    static_cast<cudaStream_t>(stream));
 }
 
 size_t madm_train_workspace_bytes(madm_ctx* ctx, int32_t B, const char* adapter) {

@@ -54,16 +54,16 @@ def max_rel(a, b):
     return ((a.double() - b.double()).abs().max() / b.double().abs().max()).item()
 
 
-def meta_training_params():
+def meta_training_params(proj_width=128):
     """(state_dict name, meta tensor) pairs of the host-only training dry runs: UNet with the LoRA adapters 'default' and 'Depth' (r = 16),
-    VAE encoder, four GN-bottleneck projections (512 / 320 / 640 / 1280 -> 512)."""
+    VAE encoder, four GN-bottleneck projections (512 / 320 / 640 / 1280 -> 512, bottleneck width proj_width)."""
     from madm_b200.sd14_params import BottleneckParams, UNetParams, VAEParams, empty_init
     with empty_init():
         unet, vae = UNetParams(device="meta"), VAEParams(device="meta")
         for name in ("default", "Depth"):
             unet.add_adapter(SimpleNamespace(r=16, lora_alpha=16, init_lora_weights="gaussian",
                                              target_modules=["to_k", "to_q", "to_v", "to_out.0"]), name)
-        projs = [BottleneckParams(c, 512, 128, device="meta") for c in (512, 320, 640, 1280)]
+        projs = [BottleneckParams(c, 512, proj_width, device="meta") for c in (512, 320, 640, 1280)]
     named = [("feature_extractor.ldm_extractor.unet." + n, p) for n, p in unet.named_parameters()]
     named += [("feature_extractor.ldm_extractor.vae." + n, p) for n, p in vae.named_parameters()]
     for i, pr in enumerate(projs):
