@@ -110,29 +110,35 @@ struct Act {
   long M() const { return long(B) * H * W; }
 };
 
+// One kernel launch of a plan and what the profile accounts to it
+struct Launch {
+  Op run;
+  int stage;          // MADM_STAGE_* bit
+  int branch;         // 0 = the caller's stream; 1..4 = independent projection branches (run on side streams, forked / joined by events)
+  int kind;           // MADM_KIND_*
+  bool optional;      // debug/taps launch that does work only when the caller asks for the extra output
+  double flops;       // algorithmic FLOPs (2*MAC of the reference's convs / linears: no K padding, no identity segments)
+  double exec_flops;  // FLOPs the launch executes (padded K, identity-weight residual segments, GEGLU both halves)
+  double bytes;       // algorithmic HBM bytes (HBM-bound kernels)
+};
+
+// Heap-allocated and never moved: its launches point into `io`.
 struct Plan {
-  int B = 0;
-  bool ema = false;
   const void* packed = nullptr;
   void* ws = nullptr;
   size_t ws_bytes = 0;
-  std::vector<Op> ops;
-  std::vector<Op> bops;       // training plans: the backward pass (replayed by madm_backward)
+  std::vector<Launch> ops;
+  std::vector<Launch> bops;   // training plans: the backward pass (replayed by madm_backward)
   bool train = false;
   const void* dpacked = nullptr;
   float loss_scale = 1.0f, lora_scale = 0.f;
   std::string adapter;
-  std::vector<int> stage_of;  // stage bit per op
-  std::vector<int> branch;    // 0 = the caller's stream; 1..4 = independent projection branches (run on side streams, forked / joined by events)
-  std::vector<char> optional; // debug/taps ops that launch only when the caller asks for the extra output
-  std::vector<int> kind;      // MADM_KIND_* per op
-  std::vector<double> flops;  // algorithmic FLOPs per op (2*MAC of the reference's convs / linears: no K padding, no identity segments)
-  std::vector<double> exec_flops;  // FLOPs the launch executes (padded K, identity-weight residual segments, GEGLU both halves)
-  std::vector<double> bytes;  // algorithmic HBM bytes per op (HBM-bound kernels)
   std::vector<cudaEvent_t> ev;  // 2 per op, created on demand when profiling
+  Plan() = default;
+  Plan(const Plan&) = delete;
   ~Plan() { for (cudaEvent_t e : ev) cudaEventDestroy(e); }
-  std::shared_ptr<IoBind> io = std::make_shared<IoBind>();
-  size_t stats_off = 0, stats_bytes = 0;
+  IoBind io;
+  size_t stats_bytes = 0;
 };
 
 }  // namespace
@@ -174,12 +180,15 @@ struct BuildError {
 //   PLAN:   emit launches with real pointers
 enum Mode { LAYOUT, SIZE, PLAN };
 
+IoBind dry_io;  // what the launches of a dry pass would read: they are not kept, so nothing reads it
+
 struct Builder {
   madm_ctx* ctx;
   Mode mode;
   int B;
   bool ema;
   Plan* plan = nullptr;
+  IoBind* io = &dry_io;  // per-call pointers the launches read (the plan's in PLAN mode)
   uint8_t* ws = nullptr;
   const uint8_t* packed = nullptr;
   int cur_stage = MADM_STAGE_VAE;
@@ -441,20 +450,9 @@ struct Builder {
 
   // ---- op emission
   void emit(Op op, bool optional = false, int kind = MADM_KIND_ELEMENTWISE, double flops = 0.0, double bytes = 0.0, double exec_flops = -1.0) {
-    if (bwd) {
-      if (mode == PLAN) plan->bops.push_back(std::move(op));
-      return;
-    }
-    if (mode == PLAN) {
-      plan->ops.push_back(std::move(op));
-      plan->stage_of.push_back(cur_stage);
-      plan->branch.push_back(cur_branch);
-      plan->optional.push_back(optional ? 1 : 0);
-      plan->kind.push_back(kind);
-      plan->flops.push_back(flops);
-      plan->exec_flops.push_back(exec_flops < 0 ? flops : exec_flops);
-      plan->bytes.push_back(bytes);
-    }
+    if (mode != PLAN) return;
+    (bwd ? plan->bops : plan->ops)
+        .push_back(Launch{std::move(op), cur_stage, cur_branch, kind, optional, flops, exec_flops < 0 ? flops : exec_flops, bytes});
   }
   // algo_flops < 0: 2*M*N*K from the descriptor (K counts real channels only when k_real is given)
   // split-K factor for a GEMM whose M x N tiling cannot fill the 148 SMs (8x8-resolution convs, small batches): the K range
@@ -487,24 +485,30 @@ struct Builder {
   }
   void gemm(const GemmDesc& d0, double algo_flops = -1.0) {
     const int splits = choose_splits(d0);
-    if (splits > 1) {  // identical allocation sequence in every builder mode
-      F32T part = f32(size_t(splits) * d0.M * d0.N);
-      if (mode == PLAN) {
-        GemmDesc d = d0;
-        d.fp16 = ctx->fp16;
+    F32T part;
+    if (splits > 1) part = f32(size_t(splits) * d0.M * d0.N);  // identical allocation sequence in every builder mode
+    if (mode == PLAN) {
+      GemmDesc d = d0;
+      d.fp16 = ctx->fp16;
+      if (splits > 1) {  // raw fp32 partials; splitk_reduce applies the epilogue
         d.bias = nullptr; d.rowbias = nullptr; d.residual = nullptr; d.res16 = 0; d.out_bf16 = nullptr; d.act = ACT_NONE; d.colstats = nullptr; d.alpha = 1.0f;
         d.out_f32 = part.p; d.ldo32 = d0.N; d.splits = splits; d.split_stride = long(d0.M) * d0.N; d.bn = 128;
-        GemmLaunch L;
-        if (const char* e = gemm_prepare(d, &L)) fail(MADM_EINVAL, std::string(e));
-        double K = 0;
-        for (int sgi = 0; sgi < d.nseg; ++sgi) K += double(d.seg[sgi].ntaps) * d.seg[sgi].C;
-        const double exec = 2.0 * double(d.M) * d.N * K;
-        if (algo_flops < 0) algo_flops = exec;
-        if (getenv("MADM_DUMP_PLAN"))
-          fprintf(stderr, "MADM_PLAN gemm M=%d N=%d K=%d bn=%d tiles=%d taps=%d nseg=%d act=%d res=%d f32=%d h16=%d gflop=%.3f splits=%d tma=%d stats=0\n", d.M, d.N,
-                  int(K), L.bn, L.num_tiles, d.seg[0].ntaps, d.nseg, d0.act, d0.residual ? 1 : 0, d0.out_f32 ? 1 : 0, d0.out_bf16 ? 1 : 0,
-                  algo_flops / 1e9, splits, L.tma_epi);
-        emit([L](cudaStream_t st) { return gemm_launch(L, st); }, false, MADM_KIND_GEMM, algo_flops, gemm_algo_bytes(d), exec);
+      }
+      GemmLaunch L;
+      if (const char* e = gemm_prepare(d, &L)) fail(MADM_EINVAL, std::string(e));
+      double K = 0;
+      for (int sgi = 0; sgi < d.nseg; ++sgi) K += double(d.seg[sgi].ntaps) * d.seg[sgi].C;
+      const double exec = 2.0 * double(d.M) * ((d.act == ACT_GEGLU) ? 2.0 * d.N : double(d.N)) * K;
+      if (algo_flops < 0) algo_flops = exec;
+      if (getenv("MADM_DUMP_PLAN")) {  // tools/layer_report.py parses these lines
+        char tail[48];
+        if (splits > 1) snprintf(tail, sizeof(tail), "splits=%d tma=%d stats=0", splits, L.tma_epi);
+        else snprintf(tail, sizeof(tail), "tma=%d stats=%d", L.tma_epi, (d.colstats ? 1 : 0) | (d.s2d_W > 0 ? 2 : 0));
+        fprintf(stderr, "MADM_PLAN gemm M=%d N=%d K=%d bn=%d tiles=%d taps=%d nseg=%d act=%d res=%d f32=%d h16=%d gflop=%.3f %s\n", d.M, d.N, int(K), L.bn,
+                L.num_tiles, d.seg[0].ntaps, d.nseg, d0.act, d0.residual ? 1 : 0, d0.out_f32 ? 1 : 0, d0.out_bf16 ? 1 : 0, algo_flops / 1e9, tail);
+      }
+      emit([L](cudaStream_t st) { return gemm_launch(L, st); }, false, MADM_KIND_GEMM, algo_flops, gemm_algo_bytes(d), exec);
+      if (splits > 1) {
         const GemmDesc e0 = d0; const float* pp = part.p; const int f16 = ctx->fp16; const long ss = d.split_stride;
         if (e0.alpha != 1.0f) fail(MADM_EINVAL, "split-K with alpha != 1 is not supported");
         emit([=](cudaStream_t st) {
@@ -512,30 +516,8 @@ struct Builder {
                                e0.ldo32, e0.out_bf16, e0.ldo16, e0.act, f16, st, e0.res16);
         }, false, MADM_KIND_ELEMENTWISE, 0.0, double(splits + 2) * e0.M * e0.N * 4);
       }
-      free(part);
-      return;
     }
-    if (mode != PLAN) return;
-    GemmDesc d = d0;
-    d.fp16 = ctx->fp16;
-    GemmLaunch L;
-    if (const char* e = gemm_prepare(d, &L)) fail(MADM_EINVAL, std::string(e));
-    double exec;
-    {
-      double K = 0;
-      for (int sgi = 0; sgi < d.nseg; ++sgi) K += double(d.seg[sgi].ntaps) * d.seg[sgi].C;
-      const double N = (d.act == ACT_GEGLU) ? 2.0 * d.N : double(d.N);
-      exec = 2.0 * double(d.M) * N * K;
-    }
-    if (algo_flops < 0) algo_flops = exec;
-    if (getenv("MADM_DUMP_PLAN")) {
-      int K = 0;
-      for (int sgi = 0; sgi < d.nseg; ++sgi) K += d.seg[sgi].ntaps * d.seg[sgi].C;
-      fprintf(stderr, "MADM_PLAN gemm M=%d N=%d K=%d bn=%d tiles=%d taps=%d nseg=%d act=%d res=%d f32=%d h16=%d gflop=%.3f tma=%d stats=%d\n", d.M, d.N, K, L.bn,
-              L.num_tiles, d.seg[0].ntaps, d.nseg, d.act, d.residual ? 1 : 0, d.out_f32 ? 1 : 0, d.out_bf16 ? 1 : 0, algo_flops / 1e9, L.tma_epi,
-              (d.colstats ? 1 : 0) | (d.s2d_W > 0 ? 2 : 0));
-    }
-    emit([L](cudaStream_t st) { return gemm_launch(L, st); }, false, MADM_KIND_GEMM, algo_flops, gemm_algo_bytes(d), exec);
+    if (splits > 1) free(part);
   }
 
   // fused attention: tcgen05/TMEM kernel (tensor maps encoded at plan time)
@@ -689,7 +671,6 @@ struct Builder {
 struct Model {
   Builder& b;
   explicit Model(Builder& bb) : b(bb) {}
-  bool dry() const { return b.mode != PLAN; }
   int f16() const { return b.ctx->fp16; }
   const float* P(const std::string& n, int64_t numel = -1) { return b.mode == LAYOUT ? nullptr : b.param(n, numel); }
 
@@ -744,8 +725,7 @@ struct Model {
       GemmDesc d; d.seg[0] = Builder::seg_3x3(n1.p, Bn, H, W, Cin); d.M = int(x0.M()); d.N = Cout;
       d.w = b.pw(b.conv_w(p + ".conv1", Cout, Cin, 9)); d.Nw = Cout;
       d.bias = P(p + ".conv1.bias", Cout);
-      if (has_temb) { d.rowbias = temb_all.p ? temb_all.p + temb_off[p] : nullptr; d.ld_rowbias = temb_total; d.rows_per_img = H * W;
-                      if (dry()) d.rowbias = nullptr; }
+      if (has_temb) { d.rowbias = temb_all.p ? temb_all.p + temb_off[p] : nullptr; d.ld_rowbias = temb_total; d.rows_per_img = H * W; }
       d.out_bf16 = h1.h.p; d.ldo16 = Cout;
       b.attach_colstats(h1, d);  // norm2 statistics come out of this epilogue
       b.gemm(d);
@@ -1134,8 +1114,7 @@ struct Model {
   Act unet_tap[3];       // 64x64x320, 32x32x640, 16x16x1280 (fp32 + bf16)
 
   void nchw_debug(const Act& a, int which) {  // taps[which] if requested
-    if (dry()) { b.emit(nullptr, true); return; }
-    std::shared_ptr<IoBind> io = b.plan->io;
+    IoBind* io = b.io;
     const float* src = a.f.p; const int Bn = a.B, HW = a.HW(), C = a.C;
     b.emit([=](cudaStream_t st) -> const char* {
       float* dst = io->a.taps[which];
@@ -1188,10 +1167,9 @@ struct Model {
     b.cur_stage = MADM_STAGE_VAE;
     const int Bn = b.B, R = 512;
     const std::string e = kVae + "encoder.";
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
+    IoBind* io = b.io;
     B16T col = b.b16(size_t(Bn) * R * R * 64);
-    if (dry()) b.emit(nullptr);
-    else { bf16* dst = col.p; const int h16 = f16();
+    { bf16* dst = col.p; const int h16 = f16();
       b.emit([=](cudaStream_t st) { return image_im2col(io->a.img, Bn, R, R, dst, io->a.range_flag, h16, st, io->a.flags & MADM_FLAG_IMG_NORMALISED); }); }
     // fp16 operands: the residual stream of the 512^2 and 256^2 stages (3/4 of the VAE's bytes) is kept in fp16 like the
     // reference's VAE (AutoencoderKL loaded with torch_dtype=float16, ldm_diffusers.py:246-249); bf16 keeps the fp32 stream.
@@ -1244,8 +1222,7 @@ struct Model {
       b.gemm(d, 2.0 * double(d.M) * 8 * (9 * 512 + 8)); }  // algorithmic: conv_out 512->8 (3x3) + quant_conv 8->8
     b.free(n);
     b.free(x);
-    if (dry()) b.emit(nullptr, true);
-    else { const float* src = latents.p;
+    { const float* src = latents.p;
       b.emit([=](cudaStream_t st) -> const char* {
         return io->a.latents ? nhwc_to_nchw(src, Bn, 64 * 64, 4, io->a.latents, st) : nullptr; }, true); }
   }
@@ -1254,12 +1231,11 @@ struct Model {
   void build_unet() {
     b.cur_stage = MADM_STAGE_UNET;
     const int Bn = b.B;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
+    IoBind* io = b.io;
     // ---- q-sample (or external noisy latents) + conv_in im2col
     F32T noisy = b.f32(size_t(Bn) * 4096 * 4);
     B16T col = b.b16(size_t(Bn) * 4096 * 64);
-    if (dry()) { b.emit(nullptr); b.emit(nullptr); }
-    else {
+    {
       const float* lat = latents.p; float* nz = noisy.p; bf16* cdst = col.p; const float* ac = b.ctx->alphas_cumprod;
       b.emit([=](cudaStream_t st) -> const char* {
         if (io->a.noisy_latents_in) return nchw_to_nhwc4(io->a.noisy_latents_in, Bn, 4096, nz, st);
@@ -1270,8 +1246,7 @@ struct Model {
     }
     // ---- time embedding: sinusoid -> linear_1 -> SiLU -> linear_2 (+ cond_emb) -> SiLU -> all 22 time_emb_proj at once
     B16T sinus = b.b16(size_t(Bn) * 320);
-    if (dry()) b.emit(nullptr);
-    else { bf16* dst = sinus.p; const int h16 = f16(); b.emit([=](cudaStream_t st) { return timestep_sinusoid(io->a.timesteps, Bn, dst, h16, st); }); }
+    { bf16* dst = sinus.p; const int h16 = f16(); b.emit([=](cudaStream_t st) { return timestep_sinusoid(io->a.timesteps, Bn, dst, h16, st); }); }
     B16T e1 = b.b16(size_t(Bn) * 1280);
     { GemmDesc d; d.seg[0] = Builder::seg_plain(sinus.p, Bn, 320); d.M = Bn; d.N = 1280; d.Nw = 1280;
       d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_1", 1280, 320, false)); d.bias = P(kUnet + "time_embedding.linear_1.bias", 1280);
@@ -1281,8 +1256,7 @@ struct Model {
       d.w = b.pw(b.linear_w(kUnet + "time_embedding.linear_2", 1280, 1280, false)); d.bias = P(kUnet + "time_embedding.linear_2.bias", 1280);
       d.out_f32 = emb_saved.p; d.ldo32 = 1280; b.gemm(d); }
     B16T emb_act = b.b16(size_t(Bn) * 1280);
-    if (dry()) b.emit(nullptr);
-    else { const float* src = emb_saved.p; bf16* dst = emb_act.p; const int h16 = f16();
+    { const float* src = emb_saved.p; bf16* dst = emb_act.p; const int h16 = f16();
       b.emit([=](cudaStream_t st) { return f32_to_bf16(src, io->a.cond_emb, long(Bn) * 1280, ACT_SILU, dst, nullptr, h16, st); }); }
     temb_all = b.f32(size_t(Bn) * temb_total);
     { const size_t reg = b.region("temb_w", size_t(temb_total) * 1280 * 2);
@@ -1296,8 +1270,7 @@ struct Model {
     b.free(sinus); b.free(e1); b.free(emb_saved); b.free(emb_act);
     // ---- cross-attention K/V of every transformer block in one GEMM
     ctx16_saved = b.b16(size_t(Bn) * 77 * 768);
-    if (dry()) b.emit(nullptr);
-    else { bf16* dst = ctx16_saved.p; const int h16 = f16();
+    { bf16* dst = ctx16_saved.p; const int h16 = f16();
       b.emit([=](cudaStream_t st) { return f32_to_bf16(io->a.cond_inputs, nullptr, long(Bn) * 77 * 768, ACT_NONE, dst, nullptr, h16, st); }); }
     kv_all = b.b16(size_t(Bn) * 77 * kv_total);
     { const size_t reg = b.region("xattn_kv", size_t(kv_total) * 768 * 2);
@@ -1327,8 +1300,7 @@ struct Model {
           F32T dact = b.f32(size_t(Bn) * 1280);
           { GemmDesc d; d.seg[0] = Builder::seg_plain(dt16.p, Bn, temb_total); d.M = Bn; d.N = 1280; d.Nw = 1280; d.w = b.dpw(wt);
             d.out_f32 = dact.p; d.ldo32 = 1280; b.gemm(d); }
-          if (dry()) b.emit(nullptr);
-          else { const float* da = dact.p; const float* em = emb_saved.p;
+          { const float* da = dact.p; const float* em = emb_saved.p;
             b.emit([=](cudaStream_t st) -> const char* {
               if (!io->b.d_cond_emb) return nullptr;
               if (!io->b.cond_emb) return "madm_backward: cond_emb is required for d_cond_emb";
@@ -1339,8 +1311,7 @@ struct Model {
           F32T dc = b.f32(size_t(Bn) * 77 * 768);
           { GemmDesc d; d.seg[0] = Builder::seg_plain(dkv_all.p, long(Bn) * 77, kv_total); d.M = Bn * 77; d.N = 768; d.Nw = 768; d.w = b.dpw(wk);
             d.out_f32 = dc.p; d.ldo32 = 768; b.gemm(d); }
-          if (dry()) b.emit(nullptr);
-          else { const float* src = dc.p; const long n = long(Bn) * 77 * 768;
+          { const float* src = dc.p; const long n = long(Bn) * 77 * 768;
             b.emit([=](cudaStream_t st) -> const char* {
               if (!io->b.d_cond_inputs) return nullptr;
               return scale_copy_f32(src, n, inv, io->b.d_cond_inputs, st); }); }
@@ -1416,7 +1387,7 @@ struct Model {
   void build_dec() {
     b.cur_stage = MADM_STAGE_DEC;
     const int Bn = b.B;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
+    IoBind* io = b.io;
     const int h16 = f16();
     {
       const Act& x = unet_tap[0];  // output of up layer 11 (64x64x320), the UNet's last hidden state
@@ -1427,8 +1398,7 @@ struct Model {
       d.w = b.pw(b.conv_w(kUnet + "conv_out", 4, 320, 9)); d.bias = P(kUnet + "conv_out.bias", 4); d.out_f32 = unet_sample.p; d.ldo32 = 4;
       b.gemm(d);
       b.free(n);
-      if (dry()) b.emit(nullptr, true);
-      else { const float* src = unet_sample.p;
+      { const float* src = unet_sample.p;
         b.emit([=](cudaStream_t st) -> const char* {
           return io->a.unet_sample ? nhwc_to_nchw(src, Bn, 64 * 64, 4, io->a.unet_sample, st) : nullptr; }, true); }
     }
@@ -1481,8 +1451,7 @@ struct Model {
     // the decoded image stays as fp32 [B*512*512][4] (3 used): the s0 projection consumes it directly (build_proj, 3-channel input)
     enc_tap = Act(); enc_tap.B = Bn; enc_tap.H = 512; enc_tap.W = 512; enc_tap.C = 3;
     enc_tap.f = img;
-    if (dry()) b.emit(nullptr, true);
-    else { const float* src = img.p;
+    { const float* src = img.p;
       b.emit([=](cudaStream_t st) -> const char* {
         if (!io->a.decoded && !io->a.decoded_raw) return nullptr;
         return decoder_image_pack(src, Bn, 512 * 512, nullptr, io->a.decoded, io->a.decoded_raw, h16, st); }, true); }
@@ -1510,7 +1479,7 @@ struct Model {
     proj_built[i] = true;
     const int saved_stage = b.cur_stage;
     b.cur_stage = MADM_STAGE_PROJ;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
+    IoBind* io = b.io;
     const std::string root = b.ema ? "ema_feature_projections." : "feature_projections.";
     const Act* taps[4] = {&enc_tap, &unet_tap[0], &unet_tap[1], &unet_tap[2]};
     b.defer_free = true;
@@ -1600,8 +1569,7 @@ struct Model {
       const float* g3 = P(p + "conv3.norm.weight", Cout); const float* b3 = P(p + "conv3.norm.bias", Cout);
       const float* gs = shortcut ? P(p + "shortcut.norm.weight", Cout) : nullptr;
       const float* bs = shortcut ? P(p + "shortcut.norm.bias", Cout) : nullptr;
-      if (dry()) b.emit(nullptr);
-      else if (rgb3) {
+      if (rgb3) {
         const float* csp = coefs.p;
         b.emit([=](cudaStream_t st) -> const char* {
           float* dst = io->a.out[i];
@@ -1625,8 +1593,7 @@ struct Model {
           const int Mi = int(M);
           // d(z) = d(out) * (out > 0), NCHW -> NHWC, scaled by the loss scale
           B16T dz = b.b16(size_t(M) * Cout);
-          if (dry()) b.emit(nullptr);
-          else { bf16* dst = dz.p;
+          { bf16* dst = dz.p;
             b.emit([=](cudaStream_t st) -> const char* {
               if (!io->b.dout[i] || !io->b.out[i]) return "madm_backward: dout / out pointer is null";
               return relu_bwd_nchw_to_nhwc16(io->b.dout[i], io->b.out[i], Bn, Cout, HW, S, dst, h16, st); }); }
@@ -1697,7 +1664,7 @@ struct Model {
   bool has_head() const { return b.ctx->params.count("sem_seg_head.conv_seg.weight") != 0; }
   void build_head() {
     b.cur_stage = MADM_STAGE_HEAD;
-    std::shared_ptr<IoBind> io = dry() ? nullptr : b.plan->io;
+    IoBind* io = b.io;
     const std::string h = "sem_seg_head.";
     const ParamRef* cs = b.find(h + "conv_seg.weight");
     const ParamRef* e0 = b.find(h + "embed_layers.0.proj.weight");
@@ -1719,8 +1686,7 @@ struct Model {
       const int Hi = H / ratio[i], Wi = W / ratio[i], HWi = Hi * Wi, Cin = i == 0 ? Cin0 : 512;
       const long Mi = long(Bn) * HWi;
       B16T x = b.b16(size_t(Mi) * Cin);
-      if (dry()) b.emit(nullptr);
-      else {
+      {
         bf16* xp = x.p;
         b.emit([=](cudaStream_t st) -> const char* {
           const float* src = io->a.out[i];
@@ -1785,8 +1751,7 @@ struct Model {
       b.gemm(d);
     }
     b.free(bott);
-    if (dry()) b.emit(nullptr);
-    else {
+    {
       const float* lp = lg.p;
       b.emit([=](cudaStream_t st) -> const char* {
         float* dst = io->a.logits;
@@ -1817,8 +1782,7 @@ struct Model {
       return;
     }
     b.bwd = true;
-    if (dry()) b.emit(nullptr);
-    else { float* dt = d_temb_all.p; bf16* dk = dkv_all.p; const size_t nt = size_t(b.B) * temb_total * 4, nk = size_t(b.B) * 77 * kv_total * 2;
+    { float* dt = d_temb_all.p; bf16* dk = dkv_all.p; const size_t nt = size_t(b.B) * temb_total * 4, nk = size_t(b.B) * 77 * kv_total * 2;
       b.emit([=](cudaStream_t st) -> const char* {
         if (cudaMemsetAsync(dt, 0, nt, st) != cudaSuccess || cudaMemsetAsync(dk, 0, nk, st) != cudaSuccess) return "cudaMemsetAsync failed";
         return nullptr; }); }
@@ -1882,11 +1846,11 @@ int build_plan(madm_ctx* ctx, const Builder& cfg, Plan* plan) {
   probe.mode = SIZE;
   int rc = traverse(ctx, probe);
   if (rc != MADM_OK) return rc;
-  plan->stats_off = 0;
   plan->stats_bytes = stats_region(probe);
   Builder bld = cfg;
   bld.mode = PLAN;
   bld.plan = plan;
+  bld.io = &plan->io;
   bld.packed = static_cast<const uint8_t*>(plan->packed);
   bld.dpacked = static_cast<const uint8_t*>(plan->dpacked);
   bld.stats_base = reinterpret_cast<float*>(plan->ws);
@@ -1895,6 +1859,40 @@ int build_plan(madm_ctx* ctx, const Builder& cfg, Plan* plan) {
   if (rc != MADM_OK) return rc;
   if (plan->stats_bytes + bld.peak > plan->ws_bytes)
     return set_err(ctx, MADM_ENOMEM, plan->train ? "madm_extract: training workspace too small for plan" : "madm_extract: workspace too small for plan");
+  return MADM_OK;
+}
+
+// Runs the launches of `ops` whose stage is in `stages` on `st`.  With `side`, branch launches run on the context's side streams: each
+// branch forks from `st` before its first launch and joins back before the first head launch (the head consumes the projections'
+// outputs) and at the end.  With `ev` (2 per launch), each launch is bracketed by its events.  A failing launch i is reported as
+// "<its message> (<what> i)".
+int replay(madm_ctx* ctx, const std::vector<Launch>& ops, int stages, cudaStream_t st, bool side, const cudaEvent_t* ev, const char* what) {
+  unsigned forked = 0;  // bit k: side stream k has work of this call
+  auto join = [&]() {
+    for (int k = 0; k < 4; ++k)
+      if (forked & (1u << k)) { cudaEventRecord(ctx->ev_join[k], ctx->side[k]); cudaStreamWaitEvent(st, ctx->ev_join[k], 0); }
+    forked = 0;
+  };
+  for (size_t i = 0; i < ops.size(); ++i) {
+    const Launch& l = ops[i];
+    if (!(l.stage & stages)) continue;
+    const int br = side ? l.branch : 0;
+    cudaStream_t s = st;
+    if (br > 0) {
+      if (!(forked & (1u << (br - 1)))) {  // fork here: everything this branch reads (its tap) has been enqueued on the caller's stream
+        cudaEventRecord(ctx->ev_fork[br - 1], st);
+        cudaStreamWaitEvent(ctx->side[br - 1], ctx->ev_fork[br - 1], 0);
+        forked |= 1u << (br - 1);
+      }
+      s = ctx->side[br - 1];
+    } else if (forked && (l.stage & MADM_STAGE_HEAD)) {
+      join();
+    }
+    if (ev) cudaEventRecord(ev[2 * i], s);
+    if (const char* e = l.run(s)) { join(); return set_err(ctx, MADM_ECUDA, std::string(e) + " (" + what + " " + std::to_string(i) + ")"); }
+    if (ev) cudaEventRecord(ev[2 * i + 1], s);
+  }
+  join();
   return MADM_OK;
 }
 
@@ -2243,12 +2241,12 @@ int madm_get_profile_stages(madm_ctx* ctx, int32_t stage_mask, madm_profile* out
   }
   if (cudaDeviceSynchronize() != cudaSuccess) return set_err(ctx, MADM_ECUDA, "cudaDeviceSynchronize failed");
   for (size_t i = 0; i < plan->ops.size(); ++i) {
-    if (!(plan->stage_of[i] & ctx->last_stages) || !(plan->stage_of[i] & stage_mask) || !plan->ops[i] || plan->optional[i]) continue;
+    const Launch& l = plan->ops[i];
+    if (!(l.stage & ctx->last_stages) || !(l.stage & stage_mask) || l.optional) continue;
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, plan->ev[2 * i], plan->ev[2 * i + 1]) != cudaSuccess) continue;
-    const int k = plan->kind[i];
-    out->kind[k].launches += 1; out->kind[k].ms += ms; out->kind[k].flops += plan->flops[i]; out->kind[k].bytes += plan->bytes[i];
-    out->kind[k].exec_flops += plan->exec_flops[i];
+    out->kind[l.kind].launches += 1; out->kind[l.kind].ms += ms; out->kind[l.kind].flops += l.flops; out->kind[l.kind].bytes += l.bytes;
+    out->kind[l.kind].exec_flops += l.exec_flops;
   }
   return MADM_OK;
 }
@@ -2260,8 +2258,8 @@ int madm_launch_count(madm_ctx* ctx, int32_t B, int32_t stages) {
     if (std::get<0>(p->first) == B) { it = p; break; }
   if (it == ctx->plans.end()) return -1;
   int n = 0;
-  for (size_t i = 0; i < it->second->ops.size(); ++i)
-    if ((it->second->stage_of[i] & stages) && it->second->ops[i] && !it->second->optional[i]) ++n;
+  for (const Launch& l : it->second->ops)
+    if ((l.stage & stages) && !l.optional) ++n;
   return n;
 }
 
@@ -2294,7 +2292,7 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
   if (it != ctx->plans.end() && it->second->packed == a->packed && it->second->ws == a->workspace) plan = it->second.get();
   if (!plan) {
     std::unique_ptr<Plan> np(new Plan());
-    np->B = a->B; np->ema = a->ema != 0; np->packed = a->packed; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
+    np->packed = a->packed; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
     Builder cfg{ctx, PLAN, a->B, a->ema != 0};
     cfg.head_h = a->head_h; cfg.head_w = a->head_w;
     rc = build_plan(ctx, cfg, np.get());
@@ -2302,7 +2300,7 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
     plan = np.get();
     ctx->plans[key] = std::move(np);
   }
-  plan->io->a = *a;
+  plan->io.a = *a;
   const bool prof = ctx->profiling;
   if (prof && plan->ev.size() != 2 * plan->ops.size()) {
     plan->ev.resize(2 * plan->ops.size());
@@ -2314,7 +2312,7 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
   bool use_side = !prof;
   if (use_side) {
     bool any = false;
-    for (size_t i = 0; i < plan->ops.size() && !any; ++i) any = plan->branch[i] != 0 && (plan->stage_of[i] & a->stages) && plan->ops[i];
+    for (size_t i = 0; i < plan->ops.size() && !any; ++i) any = plan->ops[i].branch != 0 && (plan->ops[i].stage & a->stages);
     use_side = any;
   }
   if (use_side && !ctx->ev_fork[0]) {
@@ -2325,31 +2323,8 @@ int madm_extract(madm_ctx* ctx, const madm_extract_args* a, madm_stream stream) 
            cudaEventCreateWithFlags(&ctx->ev_join[k], cudaEventDisableTiming) == cudaSuccess;
     if (!ok) return set_err(ctx, MADM_ECUDA, "madm_extract: could not create the projection streams");
   }
-  unsigned forked = 0;  // bit k: side stream k has work of this call
-  auto join = [&]() {
-    for (int k = 0; k < 4; ++k)
-      if (forked & (1u << k)) { cudaEventRecord(ctx->ev_join[k], ctx->side[k]); cudaStreamWaitEvent(st, ctx->ev_join[k], 0); }
-    forked = 0;
-  };
-  for (size_t i = 0; i < plan->ops.size(); ++i) {
-    if (!(plan->stage_of[i] & a->stages) || !plan->ops[i]) continue;
-    const int br = use_side ? plan->branch[i] : 0;
-    cudaStream_t s = st;
-    if (br > 0) {
-      if (!(forked & (1u << (br - 1)))) {  // fork here: everything this branch reads (its tap) has been enqueued on the caller's stream
-        cudaEventRecord(ctx->ev_fork[br - 1], st);
-        cudaStreamWaitEvent(ctx->side[br - 1], ctx->ev_fork[br - 1], 0);
-        forked |= 1u << (br - 1);
-      }
-      s = ctx->side[br - 1];
-    } else if (forked && (plan->stage_of[i] & MADM_STAGE_HEAD)) {
-      join();  // the head consumes the projections' outputs
-    }
-    if (prof) cudaEventRecord(plan->ev[2 * i], s);
-    if (const char* e = plan->ops[i](s)) { join(); return set_err(ctx, MADM_ECUDA, std::string(e) + " (op " + std::to_string(i) + ")"); }
-    if (prof) cudaEventRecord(plan->ev[2 * i + 1], s);
-  }
-  join();
+  rc = replay(ctx, plan->ops, a->stages, st, use_side, prof ? plan->ev.data() : nullptr, "op");
+  if (rc != MADM_OK) return rc;
   ctx->last_plan = plan;
   ctx->last_stages = a->stages;
   return MADM_OK;
@@ -2385,7 +2360,7 @@ int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
     if (need == 0) return MADM_EINVAL;
     if (a->workspace_bytes < need) return set_err(ctx, MADM_ENOMEM, "madm_extract: training workspace too small (madm_train_workspace_bytes)");
     std::unique_ptr<Plan> np(new Plan());
-    np->B = a->B; np->packed = a->packed; np->dpacked = a->packed_dgrad; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
+    np->packed = a->packed; np->dpacked = a->packed_dgrad; np->ws = a->workspace; np->ws_bytes = a->workspace_bytes;
     np->train = true; np->adapter = ad; np->loss_scale = a->train_loss_scale; np->lora_scale = a->train_lora_scale;
     Builder cfg{ctx, PLAN, a->B, false};
     cfg.train = true; cfg.adapter = ad; cfg.lora_scale = a->train_lora_scale; cfg.loss_scale = a->train_loss_scale;
@@ -2394,13 +2369,9 @@ int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
     plan = np.get();
     ctx->train_plans[tkey] = std::move(np);
   }
-  plan->io->a = *a;
+  plan->io.a = *a;
   PdlTrainScope pdl;  // programmatic dependent launch for the training forward's ~550 small launches (launch.cuh)
-  for (size_t i = 0; i < plan->ops.size(); ++i) {
-    if (!plan->ops[i]) continue;
-    if (const char* e = plan->ops[i](st)) return set_err(ctx, MADM_ECUDA, std::string(e) + " (training forward op " + std::to_string(i) + ")");
-  }
-  return MADM_OK;
+  return replay(ctx, plan->ops, ~0, st, false, nullptr, "training forward op");
 }
 }  // namespace
 
@@ -2447,11 +2418,7 @@ size_t madm_train_workspace_bytes(madm_ctx* ctx, int32_t B, const char* adapter)
 int madm_backward_launch_count(madm_ctx* ctx, int32_t B) {
   if (!ctx) return -1;
   for (auto& kv : ctx->train_plans)
-    if (kv.first.first == B) {
-      int n = 0;
-      for (const Op& op : kv.second->bops) if (op) ++n;
-      return n;
-    }
+    if (kv.first.first == B) return int(kv.second->bops.size());
   return -1;
 }
 
@@ -2465,14 +2432,9 @@ int madm_backward(madm_ctx* ctx, const madm_backward_args* a, madm_stream stream
   if (plan->ws != a->workspace || plan->packed != a->packed || plan->dpacked != a->packed_dgrad || plan->adapter != ad ||
       plan->loss_scale != a->loss_scale || plan->lora_scale != a->lora_alpha_over_r)
     return set_err(ctx, MADM_ESTATE, "madm_backward: arguments differ from the MADM_FLAG_TRAIN forward this plan was built for");
-  plan->io->b = *a;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  plan->io.b = *a;
   PdlTrainScope pdl;  // programmatic dependent launch for the backward's ~640 small launches (launch.cuh)
-  for (size_t i = 0; i < plan->bops.size(); ++i) {
-    if (!plan->bops[i]) continue;
-    if (const char* e = plan->bops[i](st)) return set_err(ctx, MADM_ECUDA, std::string(e) + " (backward op " + std::to_string(i) + ")");
-  }
-  return MADM_OK;
+  return replay(ctx, plan->bops, ~0, static_cast<cudaStream_t>(stream), false, nullptr, "backward op");
 }
 
 }  // extern "C"
