@@ -45,7 +45,8 @@ int madm_op_gemm(const madm_gemm_args* a, madm_stream stream) {
   d.residual = a->residual; d.ldr = a->ldr;
   d.out_f32 = a->out_f32; d.ldo32 = a->ldo32; d.out_bf16 = a->out_bf16; d.ldo16 = a->ldo16;
   d.act = a->act; d.alpha = a->alpha; d.bn = a->bn; d.fp16 = a->dtype == MADM_DTYPE_FP16;
-  d.colstats = a->colstats; d.stat_rows = a->stat_rows ? a->stat_rows : 32; d.mt = a->mt; d.s2d_H = a->s2d_H; d.s2d_W = a->s2d_W; d.pair = a->pair; d.res16 = a->res16;
+  if (a->colstats && a->stat_rows != 0 && a->stat_rows != 32) return fail("gemm: stat_rows must be 32");
+  d.colstats = a->colstats; d.mt = a->mt; d.s2d_H = a->s2d_H; d.s2d_W = a->s2d_W; d.pair = a->pair; d.res16 = a->res16;
   GemmLaunch L;
   if (const char* e = gemm_prepare(d, &L)) return fail(e);
   RUN(gemm_launch(L, static_cast<cudaStream_t>(stream)));
@@ -262,9 +263,12 @@ int madm_op_attention_bwd(const void* q, int32_t ldq, const void* k, int32_t ldk
                           const void* dout, int32_t lddo, void* dq, int32_t lddq, void* dk, int32_t lddk, void* dv, int32_t lddv, int32_t B,
                           int32_t heads, int32_t d, int32_t Nq, int32_t Nk, int64_t q_bs, int64_t kv_bs, int64_t o_bs, int64_t do_bs, int64_t dq_bs,
                           int64_t dkv_bs, float scale, float* scratch, int32_t dtype, madm_stream stream) {
-  RUN(attention_bwd(q, ldq, k, ldk, v, ldv, o, ldo, dout, lddo, dq, lddq, dk, lddk, dv, lddv, B, heads, d, Nq, Nk, long(q_bs), long(kv_bs), long(kv_bs),
-                    long(o_bs), long(do_bs), long(dq_bs), long(dkv_bs), long(dkv_bs), scale, scratch, dtype == MADM_DTYPE_FP16,
-                    static_cast<cudaStream_t>(stream)));
+  AttnBwdLaunch L;
+  if (const char* e = attention_bwd_prepare(q, ldq, k, ldk, v, ldv, o, ldo, dout, lddo, dq, lddq, dk, lddk, dv, lddv, B, heads, d, Nq, Nk, long(q_bs),
+                                            long(kv_bs), long(kv_bs), long(o_bs), long(do_bs), long(dq_bs), long(dkv_bs), long(dkv_bs), scale, scratch,
+                                            dtype == MADM_DTYPE_FP16, &L))
+    return fail(e);
+  RUN(attention_bwd_launch(L, static_cast<cudaStream_t>(stream)));
 }
 int64_t madm_op_wgrad_scratch_floats(int32_t M, int32_t N, int32_t K, int32_t taps) { return int64_t(wgrad_scratch_floats(M, N, K, taps)); }
 int madm_op_wgrad(const void* dy16, int32_t lda, const void* x16, int32_t ldb, int32_t M, int32_t N, int32_t K, int32_t taps, int32_t Bimg, int32_t H,

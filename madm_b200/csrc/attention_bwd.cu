@@ -448,7 +448,7 @@ __global__ void attn_bwd_kv_reduce_kernel(const AttnBwdParams p, int B) {
 }
 
 template <typename T, int DP>
-const char* launch_all(const AttnBwdParams& p, int B, cudaStream_t st, bool have_lse, int fp16) {
+const char* launch_all(const AttnBwdLaunch& L, cudaStream_t st) {
   static bool attr = false;
   if (!attr) {
     if (cudaFuncSetAttribute(attn_bwd_dkv_kernel<T, DP>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(AttnSmem<DP>::DKV)) != cudaSuccess ||
@@ -457,20 +457,19 @@ const char* launch_all(const AttnBwdParams& p, int B, cudaStream_t st, bool have
       return "attention_bwd: cudaFuncSetAttribute failed";
     attr = true;
   }
-  const dim3 gq((p.Nq + AB - 1) / AB, p.heads, B), gk(((p.Nk + AB - 1) / AB) * p.qsplit, p.heads, B);
-  if (have_lse) launch_k(attn_bwd_d_kernel, dim3(gq), dim3(AB_THREADS), 0, st, p, fp16);
-  else launch_k(attn_bwd_prep_kernel<T, DP>, dim3(gq), dim3(AB_THREADS), AttnSmem<DP>::PREP, st, p);
+  const AttnBwdParams& p = *reinterpret_cast<const AttnBwdParams*>(L.params);
+  if (L.have_lse) launch_k(attn_bwd_d_kernel, L.gq, dim3(AB_THREADS), 0, st, p, L.fp16);
+  else launch_k(attn_bwd_prep_kernel<T, DP>, L.gq, dim3(AB_THREADS), AttnSmem<DP>::PREP, st, p);
   if (p.L2out) {  // large self-attention: the tcgen05 / TMEM kernels (attention_bwd_tc.cu) take over after the L / D pass
     if (cudaGetLastError() != cudaSuccess) return "attention_bwd launch failed";
-    return attention_bwd_tc(p.q, p.ldq, p.k, p.ldk, p.v, p.ldv, p.dout, p.lddo, p.dq, p.lddq, p.dk, p.lddk, p.dv, p.lddv, B, p.heads, p.d, p.Nq, p.Nk, p.q_bs,
-                            p.k_bs, p.v_bs, p.do_bs, p.dq_bs, p.dk_bs, p.dv_bs, p.scale, p.L2out, p.D, fp16, st);
+    return attention_bwd_tc_launch(L, st);
   }
-  launch_k(attn_bwd_dkv_kernel<T, DP>, dim3(gk), dim3(AB_THREADS), AttnSmem<DP>::DKV, st, p);
+  launch_k(attn_bwd_dkv_kernel<T, DP>, L.gk, dim3(AB_THREADS), AttnSmem<DP>::DKV, st, p);
   if (p.qsplit > 1) {
-    const long total = long(B) * p.heads * p.Nk * (p.d / 2);
-    launch_k(attn_bwd_kv_reduce_kernel<T, DP>, dim3(unsigned((total + 255) / 256)), dim3(256), 0, st, p, B);
+    const long total = long(L.B) * p.heads * p.Nk * (p.d / 2);
+    launch_k(attn_bwd_kv_reduce_kernel<T, DP>, dim3(unsigned((total + 255) / 256)), dim3(256), 0, st, p, L.B);
   }
-  launch_k(attn_bwd_dq_kernel<T, DP>, dim3(gq), dim3(AB_THREADS), AttnSmem<DP>::DQ, st, p);
+  launch_k(attn_bwd_dq_kernel<T, DP>, L.gq, dim3(AB_THREADS), AttnSmem<DP>::DQ, st, p);
   return cudaGetLastError() == cudaSuccess ? nullptr : "attention_bwd launch failed";
 }
 
@@ -494,16 +493,17 @@ size_t attention_bwd_scratch_floats(int B, int heads, int d, int Nq, int Nk) {
   return n;
 }
 
-const char* attention_bwd(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* o, int ldo, const void* dout, int lddo,
-                          void* dq, int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs,
-                          long v_bs, long o_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, float* scratch, int fp16, cudaStream_t st,
-                          const float* lse) {
+const char* attention_bwd_prepare(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* o, int ldo, const void* dout,
+                                  int lddo, void* dq, int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs,
+                                  long k_bs, long v_bs, long o_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, float* scratch, int fp16,
+                                  AttnBwdLaunch* L, const float* lse) {
   if (d != 40 && d != 80 && d != 160) return "attention_bwd: head dim must be 40, 80 or 160";
   const int lds[8] = {ldq, ldk, ldv, ldo, lddo, lddq, lddk, lddv};
   for (int i = 0; i < 8; ++i) if (lds[i] % 8 != 0) return "attention_bwd: row pitches must be multiples of 8 elements";
   const void* ptrs[8] = {q, k, v, o, dout, dq, dk, dv};
   for (int i = 0; i < 8; ++i) if (reinterpret_cast<uintptr_t>(ptrs[i]) & 15) return "attention_bwd: pointers must be 16-byte aligned";
-  AttnBwdParams p;
+  static_assert(sizeof(AttnBwdParams) <= sizeof(L->params), "AttnBwdLaunch::params too small");
+  AttnBwdParams& p = *reinterpret_cast<AttnBwdParams*>(L->params);
   p.q = static_cast<const uint16_t*>(q); p.k = static_cast<const uint16_t*>(k); p.v = static_cast<const uint16_t*>(v);
   p.o = static_cast<const uint16_t*>(o); p.dout = static_cast<const uint16_t*>(dout);
   p.dq = static_cast<uint16_t*>(dq); p.dk = static_cast<uint16_t*>(dk); p.dv = static_cast<uint16_t*>(dv);
@@ -520,15 +520,27 @@ const char* attention_bwd(const void* q, int ldq, const void* k, int ldk, const 
     const size_t one = size_t(p.qsplit) * B * heads * (((Nk + AB - 1) / AB) * AB) * attn_dp(d);
     p.part_k = base; p.part_v = base + one;
   }
-  const bool hl = lse != nullptr;
-  if (fp16) {
-    if (d == 40) return launch_all<__half, 48>(p, B, st, hl, fp16);
-    if (d == 80) return launch_all<__half, 80>(p, B, st, hl, fp16);
-    return launch_all<__half, 160>(p, B, st, hl, fp16);
+  L->gq = dim3((Nq + AB - 1) / AB, heads, B);
+  L->gk = dim3(((Nk + AB - 1) / AB) * p.qsplit, heads, B);
+  L->B = B;
+  L->fp16 = fp16;
+  L->dp = attn_dp(d);
+  L->have_lse = lse != nullptr;
+  if (p.L2out)
+    return attention_bwd_tc_prepare(q, ldq, k, ldk, v, ldv, dout, lddo, dq, lddq, dk, lddk, dv, lddv, B, heads, d, Nq, Nk, q_bs, k_bs, v_bs, do_bs, dq_bs,
+                                    dk_bs, dv_bs, scale, p.L2out, p.D, L);
+  return nullptr;
+}
+
+const char* attention_bwd_launch(const AttnBwdLaunch& L, cudaStream_t st) {
+  if (L.fp16) {
+    if (L.dp == 48) return launch_all<__half, 48>(L, st);
+    if (L.dp == 80) return launch_all<__half, 80>(L, st);
+    return launch_all<__half, 160>(L, st);
   }
-  if (d == 40) return launch_all<__nv_bfloat16, 48>(p, B, st, hl, fp16);
-  if (d == 80) return launch_all<__nv_bfloat16, 80>(p, B, st, hl, fp16);
-  return launch_all<__nv_bfloat16, 160>(p, B, st, hl, fp16);
+  if (L.dp == 48) return launch_all<__nv_bfloat16, 48>(L, st);
+  if (L.dp == 80) return launch_all<__nv_bfloat16, 80>(L, st);
+  return launch_all<__nv_bfloat16, 160>(L, st);
 }
 
 }  // namespace madm

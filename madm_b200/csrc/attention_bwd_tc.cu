@@ -24,7 +24,6 @@
 #include "launch.cuh"
 #include "ptx.cuh"
 
-#include <mutex>
 #include <stdio.h>
 
 namespace madm {
@@ -306,34 +305,6 @@ __global__ void __launch_bounds__(BT_THREADS, 1) attn_bwd_tc_kernel(const __grid
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn bt_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* q = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &q, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(q);
-  });
-  return fn;
-}
-// [d, heads, tokens, batch] view of a [batch, tokens, ld] buffer whose head h occupies columns [h*d, (h+1)*d); box = 64 columns (zero-filled
-// past d) x 128 tokens
-const char* bt_map(CUtensorMap* tm, const void* ptr, int d, int heads, int ntok, int B, int ld, long bstride, int box_rows) {
-  EncodeTiledFn fn = bt_encode_fn();
-  if (!fn) return "attention_bwd: cuTensorMapEncodeTiled unavailable";
-  cuuint64_t dims[4] = {cuuint64_t(d), cuuint64_t(heads), cuuint64_t(ntok), cuuint64_t(B)};
-  cuuint64_t strides[3] = {cuuint64_t(d) * 2, cuuint64_t(ld) * 2, cuuint64_t(bstride) * 2};
-  if (B == 1) strides[2] = cuuint64_t(ntok) * ld * 2;
-  cuuint32_t box[4] = {64, 1, cuuint32_t(box_rows), 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  const CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_UINT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS ? nullptr : "attention_bwd: cuTensorMapEncodeTiled failed";
-}
-
 template <int MODE, bool FP16, int KC, int TN>
 const char* bt_launch(const BwdTcParams& p, dim3 grid, cudaStream_t st) {
   static bool attr = false;
@@ -359,43 +330,46 @@ bool attention_bwd_tc_supported(int d, int Nq, int Nk) {
 }
 
 // dK / dV and dQ of one attention layer on the tcgen05 kernels.  L2 = log2-domain log-sum-exp, D = rowsum(dO * O), both [B, heads, Nq].
-const char* attention_bwd_tc(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* dout, int lddo, void* dq, int lddq,
-                             void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs, long v_bs, long do_bs,
-                             long dq_bs, long dk_bs, long dv_bs, float scale, const float* L2, const float* D, int fp16, cudaStream_t st) {
+const char* attention_bwd_tc_prepare(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* dout, int lddo, void* dq,
+                                     int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs,
+                                     long v_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, const float* L2, const float* D,
+                                     AttnBwdLaunch* L) {
   if (!attention_bwd_tc_supported(d, Nq, Nk)) return "attention_bwd_tc: unsupported shape";
-  BwdTcParams p;
-  p.L2 = L2; p.D = D; p.Nq = Nq; p.d = d;
-  p.ksteps = (d + 15) / 16;
-  p.dv = (d + 15) / 16 * 16;
-  p.scale_log2 = scale * 1.4426950408889634f;
-  p.out_scale_s = scale / kDsScale;
-  p.out_scale_p = 1.0f / kPScale;
+  static_assert(sizeof(BwdTcParams) <= sizeof(L->tc[0]), "AttnBwdLaunch::tc too small");
+  BwdTcParams& pkv = *reinterpret_cast<BwdTcParams*>(L->tc[0]);  // dK, dV: K / V resident, Q / dO streamed
+  BwdTcParams& pq = *reinterpret_cast<BwdTcParams*>(L->tc[1]);   // dQ: Q / dO resident, K / V streamed
+  pkv.L2 = L2; pkv.D = D; pkv.Nq = Nq; pkv.d = d;
+  pkv.ksteps = (d + 15) / 16;
+  pkv.dv = (d + 15) / 16 * 16;
+  pkv.scale_log2 = scale * 1.4426950408889634f;
+  pkv.out_scale_s = scale / kDsScale;
+  pkv.out_scale_p = 1.0f / kPScale;
+  pq = pkv;
   const int TN = d <= 64 ? 128 : 64;  // rows of a streamed tile (BtCfg)
-  CUtensorMap tq, tk, tv, tdo, tqs, tks, tvs, tdos;  // resident-role maps (128-row boxes) and streamed-role maps (TN-row boxes)
-  if (const char* e = bt_map(&tq, q, d, heads, Nq, B, ldq, q_bs, 128)) return e;
-  if (const char* e = bt_map(&tk, k, d, heads, Nk, B, ldk, k_bs, 128)) return e;
-  if (const char* e = bt_map(&tv, v, d, heads, Nk, B, ldv, v_bs, 128)) return e;
-  if (const char* e = bt_map(&tdo, dout, d, heads, Nq, B, lddo, do_bs, 128)) return e;
-  if (const char* e = bt_map(&tqs, q, d, heads, Nq, B, ldq, q_bs, TN)) return e;
-  if (const char* e = bt_map(&tks, k, d, heads, Nk, B, ldk, k_bs, TN)) return e;
-  if (const char* e = bt_map(&tvs, v, d, heads, Nk, B, ldv, v_bs, TN)) return e;
-  if (const char* e = bt_map(&tdos, dout, d, heads, Nq, B, lddo, do_bs, TN)) return e;
-  {  // dK, dV
-    p.tmR1 = tk; p.tmR2 = tv; p.tmT1 = tqs; p.tmT2 = tdos;
-    p.out_s = static_cast<uint16_t*>(dk); p.ld_s = lddk; p.bs_s = dk_bs;
-    p.out_p = static_cast<uint16_t*>(dv); p.ld_p = lddv; p.bs_p = dv_bs;
-    p.n_stream = Nq / TN;
-    const dim3 grid(Nk / 128, heads, B);
-    if (const char* e = bt_dispatch<0>(p, grid, fp16, st)) return e;
-  }
-  {  // dQ
-    p.tmR1 = tq; p.tmR2 = tdo; p.tmT1 = tks; p.tmT2 = tvs;
-    p.out_s = static_cast<uint16_t*>(dq); p.ld_s = lddq; p.bs_s = dq_bs;
-    p.out_p = nullptr; p.ld_p = 0; p.bs_p = 0;
-    p.n_stream = Nk / TN;
-    const dim3 grid(Nq / 128, heads, B);
-    if (const char* e = bt_dispatch<1>(p, grid, fp16, st)) return e;
-  }
+  pkv.out_s = static_cast<uint16_t*>(dk); pkv.ld_s = lddk; pkv.bs_s = dk_bs;
+  pkv.out_p = static_cast<uint16_t*>(dv); pkv.ld_p = lddv; pkv.bs_p = dv_bs;
+  pkv.n_stream = Nq / TN;
+  pq.out_s = static_cast<uint16_t*>(dq); pq.ld_s = lddq; pq.bs_s = dq_bs;
+  pq.out_p = nullptr; pq.ld_p = 0; pq.bs_p = 0;
+  pq.n_stream = Nk / TN;
+  // resident-role maps in 128-row boxes, streamed-role maps in TN-row boxes
+  const char* op = "attention_bwd";
+  if (const char* e = attention_head_map(&pkv.tmR1, op, k, d, heads, Nk, B, ldk, k_bs, 128)) return e;
+  if (const char* e = attention_head_map(&pkv.tmR2, op, v, d, heads, Nk, B, ldv, v_bs, 128)) return e;
+  if (const char* e = attention_head_map(&pkv.tmT1, op, q, d, heads, Nq, B, ldq, q_bs, TN)) return e;
+  if (const char* e = attention_head_map(&pkv.tmT2, op, dout, d, heads, Nq, B, lddo, do_bs, TN)) return e;
+  if (const char* e = attention_head_map(&pq.tmR1, op, q, d, heads, Nq, B, ldq, q_bs, 128)) return e;
+  if (const char* e = attention_head_map(&pq.tmR2, op, dout, d, heads, Nq, B, lddo, do_bs, 128)) return e;
+  if (const char* e = attention_head_map(&pq.tmT1, op, k, d, heads, Nk, B, ldk, k_bs, TN)) return e;
+  if (const char* e = attention_head_map(&pq.tmT2, op, v, d, heads, Nk, B, ldv, v_bs, TN)) return e;
+  L->gtc[0] = dim3(Nk / 128, heads, B);
+  L->gtc[1] = dim3(Nq / 128, heads, B);
+  return nullptr;
+}
+
+const char* attention_bwd_tc_launch(const AttnBwdLaunch& L, cudaStream_t st) {
+  if (const char* e = bt_dispatch<0>(*reinterpret_cast<const BwdTcParams*>(L.tc[0]), L.gtc[0], L.fp16, st)) return e;
+  if (const char* e = bt_dispatch<1>(*reinterpret_cast<const BwdTcParams*>(L.tc[1]), L.gtc[1], L.fp16, st)) return e;
   return cudaGetLastError() == cudaSuccess ? nullptr : "attention_bwd_tc launch failed";
 }
 

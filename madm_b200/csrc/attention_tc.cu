@@ -16,7 +16,6 @@
 #include "launch.cuh"
 #include "ptx.cuh"
 
-#include <mutex>
 #include <stdio.h>
 
 namespace madm {
@@ -502,38 +501,12 @@ __global__ void __launch_bounds__(FaCfg<D, NQT>::THREADS, 1) fa_tc_kernel(const 
 }
 
 // ------------------------------------------------------------------------------------------------ host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn fa_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static std::once_flag once;
-  std::call_once(once, [] {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  });
-  return fn;
-}
-
-// [d, heads, tokens, batch] view of a [batch, tokens, ld] buffer whose head h occupies columns [h*d, (h+1)*d)
-static const char* fa_map(CUtensorMap* tm, const void* ptr, int d, int heads, int ntok, int B, int ld, long bstride) {
-  EncodeTiledFn fn = fa_encode_fn();
-  if (!fn) return "cuTensorMapEncodeTiled unavailable";
+const char* attention_head_map(CUtensorMap* tm, const char* op, const void* ptr, int d, int heads, int ntok, int B, int ld, long bstride, int box_rows) {
   cuuint64_t dims[4] = {cuuint64_t(d), cuuint64_t(heads), cuuint64_t(ntok), cuuint64_t(B)};
   cuuint64_t strides[3] = {cuuint64_t(d) * 2, cuuint64_t(ld) * 2, cuuint64_t(bstride) * 2};
   if (B == 1) strides[2] = cuuint64_t(ntok) * ld * 2;
-  cuuint32_t box[4] = {64, 1, 128, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_UINT16, 4, const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    static thread_local char buf[128];
-    snprintf(buf, sizeof(buf), "attention: cuTensorMapEncodeTiled failed (CUresult %d)", int(r));
-    return buf;
-  }
-  return nullptr;
+  cuuint32_t box[4] = {64, 1, cuuint32_t(box_rows), 1};
+  return encode_tensor_map(tm, op, ptr, 4, dims, strides, box);
 }
 
 const char* flash_attention_tc_prepare(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, void* o, int ldo, int B,
@@ -546,9 +519,9 @@ const char* flash_attention_tc_prepare(const void* q, int ldq, const void* k, in
   if (Nq < 1 || Nk < 1) return "attention: empty problem";
   static_assert(sizeof(FaParams) <= sizeof(L->params), "FaLaunch::params too small");
   FaParams* p = reinterpret_cast<FaParams*>(L->params);
-  if (const char* e = fa_map(&p->tmQ, q, d, heads, Nq, B, ldq, q_bs)) return e;
-  if (const char* e = fa_map(&p->tmK, k, d, heads, Nk, B, ldk, kv_bs)) return e;
-  if (const char* e = fa_map(&p->tmV, v, d, heads, Nk, B, ldv, kv_bs)) return e;
+  if (const char* e = attention_head_map(&p->tmQ, "attention", q, d, heads, Nq, B, ldq, q_bs, 128)) return e;
+  if (const char* e = attention_head_map(&p->tmK, "attention", k, d, heads, Nk, B, ldk, kv_bs, 128)) return e;
+  if (const char* e = attention_head_map(&p->tmV, "attention", v, d, heads, Nk, B, ldv, kv_bs, 128)) return e;
   p->O = reinterpret_cast<uint16_t*>(o);
   p->ldo = ldo; p->o_bs = o_bs; p->Nq = Nq; p->Nk = Nk;
   p->scale_log2 = scale * 1.4426950408889634f;

@@ -97,12 +97,13 @@ struct GradBuf {
   bool stop = false;     // nothing trainable lies upstream: contributions are skipped
 };
 
+constexpr int kStatRows = 32;  // rows per block of a GEMM epilogue's column statistics (GemmDesc::colstats: one block per epilogue warp)
+
 // fp32 residual-stream activation, NHWC, optionally with a bf16 copy for consumers that take it as a GEMM operand
 struct Act {
   F32T f; B16T h;
   std::shared_ptr<struct GradBuf> gr;  // training plans: gradient of this activation (fp32 [M,C]), shared by all copies of the handle
-  float* cs = nullptr;  // per-column statistics written by the producing GEMM's epilogue ([M/sr][C][2]), if any
-  int sr = 0;           // rows per statistics block (64 or 128)
+  float* cs = nullptr;  // per-column statistics written by the producing GEMM's epilogue ([M/kStatRows][C][2]), if any
   bool has_cs = false;  // valid in every builder mode (cs itself is null outside PLAN mode)
   bool h_s2d = false;   // the 16-bit copy `h` is stored in space-to-depth layout [4][B][H/2][W/2][C] (input of a stride-2 conv)
   int B = 0, H = 0, W = 0, C = 0;
@@ -305,17 +306,15 @@ struct Builder {
 
   // per-column statistics buffer for a GEMM whose output feeds a GroupNorm; lives in the statistics arena
   void attach_colstats(Act& a, GemmDesc& d) {
-    a.sr = 32;
-    if (a.HW() % a.sr != 0 || a.C % 32 != 0) return;  // shape not eligible: the consumer falls back to a statistics pass
+    if (a.HW() % kStatRows != 0 || a.C % 32 != 0) return;  // shape not eligible: the consumer falls back to a statistics pass
     // The fused statistics add ~25 % to the epilogue's instruction count (separate kernel variant, gemm_tc_kernel<BN,true>):
     // measured +0.25 ms on the GEMM family against -1.0 ms of statistics passes, at every K.
     if (choose_splits(d) > 1) return;  // split-K launches leave the statistics to a separate pass
-    const size_t n = size_t((a.M() + a.sr - 1) / a.sr) * a.C * 2;
+    const size_t n = size_t((a.M() + kStatRows - 1) / kStatRows) * a.C * 2;
     a.cs = stats_base ? stats_base + stats_used : nullptr;
     stats_used += n;
     a.has_cs = true;
     d.colstats = a.cs;
-    d.stat_rows = a.sr;
   }
 
   // ---- parameters
@@ -502,10 +501,10 @@ struct Builder {
       if (algo_flops < 0) algo_flops = exec;
       if (getenv("MADM_DUMP_PLAN")) {  // tools/layer_report.py parses these lines
         char tail[48];
-        if (splits > 1) snprintf(tail, sizeof(tail), "splits=%d tma=%d stats=0", splits, L.tma_epi);
-        else snprintf(tail, sizeof(tail), "tma=%d stats=%d", L.tma_epi, (d.colstats ? 1 : 0) | (d.s2d_W > 0 ? 2 : 0));
+        if (splits > 1) snprintf(tail, sizeof(tail), "splits=%d tma=%d stats=0", splits, L.p.tma_epi);
+        else snprintf(tail, sizeof(tail), "tma=%d stats=%d", L.p.tma_epi, (d.colstats ? 1 : 0) | (d.s2d_W > 0 ? 2 : 0));
         fprintf(stderr, "MADM_PLAN gemm M=%d N=%d K=%d bn=%d tiles=%d taps=%d nseg=%d act=%d res=%d f32=%d h16=%d gflop=%.3f %s\n", d.M, d.N, int(K), L.bn,
-                L.num_tiles, d.seg[0].ntaps, d.nseg, d0.act, d0.residual ? 1 : 0, d0.out_f32 ? 1 : 0, d0.out_bf16 ? 1 : 0, algo_flops / 1e9, tail);
+                L.p.num_tiles, d.seg[0].ntaps, d.nseg, d0.act, d0.residual ? 1 : 0, d0.out_f32 ? 1 : 0, d0.out_bf16 ? 1 : 0, algo_flops / 1e9, tail);
       }
       emit([L](cudaStream_t st) { return gemm_launch(L, st); }, false, MADM_KIND_GEMM, algo_flops, gemm_algo_bytes(d), exec);
       if (splits > 1) {
@@ -530,6 +529,17 @@ struct Builder {
     if (const char* e = flash_attention_tc_prepare(q, ldq, k, ldk, v, ldv, o, ldo, Bn, heads, d, Nq, Nk, q_bs, kv_bs, o_bs, scale, h16, &L, lse))
       fail(MADM_EINVAL, std::string(e));
     emit([L](cudaStream_t st) { return flash_attention_tc_launch(L, st); }, false, MADM_KIND_ATTENTION, flops, 0.0);
+  }
+  // its backward (training plans): prepared like the forward, with the gradient kernels' scratch
+  void attention_bwd(const bf16* q, int ldq, const bf16* k, int ldk, const bf16* v, int ldv, const bf16* o, int ldo, const bf16* dout, int lddo, bf16* dq,
+                     int lddq, bf16* dk, int lddk, bf16* dv, int lddv, int Bn, int heads, int d, int Nq, int Nk, long q_bs, long k_bs, long v_bs, long o_bs,
+                     long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, float* scratch, const float* lse) {
+    if (mode != PLAN) return;
+    AttnBwdLaunch L;
+    if (const char* e = attention_bwd_prepare(q, ldq, k, ldk, v, ldv, o, ldo, dout, lddo, dq, lddq, dk, lddk, dv, lddv, Bn, heads, d, Nq, Nk, q_bs, k_bs,
+                                              v_bs, o_bs, do_bs, dq_bs, dk_bs, dv_bs, scale, scratch, ctx->fp16, &L, lse))
+      fail(MADM_EINVAL, std::string(e));
+    emit([L](cudaStream_t st) { return attention_bwd_launch(L, st); });
   }
 
   static GemmASeg seg_1x1(const bf16* p, int Bn, int H, int W, int C, int ld = 0) {
@@ -572,11 +582,11 @@ struct Builder {
     const double elems = double(Bn) * HW * (C0 + C1);
     const int f16 = ctx->fp16, i16 = in16 ? 1 : 0;
     const double in_b = in16 ? 2 : 4;
-    const bool fused = x0.has_cs && (!x1 || (x1->has_cs && x1->sr == x0.sr));
+    const bool fused = x0.has_cs && (!x1 || x1->has_cs);
     float* stats;
     int slabs;
     if (fused) {  // statistics came out of the producing GEMM epilogues: one small fixed-order reduction, no pass over x
-      const int nb = HW / x0.sr;
+      const int nb = HW / kStatRows;
       slabs = groupnorm_colstats_chunks(nb);
       stats = new_stats(slabs);
       const float* c0 = x0.cs; const float* c1 = x1 ? x1->cs : nullptr;
@@ -945,12 +955,10 @@ struct Model {
       { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o2); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
       lora_wgrad(tb + ".attn2.to_out.0", att2.p, C, dh16.p, C, M, C, C);
       B16T dq2 = b.b16(size_t(M) * C);
-      { const bf16* q = q2.p; const bf16* kv = kv_all.p; const bf16* o = att2.p; const bf16* dop = datt.p; bf16* dqp = dq2.p; bf16* dkv = dkv_all.p; float* sp = ascr.p;
-        const float* lse = lse2.p;
-        b.emit([=](cudaStream_t st) {
-          return attention_bwd(q, C, kv + kvo, ldkv, kv + kvo + C, ldkv, o, C, dop, C, dqp, C, dkv + kvo, ldkv, dkv + kvo + C, ldkv, Bn, heads, d_head, n_tok, 77,
-                               long(n_tok) * C, long(77) * ldkv, long(77) * ldkv, long(n_tok) * C, long(n_tok) * C, long(n_tok) * C, long(77) * ldkv,
-                               long(77) * ldkv, sc, sp, h16, st, lse); }); }
+      { const bf16* kv = kv_all.p; bf16* dkv = dkv_all.p;
+        b.attention_bwd(q2.p, C, kv ? kv + kvo : nullptr, ldkv, kv ? kv + kvo + C : nullptr, ldkv, att2.p, C, datt.p, C, dq2.p, C, dkv ? dkv + kvo : nullptr,
+                        ldkv, dkv ? dkv + kvo + C : nullptr, ldkv, Bn, heads, d_head, n_tok, 77, long(n_tok) * C, long(77) * ldkv, long(77) * ldkv,
+                        long(n_tok) * C, long(n_tok) * C, long(n_tok) * C, long(77) * ldkv, long(77) * ldkv, sc, ascr.p, lse2.p); }
       lora_wgrad(tb + ".attn2.to_q", l2.p, C, dq2.p, C, M, C, C);
       lora_wgrad(tb + ".attn2.to_k", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo : nullptr, ldkv, long(Bn) * 77, C, 768);
       lora_wgrad(tb + ".attn2.to_v", ctx16_saved.p, 768, dkv_all.p ? dkv_all.p + kvo + C : nullptr, ldkv, long(Bn) * 77, C, 768);
@@ -961,12 +969,10 @@ struct Model {
       { GemmDesc d; d.seg[0] = Builder::seg_plain(dh16.p, M, C); d.M = Mi; d.N = C; d.Nw = C; d.w = b.dpw(w_o1); d.out_bf16 = datt.p; d.ldo16 = C; b.gemm(d); }
       lora_wgrad(tb + ".attn1.to_out.0", att.p, C, dh16.p, C, M, C, C);
       B16T dqkv = b.b16(size_t(M) * 3 * C);
-      { const bf16* q = qkv.p; const bf16* o = att.p; const bf16* dop = datt.p; bf16* dq = dqkv.p; float* sp = ascr.p;
-        const float* lse = lse1.p;
-        b.emit([=](cudaStream_t st) {
-          return attention_bwd(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, o, C, dop, C, dq, 3 * C, dq + C, 3 * C, dq + 2 * C, 3 * C, Bn, heads, d_head, n_tok, n_tok,
-                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * C, long(n_tok) * C, long(n_tok) * 3 * C,
-                               long(n_tok) * 3 * C, long(n_tok) * 3 * C, sc, sp, h16, st, lse); }); }
+      { const bf16* q = qkv.p; bf16* dq = dqkv.p;
+        b.attention_bwd(q, 3 * C, q + C, 3 * C, q + 2 * C, 3 * C, att.p, C, datt.p, C, dq, 3 * C, dq + C, 3 * C, dq + 2 * C, 3 * C, Bn, heads, d_head, n_tok,
+                        n_tok, long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * 3 * C, long(n_tok) * C, long(n_tok) * C, long(n_tok) * 3 * C,
+                        long(n_tok) * 3 * C, long(n_tok) * 3 * C, sc, ascr.p, lse1.p); }
       b.free(datt);
       lora_wgrad(tb + ".attn1.to_q", l1.p, C, dqkv.p, 3 * C, M, C, C);
       lora_wgrad(tb + ".attn1.to_k", l1.p, C, dqkv.p ? dqkv.p + C : nullptr, 3 * C, M, C, C);
@@ -1552,7 +1558,7 @@ struct Model {
       const double pel = double(Bn) * HW * Cout;
       auto tail_stats = [&](const Act& t, const float* src, float* dst) {  // [B,32,2] group sums of a fp32 [M,Cout] tensor
         if (t.has_cs) {
-          const float* cst = t.cs; const int nb = HW / t.sr; const int S = groupnorm_colstats_chunks(nb);
+          const float* cst = t.cs; const int nb = HW / kStatRows; const int S = groupnorm_colstats_chunks(nb);
           float* part = b.new_stats(S);
           b.emit([=](cudaStream_t st) { return groupnorm_colstats_reduce(cst, Cout, nullptr, 0, Bn, nb, part, st); }, false, MADM_KIND_GROUPNORM,
                  0.0, double(Bn) * nb * Cout * 8);

@@ -43,46 +43,6 @@ enum { TMA_EPI_NONE = 0, TMA_EPI_F32 = 1, TMA_EPI_RED = 2, TMA_EPI_H16 = 3, TMA_
 #define EPI_BATCH 4
 #endif
 
-struct GemmParams {
-  CUtensorMap tmA[2];
-  CUtensorMap tmB;
-  CUtensorMap tmR;   // TMA_EPI_RES_H16: the out-of-place fp32 residual (box 32 x 32, 128B swizzle), loaded per chunk into the warp's staging
-  CUtensorMap tmO;   // output tensor map of the TMA-store epilogue (box 32 columns x 32 rows; fp32 with 128B swizzle or 16-bit with 64B swizzle)
-  int tma_epi;       // TMA_EPI_*: 0 = coalesced-store epilogue, else the epilogue hands 32x32 tiles to cp(.reduce).async.bulk.tensor
-  int nseg;
-  int kchunks[2];
-  int cpt[2];
-  int8_t dx[2][9];
-  int8_t dy[2][9];
-  int boff[2][9];
-  int M, N;
-  int W, pix;  // output grid width and pixels per image
-  int box_w, box_h, box_b;
-  const float* bias;
-  const float* rowbias;
-  int rows_per_img;
-  int ld_rowbias;
-  const float* residual;
-  int ldr;
-  int res16;  // the residual is a 16-bit tensor (operand dtype) instead of fp32
-  float* out_f32;
-  int ldo32;
-  __nv_bfloat16* out_bf16;
-  int ldo16;
-  int act;
-  float alpha;
-  int vec_ok;
-  int n_tiles;
-  int fp16;
-  int num_tiles;
-  int s2d_H, s2d_W;  // if s2d_W > 0 the 16-bit output is written in space-to-depth layout [4 phases][B][H/2][W/2][N] of an HxW image grid
-  int s2d_B;
-  int splits;        // split-K factor: tile t covers K range (t % splits) of output tile (t / splits) and writes raw partials
-  long split_stride; // elements between the partial outputs of consecutive splits (out_f32 + split * split_stride)
-  float* colstats;   // [ceil(M/32)][N][2] per-column (sum, sum of squares) of the stored outputs per 32-row block, or null
-  int stat_rows;     // always 32 (one block per epilogue warp)
-};
-
 // MT = M sub-tiles (128 rows each) per CTA tile.  MT = 2 loads one W box per K chunk for two A boxes (tile 256 x BN): the
 // L2->SM operand traffic per FLOP drops from (128+BN) to (256+BN)/2 bytes-equivalents, which is what bounds the BN = 128
 // layers (measured 12.7 TB/s of L2->SM reads at 42 % tensor-pipe activity on the VAE 512^2 convs).
@@ -809,7 +769,8 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-static EncodeTiledFn get_encode_fn() {
+const char* encode_tensor_map(CUtensorMap* tm, const char* op, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
+                              const cuuint32_t* box, CUtensorMapDataType dt, CUtensorMapSwizzle sw) {
   static EncodeTiledFn fn = nullptr;
   static std::once_flag once;
   std::call_once(once, [] {
@@ -819,20 +780,16 @@ static EncodeTiledFn get_encode_fn() {
         qres == cudaDriverEntryPointSuccess)
       fn = reinterpret_cast<EncodeTiledFn>(p);
   });
-  return fn;
-}
-
-static const char* encode_map(CUtensorMap* tm, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
-                              const cuuint32_t* box, CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_UINT16,
-                              CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B) {
-  EncodeTiledFn fn = get_encode_fn();
-  if (!fn) return "cuTensorMapEncodeTiled unavailable (no CUDA driver)";
+  static thread_local char buf[192];
+  if (!fn) {
+    snprintf(buf, sizeof(buf), "%s: cuTensorMapEncodeTiled unavailable (no CUDA driver)", op);
+    return buf;
+  }
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = fn(tm, dt, rank, const_cast<void*>(ptr), dims, strides_bytes, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, sw,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    static thread_local char buf[160];
-    snprintf(buf, sizeof(buf), "cuTensorMapEncodeTiled failed (CUresult %d, rank %d, dims %llu/%llu)", int(r), rank,
+    snprintf(buf, sizeof(buf), "%s: cuTensorMapEncodeTiled failed (CUresult %d, rank %d, dims %llu/%llu)", op, int(r), rank,
              (unsigned long long)dims[0], (unsigned long long)dims[1]);
     return buf;
   }
@@ -875,15 +832,9 @@ static int pick_bn(const GemmDesc& d) {
   return best;
 }
 
-int gemm_auto_tiles(const GemmDesc& d) {
-  const int bn = d.bn ? d.bn : pick_bn(d);
-  const int Ncols = (d.act == ACT_GEGLU) ? 2 * d.N : d.N;
-  return ((d.M + BM - 1) / BM) * ((Ncols + bn - 1) / bn);
-}
-
 const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
   GemmLaunch& L = *out;
-  L.d = d;
+  GemmParams& p = L.p;
   if (d.nseg < 1 || d.nseg > 2) return "gemm: nseg must be 1 or 2";
   if (d.M <= 0 || d.N <= 0) return "gemm: empty problem";
   if (!d.out_f32 && !d.out_bf16) return "gemm: no output";
@@ -900,32 +851,32 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     if (d.N % 32 != 0 || d.ldr % 4 != 0 || (reinterpret_cast<uintptr_t>(d.residual) & 7) != 0)
       return "gemm: a 16-bit residual needs N % 32 == 0, ldr % 4 == 0 and an 8B-aligned pointer (vector epilogue only)";
   }
-  if (d.colstats) {
-    if (d.stat_rows != 32) return "gemm: stat_rows must be 32";
-    if (d.N % 32 != 0 || d.act == ACT_GEGLU) return "gemm: column statistics need N % 32 == 0 and a plain epilogue";
-  }
+  if (d.colstats && (d.N % 32 != 0 || d.act == ACT_GEGLU)) return "gemm: column statistics need N % 32 == 0 and a plain epilogue";
   L.bn = d.bn ? d.bn : pick_bn(d);
   const GemmASeg& s0 = d.seg[0];
   const int pix = s0.H * s0.W;
   if (d.M % pix != 0 && !(s0.H == 1)) return "gemm: M must be a multiple of H*W";
   // M-tile box over (W, H, B)
   if (s0.H == 1 && s0.Bt == 1) {  // plain [M,K] matrix: rows past M are zero-filled by TMA and masked in the epilogue
-    L.box_w = BM; L.box_h = 1; L.box_b = 1;
+    p.box_w = BM; p.box_h = 1; p.box_b = 1;
   } else if (s0.W >= BM) {
     if (s0.W % BM != 0) return "gemm: W must be a multiple of 128 when W >= 128";
-    L.box_w = BM; L.box_h = 1; L.box_b = 1;
+    p.box_w = BM; p.box_h = 1; p.box_b = 1;
   } else {
     if (BM % s0.W != 0) return "gemm: W must divide 128";
-    L.box_w = s0.W;
+    p.box_w = s0.W;
     int rows = BM / s0.W;
     if (s0.H >= rows) {
       if (s0.H % rows != 0) return "gemm: H must be a multiple of 128/W";
-      L.box_h = rows; L.box_b = 1;
+      p.box_h = rows; p.box_b = 1;
     } else {
       if (rows % s0.H != 0) return "gemm: H*W must divide 128";
-      L.box_h = s0.H; L.box_b = rows / s0.H;
+      p.box_h = s0.H; p.box_b = rows / s0.H;
     }
   }
+  p.nseg = d.nseg;
+  p.kchunks[1] = 0;
+  p.cpt[1] = 1;
   int ktot = 0;
   for (int s = 0; s < d.nseg; ++s) {
     const GemmASeg& sg = d.seg[s];
@@ -935,21 +886,31 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     const int ld = sg.ld ? sg.ld : sg.C;
     if (ld % 8 != 0) return "gemm: channel pitch must be a multiple of 8";
     if ((reinterpret_cast<uintptr_t>(sg.ptr) & 15) != 0) return "gemm: A pointer must be 16B aligned";
-    L.cpt[s] = sg.C / BK;
-    L.kchunks[s] = sg.ntaps * L.cpt[s];
+    p.cpt[s] = sg.C / BK;
+    p.kchunks[s] = sg.ntaps * p.cpt[s];
     ktot += sg.ntaps * sg.C;
     cuuint64_t dims[4] = {cuuint64_t(sg.C), cuuint64_t(sg.W), cuuint64_t(sg.H), cuuint64_t(sg.Bt)};
     cuuint64_t strides[3] = {cuuint64_t(ld) * 2, cuuint64_t(sg.W) * ld * 2, cuuint64_t(sg.H) * sg.W * ld * 2};
-    cuuint32_t box[4] = {cuuint32_t(BK), cuuint32_t(L.box_w), cuuint32_t(L.box_h), cuuint32_t(L.box_b)};
-    if (const char* e = encode_map(&L.tmA[s], sg.ptr, 4, dims, strides, box)) return e;
+    cuuint32_t box[4] = {cuuint32_t(BK), cuuint32_t(p.box_w), cuuint32_t(p.box_h), cuuint32_t(p.box_b)};
+    if (const char* e = encode_tensor_map(&p.tmA[s], "gemm", sg.ptr, 4, dims, strides, box)) return e;
   }
-  const int Ncols = (d.act == ACT_GEGLU) ? 2 * d.N : d.N;
-  const int n_tiles = (Ncols + L.bn - 1) / L.bn;
+  if (d.nseg == 1) p.tmA[1] = p.tmA[0];
+  for (int s = 0; s < 2; ++s)
+    for (int t = 0; t < 9; ++t) {
+      p.dx[s][t] = d.seg[s].dx[t];
+      p.dy[s][t] = d.seg[s].dy[t];
+      p.boff[s][t] = d.seg[s].b_off[t];
+    }
+  p.M = d.M;
+  p.N = (d.act == ACT_GEGLU) ? 2 * d.N : d.N;
+  p.W = s0.W;
+  p.pix = pix;
+  p.n_tiles = (p.N + L.bn - 1) / L.bn;
   // 256-row CTA tiles (two M sub-tiles sharing each W box) for the 128-wide N tile when there is enough work to keep every SM
   // busy with the larger tiles
   L.mt = 1;
   if (L.bn == 128 && d.mt != 1) {
-    const long tiles2 = long((d.M + 2 * BM - 1) / (2 * BM)) * n_tiles;
+    const long tiles2 = long((d.M + 2 * BM - 1) / (2 * BM)) * p.n_tiles;
     if (d.mt == 2 || tiles2 >= 2L * num_sms()) L.mt = 2;
   }
   int m_tiles = (d.M + BM * L.mt - 1) / (BM * L.mt);
@@ -957,7 +918,7 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
   L.pair = 0;
   {
     const bool shape_ok = L.bn >= 128 && num_sms() % 2 == 0;
-    const long pair_tiles = long((m_tiles + 1) / 2) * n_tiles;
+    const long pair_tiles = long((m_tiles + 1) / 2) * p.n_tiles;
     if (shape_ok && d.pair >= 0 && (d.pair == 1 || pair_tiles >= num_sms() / 2)) L.pair = 1;
   }
   if (L.pair) m_tiles = (m_tiles + 1) / 2;  // tiles of the pair
@@ -969,61 +930,64 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     if (ldw % 8 != 0 || ldw < ktot) return "gemm: weight pitch must be >= Ktot and a multiple of 8";
     cuuint64_t strides[1] = {cuuint64_t(ldw) * 2};
     cuuint32_t box[2] = {cuuint32_t(BK), cuuint32_t(L.pair ? L.bn / 2 : L.bn)};  // a pair's CTAs stage half of the W tile each
-    if (const char* e = encode_map(&L.tmB, d.w, 2, dims, strides, box)) return e;
+    if (const char* e = encode_tensor_map(&p.tmB, "gemm", d.w, 2, dims, strides, box)) return e;
   }
-  L.splits = 1;
-  L.split_stride = 0;
+  p.splits = 1;
+  p.split_stride = 0;
   if (d.splits > 1) {  // split-K: raw fp32 partials, reduced (with the fused epilogue) by splitk_reduce
     if (d.bias || d.rowbias || d.residual || d.out_bf16 || d.act != ACT_NONE || d.colstats || d.alpha != 1.0f || !d.out_f32)
       return "gemm: a split-K launch writes raw fp32 partials only";
-    L.splits = d.splits;
-    L.split_stride = d.split_stride;
+    p.splits = d.splits;
+    p.split_stride = d.split_stride;
   }
-  L.num_tiles = n_tiles * m_tiles * L.splits;
+  p.num_tiles = p.n_tiles * m_tiles * p.splits;
   // TMA-store epilogue: single-output launches whose 32-column chunks tile N exactly.  fp32 output -> bulk tensor store; in-place fp32
   // residual (hs += GEMM, no activation) -> bulk reduce-add at the L2; 16-bit output (also GEGLU) -> 16-bit tile store; fused GroupNorm
   // column statistics ride along (EPI_TMA | EPI_STATS), except with the reduce-add, whose sums never enter the SM.  Space-to-depth,
   // split-K, two outputs and out-of-place / 16-bit residuals keep the coalesced epilogue.  MADM_GEMM_TMA_EPI=0 disables.
-  L.tma_epi = TMA_EPI_NONE;
+  auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+  p.tma_epi = TMA_EPI_NONE;
+  p.tmO = p.tmB;  // unused map slots hold a valid map
+  p.tmR = p.tmB;
   {
     const char* env = getenv("MADM_GEMM_TMA_EPI");
     const bool on = !(env && strcmp(env, "0") == 0);
-    auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
-    const bool plain = on && L.bn >= 32 && L.splits == 1 && d.s2d_W == 0 && d.N % 32 == 0 && (!d.bias || al16(d.bias)) &&
+    const bool plain = on && L.bn >= 32 && p.splits == 1 && d.s2d_W == 0 && d.N % 32 == 0 && (!d.bias || al16(d.bias)) &&
                        (!d.rowbias || (al16(d.rowbias) && (d.ld_rowbias ? d.ld_rowbias : d.N) % 4 == 0));
     if (plain && d.act == ACT_GEGLU) {
-      if (al16(d.out_bf16) && d.ldo16 % 8 == 0) L.tma_epi = TMA_EPI_H16;
+      if (al16(d.out_bf16) && d.ldo16 % 8 == 0) p.tma_epi = TMA_EPI_H16;
     } else if (plain && d.out_f32 && !d.out_bf16 && al16(d.out_f32) && d.ldo32 % 4 == 0) {
-      if (!d.residual) L.tma_epi = TMA_EPI_F32;
-      else if (!d.res16 && d.residual == d.out_f32 && d.ldr == d.ldo32 && d.act == ACT_NONE && !d.colstats) L.tma_epi = TMA_EPI_RED;
+      if (!d.residual) p.tma_epi = TMA_EPI_F32;
+      else if (!d.res16 && d.residual == d.out_f32 && d.ldr == d.ldo32 && d.act == ACT_NONE && !d.colstats) p.tma_epi = TMA_EPI_RED;
     } else if (plain && d.out_bf16 && !d.out_f32 && !d.residual && al16(d.out_bf16) && d.ldo16 % 8 == 0) {
-      L.tma_epi = TMA_EPI_H16;
+      p.tma_epi = TMA_EPI_H16;
     } else if (plain && d.out_bf16 && !d.out_f32 && d.residual && !d.res16 && !d.colstats && d.act == ACT_NONE && al16(d.out_bf16) && d.ldo16 % 8 == 0 &&
                al16(d.residual) && d.ldr % 4 == 0 && EPI_NBUF >= 2) {
-      L.tma_epi = TMA_EPI_RES_H16;  // out16 = 16-bit(GEMM + fp32 residual), residual out of place: the transformer's FF out-projection
+      p.tma_epi = TMA_EPI_RES_H16;  // out16 = 16-bit(GEMM + fp32 residual), residual out of place: the transformer's FF out-projection
     }
-    if (L.tma_epi == TMA_EPI_RES_H16) {
+    if (p.tma_epi == TMA_EPI_RES_H16) {
       cuuint64_t dims[2] = {cuuint64_t(d.N), cuuint64_t(d.M)};
       cuuint64_t strides[1] = {cuuint64_t(d.ldr) * 4};
       cuuint32_t box[2] = {32, 32};
-      if (const char* e = encode_map(&L.tmR, d.residual, 2, dims, strides, box, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, CU_TENSOR_MAP_SWIZZLE_128B)) return e;
+      if (const char* e = encode_tensor_map(&p.tmR, "gemm", d.residual, 2, dims, strides, box, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, CU_TENSOR_MAP_SWIZZLE_128B))
+        return e;
     }
-    if (L.tma_epi) {
-      const bool h16 = L.tma_epi == TMA_EPI_H16 || L.tma_epi == TMA_EPI_RES_H16;
+    if (p.tma_epi) {
+      const bool h16 = p.tma_epi == TMA_EPI_H16 || p.tma_epi == TMA_EPI_RES_H16;
       cuuint64_t dims[2] = {cuuint64_t(d.N), cuuint64_t(d.M)};
       cuuint64_t strides[1] = {h16 ? cuuint64_t(d.ldo16) * 2 : cuuint64_t(d.ldo32) * 4};
       cuuint32_t box[2] = {32, 32};
       const void* base = h16 ? static_cast<const void*>(d.out_bf16) : static_cast<const void*>(d.out_f32);
-      if (const char* e = encode_map(&L.tmO, base, 2, dims, strides, box, h16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
-                                     h16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B))
+      if (const char* e = encode_tensor_map(&p.tmO, "gemm", base, 2, dims, strides, box, h16 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
+                                            h16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B))
         return e;
     }
   }
   if (L.pair) {
-    const int pairs = L.num_tiles < num_sms() / 2 ? L.num_tiles : num_sms() / 2;
+    const int pairs = p.num_tiles < num_sms() / 2 ? p.num_tiles : num_sms() / 2;
     L.grid = dim3(unsigned(2 * pairs));
   } else {
-    L.grid = dim3(unsigned(L.num_tiles < num_sms() ? L.num_tiles : num_sms()));
+    L.grid = dim3(unsigned(p.num_tiles < num_sms() ? p.num_tiles : num_sms()));
   }
   switch (L.bn) {
     case 16: L.smem = Cfg<16, 1>::SMEM; break;
@@ -1035,98 +999,7 @@ const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out) {
     case 256: L.smem = L.pair ? Cfg<256, 1, true>::SMEM : Cfg<256, 1>::SMEM; break;
     default: return "gemm: unsupported N tile";
   }
-  return nullptr;
-}
-
-template <int BN, int MT, int EPI, bool PAIR>
-static const char* launch_bn_s(const GemmLaunch& L, const GemmParams& p, cudaStream_t stream) {
-  static bool attr_set = false;
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(gemm_tc_kernel<BN, MT, EPI, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                             int(Cfg<BN, MT, PAIR>::SMEM)) != cudaSuccess)
-      return "gemm: cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
-    attr_set = true;
-  }
-  if constexpr (PAIR) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = L.grid;
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = Cfg<BN, MT, PAIR>::SMEM;
-    cfg.stream = stream;
-    cudaLaunchAttribute at[2];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
-    if (pdl_train_scope()) {
-      at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-      at[1].val.programmaticStreamSerializationAllowed = 1;
-      cfg.numAttrs = 2;
-    }
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_tc_kernel<BN, MT, EPI, PAIR>, p);
-    if (e == cudaSuccess) return nullptr;
-    static thread_local char buf[160];
-    snprintf(buf, sizeof(buf), "gemm: cluster launch failed (%s)", cudaGetErrorString(e));
-    return buf;
-  } else {
-    const cudaError_t e = launch_k(gemm_tc_kernel<BN, MT, EPI, PAIR>, L.grid, dim3(kThreads), Cfg<BN, MT, PAIR>::SMEM, stream, p);
-    if (e == cudaSuccess) return nullptr;
-    static thread_local char buf[160];
-    cudaFuncAttributes fa{};
-    cudaFuncGetAttributes(&fa, gemm_tc_kernel<BN, MT, EPI, PAIR>);
-    snprintf(buf, sizeof(buf), "gemm: kernel launch failed (%s; %d regs, max %d threads, %d B smem)", cudaGetErrorString(e), fa.numRegs,
-             fa.maxThreadsPerBlock, int(Cfg<BN, MT, PAIR>::SMEM));
-    return buf;
-  }
-}
-template <int BN, int MT, bool PAIR>
-static const char* launch_epi(const GemmLaunch& L, const GemmParams& p, cudaStream_t stream) {
-  const int epi = (p.s2d_W > 0 ? EPI_S2D : 0) | (p.colstats ? EPI_STATS : 0);
-  if constexpr (BN >= 32) {  // (tma_epi is only chosen for launches without a space-to-depth output, see gemm_prepare)
-    if (p.tma_epi) return p.colstats ? launch_bn_s<BN, MT, EPI_TMA | EPI_STATS, PAIR>(L, p, stream) : launch_bn_s<BN, MT, EPI_TMA, PAIR>(L, p, stream);
-  }
-  switch (epi) {
-    case 0: return launch_bn_s<BN, MT, 0, PAIR>(L, p, stream);
-    case 1: return launch_bn_s<BN, MT, 1, PAIR>(L, p, stream);
-    case 2: return launch_bn_s<BN, MT, 2, PAIR>(L, p, stream);
-    default: return launch_bn_s<BN, MT, 3, PAIR>(L, p, stream);
-  }
-}
-template <int BN>
-static const char* launch_bn(const GemmLaunch& L, const GemmParams& p, cudaStream_t stream) {
-  if constexpr (BN == 128) {
-    if (L.mt == 2) return L.pair ? launch_epi<BN, 2, true>(L, p, stream) : launch_epi<BN, 2, false>(L, p, stream);
-  }
-  if constexpr (BN >= 128) {
-    if (L.pair) return launch_epi<BN, 1, true>(L, p, stream);
-  }
-  return launch_epi<BN, 1, false>(L, p, stream);
-}
-
-const char* gemm_launch(const GemmLaunch& L, cudaStream_t stream) {
-  const GemmDesc& d = L.d;
-  GemmParams p;
-  p.tmA[0] = L.tmA[0];
-  p.tmA[1] = L.tmA[d.nseg > 1 ? 1 : 0];
-  p.tmB = L.tmB;
-  p.tma_epi = L.tma_epi;
-  if (L.tma_epi) p.tmO = L.tmO; else p.tmO = L.tmB;
-  p.tmR = L.tma_epi == TMA_EPI_RES_H16 ? L.tmR : L.tmB;
-  p.nseg = d.nseg;
-  for (int s = 0; s < 2; ++s) {
-    p.kchunks[s] = s < d.nseg ? L.kchunks[s] : 0;
-    p.cpt[s] = s < d.nseg ? L.cpt[s] : 1;
-    for (int t = 0; t < 9; ++t) {
-      p.dx[s][t] = d.seg[s].dx[t];
-      p.dy[s][t] = d.seg[s].dy[t];
-      p.boff[s][t] = d.seg[s].b_off[t];
-    }
-  }
-  p.M = d.M;
-  p.N = (d.act == ACT_GEGLU) ? 2 * d.N : d.N;
-  p.W = d.seg[0].W;
-  p.pix = d.seg[0].H * d.seg[0].W;
-  p.box_w = L.box_w; p.box_h = L.box_h; p.box_b = L.box_b;
+  // epilogue operands
   p.bias = d.bias;
   p.rowbias = d.rowbias;
   p.rows_per_img = d.rows_per_img > 0 ? d.rows_per_img : 1;
@@ -1136,20 +1009,14 @@ const char* gemm_launch(const GemmLaunch& L, cudaStream_t stream) {
   p.out_bf16 = reinterpret_cast<__nv_bfloat16*>(d.out_bf16); p.ldo16 = d.ldo16;
   p.act = d.act;
   p.alpha = d.alpha;
-  auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+  p.fp16 = d.fp16;
+  p.colstats = d.colstats;
   p.vec_ok = (d.N % 8 == 0) && (!d.bias || al16(d.bias)) && (!d.rowbias || (al16(d.rowbias) && p.ld_rowbias % 4 == 0)) &&
              (!d.residual || (al16(d.residual) && d.ldr % 4 == 0)) && (!d.out_f32 || (al16(d.out_f32) && d.ldo32 % 4 == 0)) &&
              (!d.out_bf16 || (al16(d.out_bf16) && d.ldo16 % 8 == 0));
   if (d.res16 && !p.vec_ok) return "gemm: a 16-bit residual needs the vector epilogue (16B-aligned operands)";
   if (d.act == ACT_GEGLU && !p.vec_ok) return "gemm: GEGLU epilogue needs 16B-aligned outputs";
   if (d.s2d_W > 0 && !p.vec_ok) return "gemm: space-to-depth output needs 16B-aligned operands";
-  p.n_tiles = (p.N + L.bn - 1) / L.bn;
-  p.fp16 = d.fp16;
-  p.num_tiles = L.num_tiles;
-  p.colstats = d.colstats;
-  p.stat_rows = d.stat_rows;
-  p.splits = L.splits;
-  p.split_stride = L.split_stride;
   p.s2d_H = 0; p.s2d_W = 0; p.s2d_B = 0;
   if (d.s2d_W > 0) {  // the kernel takes log2(H), log2(W)
     int lh = 0, lw = 0;
@@ -1158,14 +1025,61 @@ const char* gemm_launch(const GemmLaunch& L, cudaStream_t stream) {
     if ((1 << lh) != d.s2d_H || (1 << lw) != d.s2d_W) return "gemm: space-to-depth output needs power-of-two H and W";
     p.s2d_H = lh; p.s2d_W = lw; p.s2d_B = d.M / (d.s2d_H * d.s2d_W);
   }
+  return nullptr;
+}
+
+template <int BN, int MT, int EPI, bool PAIR>
+static const char* launch_bn_s(const GemmLaunch& L, cudaStream_t stream) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    if (cudaFuncSetAttribute(gemm_tc_kernel<BN, MT, EPI, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             int(Cfg<BN, MT, PAIR>::SMEM)) != cudaSuccess)
+      return "gemm: cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed";
+    attr_set = true;
+  }
+  const cudaError_t e = launch_k<PAIR ? 2 : 1>(gemm_tc_kernel<BN, MT, EPI, PAIR>, L.grid, dim3(kThreads), L.smem, stream, L.p);
+  if (e == cudaSuccess) return nullptr;
+  static thread_local char buf[160];
+  cudaFuncAttributes fa{};
+  cudaFuncGetAttributes(&fa, gemm_tc_kernel<BN, MT, EPI, PAIR>);
+  snprintf(buf, sizeof(buf), "gemm: %s launch failed (%s; %d regs, max %d threads, %d B smem)", PAIR ? "cluster" : "kernel", cudaGetErrorString(e),
+           fa.numRegs, fa.maxThreadsPerBlock, int(L.smem));
+  return buf;
+}
+template <int BN, int MT, bool PAIR>
+static const char* launch_epi(const GemmLaunch& L, cudaStream_t stream) {
+  const GemmParams& p = L.p;
+  const int epi = (p.s2d_W > 0 ? EPI_S2D : 0) | (p.colstats ? EPI_STATS : 0);
+  if constexpr (BN >= 32) {  // (tma_epi is only chosen for launches without a space-to-depth output, see gemm_prepare)
+    if (p.tma_epi) return p.colstats ? launch_bn_s<BN, MT, EPI_TMA | EPI_STATS, PAIR>(L, stream) : launch_bn_s<BN, MT, EPI_TMA, PAIR>(L, stream);
+  }
+  switch (epi) {
+    case 0: return launch_bn_s<BN, MT, 0, PAIR>(L, stream);
+    case 1: return launch_bn_s<BN, MT, 1, PAIR>(L, stream);
+    case 2: return launch_bn_s<BN, MT, 2, PAIR>(L, stream);
+    default: return launch_bn_s<BN, MT, 3, PAIR>(L, stream);
+  }
+}
+template <int BN>
+static const char* launch_bn(const GemmLaunch& L, cudaStream_t stream) {
+  if constexpr (BN == 128) {
+    if (L.mt == 2) return L.pair ? launch_epi<BN, 2, true>(L, stream) : launch_epi<BN, 2, false>(L, stream);
+  }
+  if constexpr (BN >= 128) {
+    if (L.pair) return launch_epi<BN, 1, true>(L, stream);
+  }
+  return launch_epi<BN, 1, false>(L, stream);
+}
+
+const char* gemm_launch(const GemmLaunch& L, cudaStream_t stream) {
   switch (L.bn) {
-    case 16: return launch_bn<16>(L, p, stream);
-    case 32: return launch_bn<32>(L, p, stream);
-    case 64: return launch_bn<64>(L, p, stream);
-    case 128: return launch_bn<128>(L, p, stream);
-    case 160: return launch_bn<160>(L, p, stream);
-    case 192: return launch_bn<192>(L, p, stream);
-    case 256: return launch_bn<256>(L, p, stream);
+    case 16: return launch_bn<16>(L, stream);
+    case 32: return launch_bn<32>(L, stream);
+    case 64: return launch_bn<64>(L, stream);
+    case 128: return launch_bn<128>(L, stream);
+    case 160: return launch_bn<160>(L, stream);
+    case 192: return launch_bn<192>(L, stream);
+    case 256: return launch_bn<256>(L, stream);
   }
   return "gemm: unsupported N tile";
 }

@@ -1,6 +1,7 @@
 // Host-side interface of the tcgen05 implicit-GEMM kernel family (gemm_tc.cu).
 #pragma once
 #include <cuda.h>
+#include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -49,33 +50,65 @@ struct GemmDesc {
   int splits = 1;                   // split-K factor (>1: raw fp32 partial outputs at out_f32 + split * split_stride)
   long split_stride = 0;
   float* colstats = nullptr;        // optional [ceil(M/32)][N][2] per-column (sum, sumsq) of the outputs per 32-row block (fused GN statistics)
-  int stat_rows = 32;               // rows per statistics block (32: one block per epilogue warp)
 };
 
-struct GemmLaunch {  // prepared launch: tensor maps encoded once, replayed per forward
-  alignas(64) CUtensorMap tmA[2];
-  alignas(64) CUtensorMap tmB;
-  alignas(64) CUtensorMap tmO;  // output map of the TMA-store epilogue (valid when tma_epi != 0)
-  alignas(64) CUtensorMap tmR;  // residual map (tma_epi == 4)
-  int tma_epi = 0;           // 0 coalesced-store epilogue, 1 fp32 bulk store, 2 fp32 bulk reduce-add (in-place residual), 3 16-bit bulk store, 4 fp32 residual tile by TMA load + 16-bit bulk store
-  GemmDesc d;
+// Kernel parameters, filled once by gemm_prepare (tensor maps encoded) and passed as they are on every launch
+struct GemmParams {
+  CUtensorMap tmA[2];
+  CUtensorMap tmB;
+  CUtensorMap tmR;   // TMA_EPI_RES_H16: the out-of-place fp32 residual (box 32 x 32, 128B swizzle), loaded per chunk into the warp's staging
+  CUtensorMap tmO;   // output tensor map of the TMA-store epilogue (box 32 columns x 32 rows; fp32 with 128B swizzle or 16-bit with 64B swizzle)
+  int tma_epi;       // TMA_EPI_*: 0 = coalesced-store epilogue, else the epilogue hands 32x32 tiles to cp(.reduce).async.bulk.tensor
+  int nseg;
+  int kchunks[2];    // 64-wide K chunks per segment
+  int cpt[2];        // chunks per tap
+  int8_t dx[2][9];
+  int8_t dy[2][9];
+  int boff[2][9];
+  int M, N;
+  int W, pix;  // output grid width and pixels per image
+  int box_w, box_h, box_b;
+  const float* bias;
+  const float* rowbias;
+  int rows_per_img;
+  int ld_rowbias;
+  const float* residual;
+  int ldr;
+  int res16;  // the residual is a 16-bit tensor (operand dtype) instead of fp32
+  float* out_f32;
+  int ldo32;
+  __nv_bfloat16* out_bf16;
+  int ldo16;
+  int act;
+  float alpha;
+  int vec_ok;
+  int n_tiles;
+  int fp16;
+  int num_tiles;
+  int s2d_H, s2d_W;  // if s2d_W > 0 the 16-bit output is written in space-to-depth layout [4 phases][B][H/2][W/2][N] of an HxW image grid
+  int s2d_B;
+  int splits;        // split-K factor: tile t covers K range (t % splits) of output tile (t / splits) and writes raw partials
+  long split_stride; // elements between the partial outputs of consecutive splits (out_f32 + split * split_stride)
+  float* colstats;   // [ceil(M/32)][N][2] per-column (sum, sum of squares) of the stored outputs per 32-row block, or null
+};
+
+struct GemmLaunch {  // prepared launch: the kernel parameters and the instantiation that runs them
+  GemmParams p;
   int bn = 128;
-  int kchunks[2] = {0, 0};   // 64-wide K chunks per segment
-  int cpt[2] = {1, 1};       // chunks per tap
-  int box_w = 128, box_h = 1, box_b = 1;
-  dim3 grid;
-  int num_tiles = 0;
   int mt = 1;
   int pair = 0;              // launched as cta_group::2 pairs (cluster of 2): tiles are 2*mt*128 rows
-  int splits = 1;
-  long split_stride = 0;
+  dim3 grid;
   size_t smem = 0;
 };
 
-// Returns nullptr on success, else a static error string.
+// Returns nullptr on success, else a static error string.  gemm_prepare runs every check; gemm_launch only launches.
 const char* gemm_prepare(const GemmDesc& d, GemmLaunch* out);
 const char* gemm_launch(const GemmLaunch& l, cudaStream_t stream);
-// tiles (M/128 x N/BN) the auto-selected N tile would give: used by the planner to decide on split-K
-int gemm_auto_tiles(const GemmDesc& d);
+
+// Encodes a tiled TMA tensor map (the driver's cuTensorMapEncodeTiled, looked up once).  Returns nullptr on success, else an error string
+// that starts with `op` (the calling operator's name).
+const char* encode_tensor_map(CUtensorMap* tm, const char* op, const void* ptr, int rank, const cuuint64_t* dims, const cuuint64_t* strides_bytes,
+                              const cuuint32_t* box, CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_UINT16,
+                              CUtensorMapSwizzle sw = CU_TENSOR_MAP_SWIZZLE_128B);
 
 }  // namespace madm

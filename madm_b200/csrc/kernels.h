@@ -59,6 +59,9 @@ const char* flash_attention_tc_prepare(const void* q, int ldq, const void* k, in
                                        int heads, int d, int Nq, int Nk, long q_bstride, long kv_bstride, long o_bstride, float scale,
                                        int fp16, FaLaunch* out, float* lse = nullptr /* optional [B,heads,Nq] log-sum-exp output */);
 const char* flash_attention_tc_launch(const FaLaunch& l, cudaStream_t st);
+// tensor map of the [d, heads, tokens, batch] view of a 16-bit [batch, tokens, ld] buffer whose head h occupies columns [h*d, (h+1)*d):
+// box = 64 columns (zero-filled past d) x box_rows tokens; errors start with `op`
+const char* attention_head_map(CUtensorMap* tm, const char* op, const void* ptr, int d, int heads, int ntok, int B, int ld, long bstride, int box_rows);
 
 // ---- elementwise.cu
 // img NCHW fp32 in [0,1] -> (img-0.5)/0.5 -> 3x3 im2col rows [B*H*W, 64] bf16 (27 real columns, tap-major (ky,kx,c))
@@ -172,11 +175,22 @@ const char* scale_copy_f32(const float* src, long n, float scale, float* dst, cu
 const char* temb_silu_bwd(const float* d_act, const float* emb, const float* cond_emb, long n, float scale, float* d_cond_emb, cudaStream_t st);
 
 // ---- attention_bwd.cu: gradients of softmax(Q K^T scale) V per (image, head); scratch = attention_bwd_scratch_floats(B, heads, d, Nq, Nk) floats
+// (prepared launch: shapes checked, parameter blocks filled and tensor maps encoded once)
+struct AttnBwdLaunch {
+  alignas(64) unsigned char tc[2][640];   // tcgen05 roles (dK / dV, then dQ) when attention_bwd_tc_supported: parameter blocks, tensor maps encoded
+  alignas(64) unsigned char params[256];  // parameter block of the warp-level kernels, query split included
+  dim3 gq, gk, gtc[2];                    // grids: query blocks, key blocks x query split, the two tcgen05 roles
+  int B = 0;
+  int fp16 = 0, dp = 0;                   // dispatch: operand dtype, head dim padded to a multiple of 16
+  bool have_lse = false;                  // the forward's log-sum-exp is given: the L / D pass only computes D
+};
 size_t attention_bwd_scratch_floats(int B, int heads, int d, int Nq, int Nk);
-const char* attention_bwd(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* o, int ldo, const void* dout, int lddo,
-                          void* dq, int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs,
-                          long v_bs, long o_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, float* scratch, int fp16, cudaStream_t st,
-                          const float* lse = nullptr /* [B,heads,Nq] from the forward kernel: skips the backward's own Q K^T pass */);
+const char* attention_bwd_prepare(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* o, int ldo, const void* dout,
+                                  int lddo, void* dq, int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs,
+                                  long k_bs, long v_bs, long o_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, float* scratch, int fp16,
+                                  AttnBwdLaunch* out,
+                                  const float* lse = nullptr /* [B,heads,Nq] from the forward kernel: skips the backward's own Q K^T pass */);
+const char* attention_bwd_launch(const AttnBwdLaunch& l, cudaStream_t st);
 
 // fused LoRA factor gradients of one rank-16 wrapped linear (wgrad.cu): gB [N,16] = alpha dY^T (X A^T), gA [16,K] = alpha (dY B)^T X;
 // a16 = lora_A [16,K], bt16 = lora_B^T [16,N] in the operand dtype; scratch = lora_grads_scratch_floats(M, N, K) floats
@@ -185,12 +199,15 @@ size_t lora_grads_scratch_floats(int M, int N, int K);
 const char* lora_grads(const void* x16, int ldx, const void* dy16, int ldy, const void* a16, const void* bt16, int M, int N, int K, float alpha, float* gA,
                        float* gB, float* scratch, int fp16, cudaStream_t st);
 
-// ---- attention_bwd_tc.cu: the same gradients on tcgen05 / TMEM for d <= 64 and token counts that are multiples of 128 (the UNet's 64x64 self-attention);
-// attention_bwd dispatches to it after its L / D pass.  L2 = log-sum-exp * log2(e), D = rowsum(dO * O), both [B, heads, Nq].
+// ---- attention_bwd_tc.cu: the same gradients on tcgen05 / TMEM for d = 40 / 80 and token counts that are multiples of 128 (the UNet's 64x64 and
+// 32x32 self-attention); attention_bwd_launch hands over to it after its L / D pass.  L2 = log-sum-exp * log2(e), D = rowsum(dO * O), both
+// [B, heads, Nq].  The prepare fills AttnBwdLaunch::tc and ::gtc.
 bool attention_bwd_tc_supported(int d, int Nq, int Nk);
-const char* attention_bwd_tc(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* dout, int lddo, void* dq, int lddq,
-                             void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs, long v_bs, long do_bs,
-                             long dq_bs, long dk_bs, long dv_bs, float scale, const float* L2, const float* D, int fp16, cudaStream_t st);
+const char* attention_bwd_tc_prepare(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, const void* dout, int lddo, void* dq,
+                                     int lddq, void* dk, int lddk, void* dv, int lddv, int B, int heads, int d, int Nq, int Nk, long q_bs, long k_bs,
+                                     long v_bs, long do_bs, long dq_bs, long dk_bs, long dv_bs, float scale, const float* L2, const float* D,
+                                     AttnBwdLaunch* out);
+const char* attention_bwd_tc_launch(const AttnBwdLaunch& l, cudaStream_t st);
 
 // ---- wgrad.cu: dW[n,k] = alpha * sum_m dY[m,n] X[m,k] (taps = 9: implicit im2col of X [Bimg,H,W,K]) -> out[n*so_n + k*so_k + tap*so_tap]
 int wgrad_splits(int M, int N, int K, int taps);

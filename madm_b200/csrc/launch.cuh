@@ -25,19 +25,25 @@ struct PdlTrainScope {  // RAII: launches issued while one is alive carry the PD
   ~PdlTrainScope() { pdl_train_scope() = prev; }
 };
 
-template <typename... KArgs, typename... Args>
+// CLUSTER > 1: the grid runs as clusters of CLUSTER consecutive CTAs along x
+template <unsigned CLUSTER = 1, typename... KArgs, typename... Args>
 inline cudaError_t launch_k(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
-  cudaLaunchAttribute at[1];
+  cudaLaunchAttribute at[2];
+  cfg.attrs = at;
+  if (CLUSTER > 1) {
+    at[cfg.numAttrs].id = cudaLaunchAttributeClusterDimension;
+    at[cfg.numAttrs].val.clusterDim.x = CLUSTER; at[cfg.numAttrs].val.clusterDim.y = 1; at[cfg.numAttrs].val.clusterDim.z = 1;
+    ++cfg.numAttrs;
+  }
   if (pdl_train_scope()) {
-    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at;
-    cfg.numAttrs = 1;
+    at[cfg.numAttrs].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[cfg.numAttrs].val.programmaticStreamSerializationAllowed = 1;
+    ++cfg.numAttrs;
   }
   return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
