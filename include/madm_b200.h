@@ -323,7 +323,11 @@ int madm_op_gn_add_relu_nchw(const float* a, const float* ga, const float* ba, c
  *   - the learned prompt / time conditioning, through d(cond_inputs) and d(cond_emb) (ldm_base.py:632-717: tiny tanh(alpha) * embed
  *     arithmetic that stays with the caller),
  * i.e. what `loss.backward()` produces in the reference's AMPTrainer.run_step (engine/train_loop.py:277-302) once the base UNet weights
- * are frozen, as BASELINE.json narrows config 5.  The VAE encoder runs without gradient (ldm_diffusers.py:282); base variant only.
+ * are frozen, as BASELINE.json narrows config 5.  The VAE encoder runs without gradient (ldm_diffusers.py:282).
+ * MADM_VARIANT_S0 (stages MADM_STAGE_ALL_S0): the VAE decoder runs without gradient too and its image is detached before it becomes the first
+ * feature (ldm_diffusers.py:191-201), so d(s0) reaches feature_projections.0.* only; madm_backward_args.d_unet_sample, the gradient of
+ * 'before_vae.decoder' (the UNet's final output, which the meta-arch's vae_decoder_loss differentiates), enters the UNet through the frozen
+ * conv_out / conv_norm_out and joins the gradient of up layer 11's output.
  *
  * Protocol: madm_pack_dgrad_weights (after every parameter update / adapter switch, next to madm_pack_weights) -> madm_extract with
  * MADM_FLAG_TRAIN (keeps every activation the backward needs in the training workspace; B <= 8) -> madm_backward with the gradients of
@@ -355,6 +359,8 @@ typedef struct madm_backward_args {
   const void* packed_dgrad;    /* madm_pack_dgrad_weights arena */
   void* workspace;             /* the training workspace the MADM_FLAG_TRAIN forward ran in */
   size_t workspace_bytes;
+  const float* d_unet_sample;  /* MADM_VARIANT_S0: gradient of madm_extract_args.unet_sample ('before_vae.decoder'), fp32 NCHW [B,4,64,64];
+                                  NULL = no loss term on it (the UNet-output backward does no work) */
 } madm_backward_args;
 int madm_backward(madm_ctx* ctx, const madm_backward_args* args, madm_stream stream);
 /* number of kernels one madm_backward call launches (after a MADM_FLAG_TRAIN forward at this B) */
@@ -369,6 +375,13 @@ int madm_op_groupnorm_bwd(const void* x0, int32_t C0, const void* x1, int32_t C1
                           const float* gamma, const float* beta, float eps, int32_t act, const void* dy16, const float* extra, float* scratch,
                           void* out16, float* dx0, int32_t acc0, float* dx1, int32_t acc1, float* dgamma, float* dbeta, int32_t dtype,
                           madm_stream stream);
+/* backward of z = GroupNorm(32)(conv1x1(x; w [C,3], no bias)) (-> ReLU if relu) on a 3-channel image, the K = 3 branches of the s0 projection
+ * (feature_projections.0 conv1 with its ReLU, shortcut without), without materialising z or the conv output: img4 fp32 [B*HW][4] (3 used);
+ * dy16 [B,HW,C] = gradient of the branch output.  Writes dw [C,3], dgamma [C], dbeta [C] (any may be NULL), multiplied by `scale`.  C % 32 == 0,
+ * C <= 1024, C/8 divides 256; scratch = madm_op_c3_gn_bwd_scratch_floats(B, C) floats */
+int64_t madm_op_c3_gn_bwd_scratch_floats(int32_t B, int32_t C);
+int madm_op_c3_gn_bwd(const float* img4, const float* w, const float* gamma, const float* beta, float eps, int32_t relu, int32_t B, int32_t HW,
+                      int32_t C, const void* dy16, float scale, float* dw, float* dgamma, float* dbeta, float* scratch, int32_t dtype, madm_stream stream);
 int madm_op_layernorm_bwd(const float* x, int32_t M, int32_t C, const float* gamma, float eps, const void* dy16, float* dx, int32_t accumulate,
                           int32_t dtype, madm_stream stream);
 /* GEGLU, natural column order: raw16 [M,2H] = (hidden | gate) -> out16 [M,H]; backward: draw16 [M,2H] */

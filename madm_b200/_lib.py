@@ -53,6 +53,7 @@ class MadmBackwardArgs(C.Structure):
         ("d_cond_inputs", c_void_p), ("d_cond_emb", c_void_p),
         ("adapter", c_char_p), ("lora_alpha_over_r", c_float), ("loss_scale", c_float),
         ("packed", c_void_p), ("packed_dgrad", c_void_p), ("workspace", c_void_p), ("workspace_bytes", c_size_t),
+        ("d_unet_sample", c_void_p),
     ]
 
 
@@ -145,6 +146,9 @@ SYMBOLS = {
     "madm_op_groupnorm_bwd_scratch_floats": (c_int, [c_int32, c_int32, c_int32]),
     "madm_op_groupnorm_bwd": (c_int, [c_void_p, c_int32, c_void_p, c_int32, c_int32, c_int32, c_int32, c_void_p, c_void_p, c_void_p, c_float, c_int32,
                                       c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_void_p, c_int32, c_void_p, c_void_p, c_int32, c_void_p]),
+    "madm_op_c3_gn_bwd_scratch_floats": (c_int64, [c_int32, c_int32]),
+    "madm_op_c3_gn_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_int32, c_int32, c_int32, c_int32, c_void_p, c_float, c_void_p,
+                                  c_void_p, c_void_p, c_void_p, c_int32, c_void_p]),
     "madm_op_layernorm_bwd": (c_int, [c_void_p, c_int32, c_int32, c_void_p, c_float, c_void_p, c_void_p, c_int32, c_int32, c_void_p]),
     "madm_op_geglu_fwd": (c_int, [c_void_p, c_int64, c_int32, c_void_p, c_int32, c_void_p]),
     "madm_op_geglu_bwd": (c_int, [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_int32, c_void_p]),

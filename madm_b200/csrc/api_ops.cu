@@ -246,6 +246,19 @@ int madm_op_groupnorm_bwd(const void* x0, int32_t C0, const void* x1, int32_t C1
   RUN(groupnorm_bwd(x0, C0, x1, C1, B, HW, in16, stats, gamma, beta, eps, act, dy16, dtype == MADM_DTYPE_FP16, partial, coef, chan, extra, out16, dx0,
                     acc0, dx1, acc1, dgamma, dbeta, 1.0f, static_cast<cudaStream_t>(stream)));
 }
+int64_t madm_op_c3_gn_bwd_scratch_floats(int32_t B, int32_t C) {
+  return int64_t(image_moments_floats(B)) + int64_t(B) * C * 4 + int64_t(c3_gn_bwd_scratch_floats(B, C));
+}
+int madm_op_c3_gn_bwd(const float* img4, const float* w, const float* gamma, const float* beta, float eps, int32_t relu, int32_t B, int32_t HW,
+                      int32_t C, const void* dy16, float scale, float* dw, float* dgamma, float* dbeta, float* scratch, int32_t dtype, madm_stream stream) {
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  float* mom = scratch;  // the forward's quantities the backward reads: image moments, folded conv + GroupNorm coefficients (ReLU mask)
+  float* coef = mom + image_moments_floats(B);
+  float* partial = coef + size_t(B) * C * 4;
+  if (const char* e = image_moments(img4, B, HW, mom, st)) return fail(e);
+  if (const char* e = c3_gn_coeffs(mom, w, gamma, beta, eps, B, HW, C, coef, st)) return fail(e);
+  RUN(c3_gn_bwd(img4, mom, coef, w, gamma, eps, relu, B, HW, C, dy16, dtype == MADM_DTYPE_FP16, scale, dw, dgamma, dbeta, partial, st));
+}
 int madm_op_layernorm_bwd(const float* x, int32_t M, int32_t C, const float* gamma, float eps, const void* dy16, float* dx, int32_t accumulate,
                           int32_t dtype, madm_stream stream) {
   RUN(layernorm_bwd(x, M, C, gamma, eps, dy16, dtype == MADM_DTYPE_FP16, dx, accumulate, static_cast<cudaStream_t>(stream)));

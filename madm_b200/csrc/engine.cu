@@ -206,8 +206,9 @@ struct Builder {
   std::string adapter;         // active LoRA adapter of this training plan ("" = none)
   float lora_scale = 0.f;
   std::vector<std::pair<int, std::function<void()>>> tape;  // (stage of the forward that recorded it, its backward)
-  // forward of a stage the training plan differentiates (not the VAE): its tensors stay allocated and each block records its backward
-  bool recording() const { return train && !bwd && cur_stage != MADM_STAGE_VAE; }
+  bool frozen = false;         // emitting a part of a differentiated stage that runs without gradient (the s0 variant's VAE decoder body)
+  // forward of a stage the training plan differentiates (not the VAE encoder): its tensors stay allocated and each block records its backward
+  bool recording() const { return train && !bwd && !frozen && cur_stage != MADM_STAGE_VAE; }
 
   // ---- workspace allocator (first-fit free list, 1 KB granularity); identical sequence in SIZE and PLAN modes
   struct Blk { size_t off, bytes; };
@@ -453,6 +454,17 @@ struct Builder {
     (bwd ? plan->bops : plan->ops)
         .push_back(Launch{std::move(op), cur_stage, cur_branch, kind, optional, flops, exec_flops < 0 ? flops : exec_flops, bytes});
   }
+  // launches emitted so far into the pass being built (PLAN mode; 0 otherwise)
+  size_t emitted() const { return mode == PLAN ? (bwd ? plan->bops : plan->ops).size() : 0; }
+  // makes the launches emitted since `from` do nothing in a call whose optional input *arg is null
+  void only_if_set(size_t from, const float* const* arg) {
+    if (mode != PLAN) return;
+    std::vector<Launch>& ops = bwd ? plan->bops : plan->ops;
+    for (size_t k = from; k < ops.size(); ++k) {
+      Op run = std::move(ops[k].run);
+      ops[k].run = [arg, run](cudaStream_t st) -> const char* { return *arg ? run(st) : nullptr; };
+    }
+  }
   // algo_flops < 0: 2*M*N*K from the descriptor (K counts real channels only when k_real is given)
   // split-K factor for a GEMM whose M x N tiling cannot fill the 148 SMs (8x8-resolution convs, small batches): the K range
   // is divided over `splits` CTAs per output tile; raw fp32 partials are reduced in fixed order by splitk_reduce, which
@@ -632,11 +644,13 @@ struct Builder {
 
   // ---- dgrad arena (training plans)
   const bf16* dpw(size_t off) const { return dpacked ? reinterpret_cast<const bf16*>(dpacked + off) : nullptr; }
-  // conv [Cout,Cin,k,k] -> [Cin, taps*Cout] (Cout % 64 == 0), the B operand of dX = dY (*) W^T
-  size_t dconv_w(const std::string& name, int Cout, int Cin, int taps) {
+  // conv [Cout,Cin,k,k] -> [Cin, taps*Cout] (Cout % 64 == 0), the B operand of dX = dY (*) W^T.  CoPad > 0: a few output channels, each tap
+  // padded to CoPad, K to a multiple of 64 (the layout latent_im2col gives the output gradient: taps x 4 channels, zero-padded to 64)
+  size_t dconv_w(const std::string& name, int Cout, int Cin, int taps, int CoPad = 0) {
+    const int Cp = CoPad > 0 ? CoPad : Cout, Kpad = CoPad > 0 ? (taps * CoPad + 63) / 64 * 64 : taps * Cout;
     return entry(ctx->dgrad, "dconv:" + name, [&] {
-      PackEntry e; e.kind = PK_CONV_DGRAD; e.src = name + ".weight"; e.N = Cout; e.C = Cin; e.taps = taps; e.Cpad = Cout; e.Kpad = taps * Cout;
-      e.ldo = taps * Cout; e.off = ctx->dgrad.reserve(size_t(Cin) * taps * Cout * 2);
+      PackEntry e; e.kind = PK_CONV_DGRAD; e.src = name + ".weight"; e.N = Cout; e.C = Cin; e.taps = taps; e.Cpad = Cp; e.Kpad = Kpad;
+      e.ldo = Kpad; e.off = ctx->dgrad.reserve(size_t(Cin) * Kpad * 2);
       return e;
     }).off;
   }
@@ -1390,6 +1404,8 @@ struct Model {
   // vae_decoder(latents=sample, output_final=True) (ldm_diffusers.py:192, :314-346): 1/0.18215 scale, post_quant_conv, conv_in,
   // mid block, 4 up blocks x 3 ResBlocks (512, 512, 256, 128 channels) with nearest-2x + conv between, GN + SiLU + conv 128 -> 3.
   // The decoded image (not clipped, ldm_diffusers.py:199) becomes the first feature of forward_features.
+  // Training plans: the UNet tail carries grad (the meta-arch's vae_decoder_loss differentiates 'before_vae.decoder') and records its backward;
+  // the decoder body runs without gradient and its image is detached (ldm_diffusers.py:191-201), so it records nothing.
   void build_dec() {
     b.cur_stage = MADM_STAGE_DEC;
     const int Bn = b.B;
@@ -1398,7 +1414,7 @@ struct Model {
     {
       const Act& x = unet_tap[0];  // output of up layer 11 (64x64x320), the UNet's last hidden state
       B16T n = b.b16(size_t(x.M()) * 320);
-      b.groupnorm(x, nullptr, kUnet + "conv_norm_out", 1e-5f, ACT_SILU, n.p, nullptr);
+      const Builder::GnSaved sv = b.groupnorm(x, nullptr, kUnet + "conv_norm_out", 1e-5f, ACT_SILU, n.p, nullptr);
       unet_sample = b.f32(size_t(x.M()) * 4);
       GemmDesc d; d.seg[0] = Builder::seg_3x3(n.p, Bn, 64, 64, 320); d.M = int(x.M()); d.N = 4; d.Nw = 4; d.bn = 16;
       d.w = b.pw(b.conv_w(kUnet + "conv_out", 4, 320, 9)); d.bias = P(kUnet + "conv_out.bias", 4); d.out_f32 = unet_sample.p; d.ldo32 = 4;
@@ -1407,7 +1423,33 @@ struct Model {
       { const float* src = unet_sample.p;
         b.emit([=](cudaStream_t st) -> const char* {
           return io->a.unet_sample ? nhwc_to_nchw(src, Bn, 64 * 64, 4, io->a.unet_sample, st) : nullptr; }, true); }
+      if (b.recording()) {
+        // ---- backward: d(unet_sample) -> conv_out input gradient -> conv_norm_out (GN + SiLU) backward, added to d(up layer 11 output)
+        const Act xin = x;
+        b.tape.push_back({b.cur_stage, [=]() {
+          const size_t w = b.dconv_w(kUnet + "conv_out", 4, 320, 9, /*CoPad=*/4);
+          const long M = xin.M();
+          const size_t from = b.emitted();
+          F32T g = b.f32(size_t(M) * 4);
+          B16T col = b.b16(size_t(M) * 64);
+          { float* gp = g.p; bf16* cp = col.p; const float S = b.loss_scale;
+            b.emit([=](cudaStream_t st) { return nchw_to_nhwc4(io->b.d_unet_sample, Bn, 4096, gp, st, S); });
+            b.emit([=](cudaStream_t st) { return latent_im2col(gp, Bn, 64, 64, cp, h16, st); }); }
+          B16T dn = b.b16(size_t(M) * 320);
+          { GemmDesc d; d.seg[0] = Builder::seg_plain(col.p, M, 64); d.M = int(M); d.N = 320; d.Nw = 320; d.w = b.dpw(w);
+            d.out_bf16 = dn.p; d.ldo16 = 320; b.gemm(d); }
+          int acc = 0;
+          float* dx = b.grad(xin, &acc);
+          // projection 1 has written this gradient already (its backward replays first), so a call without d_unet_sample may skip the term
+          if (!acc) b.fail(MADM_ESTATE, "training plan: the UNet-output backward must accumulate onto projection 1's input gradient");
+          b.groupnorm_bwd(xin, nullptr, false, sv, nullptr, kUnet + "conv_norm_out", 1e-5f, ACT_SILU, dn.p, nullptr, nullptr, dx, acc, nullptr, 0, nullptr,
+                          nullptr);
+          b.only_if_set(from, &io->b.d_unet_sample);
+          b.free(dn); b.free(col); b.free(g);
+        }});
+      }
     }
+    b.frozen = b.train;  // the decoder body: no gradient in a training plan
     const std::string dc = kVae + "decoder.";
     const long M0 = long(Bn) * 4096;
     F32T z = b.f32(size_t(M0) * 4);
@@ -1462,9 +1504,10 @@ struct Model {
         if (!io->a.decoded && !io->a.decoded_raw) return nullptr;
         return decoder_image_pack(src, Bn, 512 * 512, nullptr, io->a.decoded, io->a.decoded_raw, h16, st); }, true); }
     b.pin(enc_tap);
+    b.frozen = false;
   }
 
-  static const char* nchw_to_nhwc4(const float* src, int Bn, int HW, float* dst, cudaStream_t st);
+  static const char* nchw_to_nhwc4(const float* src, int Bn, int HW, float* dst, cudaStream_t st, float scale = 1.0f);
 
   // =========================================================================== feature projections
   // The four bottleneck projections are independent chains of small launches (1.0 ms of latency-bound kernels at B = 8).  Each is tagged as a
@@ -1594,7 +1637,8 @@ struct Model {
         // ---- backward
         b.tape.push_back({b.cur_stage, [=]() {
           const size_t wd3 = b.dconv_w(p + "conv3", Cout, Cb, 1), wd2 = b.dconv_w(p + "conv2", Cb, Cb, 9);
-          const size_t wd1 = b.dconv_w(p + "conv1", Cb, Cin, 1), wds = shortcut ? b.dconv_w(p + "shortcut", Cout, Cin, 1) : 0;
+          // (a 3-channel input is the detached decoded image: no input gradient, so no operands for it)
+          const size_t wd1 = rgb3 ? 0 : b.dconv_w(p + "conv1", Cb, Cin, 1), wds = shortcut && !rgb3 ? b.dconv_w(p + "shortcut", Cout, Cin, 1) : 0;
           const float S = b.loss_scale, inv = 1.0f / b.loss_scale;
           const int Mi = int(M);
           // d(z) = d(out) * (out > 0), NCHW -> NHWC, scaled by the loss scale
@@ -1630,6 +1674,24 @@ struct Model {
           B16T da1 = b.b16(size_t(M) * Cb);
           { GemmDesc d; d.seg[0] = Builder::seg_3x3(dc2.p, Bn, H, W, Cb); d.M = Mi; d.N = Cb; d.Nw = Cb; d.w = b.dpw(wd2); d.out_bf16 = da1.p; d.ldo16 = Cb; b.gemm(d); }
           b.free(dc2);
+          if (rgb3) {
+            // the two K = 3 branches: their conv / GroupNorm gradients from the image, its moments and the forward's folded coefficients
+            // (norm.cu c3_gn_bwd), without the conv outputs the forward never stored
+            auto c3_bwd = [&](const std::string& name, int C, const float* coef, const bf16* dy, int relu) {
+              F32T part = b.f32(c3_gn_bwd_scratch_floats(Bn, C));
+              const float* mp = mom.p; const float* wp = P(p + name + ".weight", int64_t(C) * 3); const float* gp = P(p + name + ".norm.weight", C);
+              float* dw = b.grad_buf(p + name + ".weight"); float* dg = b.grad_buf(p + name + ".norm.weight"); float* db = b.grad_buf(p + name + ".norm.bias");
+              float* pp = part.p;
+              b.emit([=](cudaStream_t st) { return c3_gn_bwd(img4, mp, coef, wp, gp, 1e-5f, relu, Bn, HW, C, dy, h16, inv, dw, dg, db, pp, st); }, false,
+                     MADM_KIND_GROUPNORM, 0.0, double(M) * (16 + 2.0 * C));
+              b.free(part);
+            };
+            c3_bwd("conv1", Cb, coef1.p, da1.p, 1);
+            b.free(da1);
+            c3_bwd("shortcut", Cout, coefs.p, dz.p, 0);
+            b.free(dz);
+            return;
+          }
           B16T dc1 = b.b16(size_t(M) * Cb);
           b.groupnorm_bwd(c1, nullptr, true, s1, nullptr, p + "conv1.norm", 1e-5f, ACT_RELU, da1.p, nullptr, dc1.p, nullptr, 0, nullptr, 0,
                           b.grad_buf(p + "conv1.norm.weight"), b.grad_buf(p + "conv1.norm.bias"));
@@ -1771,7 +1833,6 @@ struct Model {
   bool has_path() const { return b.ctx->params.count(kUnet + "conv_in.weight") != 0; }
   void build_all() {
     if (b.train) {  // forward that keeps its activations + the backward pass (SURVEY §8 row f-3)
-      if (s0()) b.fail(MADM_EINVAL, "training path: the base variant only (the s0 / vae_decoder_loss variant has no backward yet)");
       if (!has_path()) b.fail(MADM_ESTATE, "training path: UNet / VAE parameters are not registered");
     }
     if (has_path() || !has_head()) {  // a context that holds only sem_seg_head.* runs the head alone
@@ -1800,16 +1861,16 @@ struct Model {
   }
 };
 
-__global__ void nchw_to_nhwc4_kernel(const float* __restrict__ src, int Bn, int HW, float* __restrict__ dst) {
+__global__ void nchw_to_nhwc4_kernel(const float* __restrict__ src, int Bn, int HW, float scale, float* __restrict__ dst) {
   const long i = long(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= long(Bn) * HW) return;
   const int p = int(i % HW), bb = int(i / HW);
   const float* s = src + size_t(bb) * 4 * HW + p;
-  *reinterpret_cast<float4*>(dst + i * 4) = make_float4(s[0], s[HW], s[2 * HW], s[3 * HW]);
+  *reinterpret_cast<float4*>(dst + i * 4) = make_float4(s[0] * scale, s[HW] * scale, s[2 * HW] * scale, s[3 * HW] * scale);
 }
-const char* Model::nchw_to_nhwc4(const float* src, int Bn, int HW, float* dst, cudaStream_t st) {
+const char* Model::nchw_to_nhwc4(const float* src, int Bn, int HW, float* dst, cudaStream_t st, float scale) {
   const long total = long(Bn) * HW;
-  nchw_to_nhwc4_kernel<<<unsigned((total + 255) / 256), 256, 0, st>>>(src, Bn, HW, dst);
+  nchw_to_nhwc4_kernel<<<unsigned((total + 255) / 256), 256, 0, st>>>(src, Bn, HW, scale, dst);
   return cudaGetLastError() == cudaSuccess ? nullptr : "nchw_to_nhwc4 launch failed";
 }
 
@@ -2343,7 +2404,8 @@ extern "C" size_t madm_train_workspace_bytes(madm_ctx* ctx, int32_t B, const cha
 namespace {
 // madm_extract with MADM_FLAG_TRAIN: the forward of a training plan (activations kept for madm_backward)
 int extract_train(madm_ctx* ctx, const madm_extract_args* a, cudaStream_t st) {
-  if (a->stages != MADM_STAGE_ALL) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN runs all stages (MADM_STAGE_ALL)");
+  if (a->stages != (ctx->variant == MADM_VARIANT_S0 ? MADM_STAGE_ALL_S0 : MADM_STAGE_ALL))
+    return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN runs all stages (MADM_STAGE_ALL; MADM_STAGE_ALL_S0 in the s0 variant)");
   if (a->ema) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_TRAIN with the EMA projections (the teacher runs without gradient)");
   if (a->flags & MADM_FLAG_OUT_FP16) return set_err(ctx, MADM_EINVAL, "madm_extract: MADM_FLAG_OUT_FP16 with MADM_FLAG_TRAIN (madm_backward reads the fp32 outputs)");
   if (!a->packed_dgrad) return set_err(ctx, MADM_ESTATE, "madm_extract: MADM_FLAG_TRAIN needs packed_dgrad (madm_pack_dgrad_weights)");

@@ -46,6 +46,12 @@ const char* c3_conv_gn_relu(const float* img4, const float* coef, int B, int HW,
 // out NCHW = relu(GN(a; stats_a) + as_c . x + ds_c): the shortcut branch recomputed from the image
 const char* gn_add_relu_nchw_c3(const float* a, const float* stats_a, const float* ga, const float* ba, const float* img4, const float* coef_s, float eps,
                                 int B, int HW, int C, float* out_nchw, cudaStream_t st);
+// backward of one such branch z = GN32(conv1x1(x; w [C][3])) (-> ReLU if relu) from the image, its moments `mom` and the forward's `coef` (ReLU
+// mask): dy16 [B*HW, C] = gradient of the branch output -> dw [C][3], dgamma / dbeta [C] (each may be null), written, times `scale`.
+// Scratch: partial = c3_gn_bwd_scratch_floats(B, C) floats.
+size_t c3_gn_bwd_scratch_floats(int B, int C);
+const char* c3_gn_bwd(const float* img4, const float* mom, const float* coef, const float* w, const float* gamma, float eps, int relu, int B, int HW,
+                      int C, const void* dy16, int fp16, float scale, float* dw, float* dgamma, float* dbeta, float* partial, cudaStream_t st);
 
 // ---- attention_tc.cu : O[b, i, h*d:(h+1)*d] = softmax(Q K^T * scale) V per (image, head); 16-bit in/out, fp32 softmax, on tcgen05 / TMEM
 // (prepared launch: TMA tensor maps encoded once)

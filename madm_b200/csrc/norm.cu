@@ -700,4 +700,141 @@ const char* gn_add_relu_nchw_c3(const float* a, const float* stats_a, const floa
   return cudaGetLastError() == cudaSuccess ? nullptr : "gn_add_relu_nchw_c3 launch failed";
 }
 
+// ---- backward of one K = 3 branch z_c = GN(w_c . x)_c (-> ReLU) of the s0 projection (training path), again without its [B*HW, C] input.
+// With u_c = w_c . x, group g of cpg channels, mean mu_g, rstd r_g (from the image moments, as in the forward), N = HW * cpg, and the
+// per-image sums S_c = sum_p g_c, G_c = sum_p g_c x (g_c = dL/dz_c, masked by the ReLU):
+//     sum_p g_c xhat_c     = r_g (w_c . G_c - mu_g S_c)                          =: T_c        -> d gamma_c, and d beta_c = S_c
+//     sum_p xhat_c x       = r_g HW (E[x x^T] w_c - mu_g E[x])
+//     d w_c = r_g (gamma_c G_c - m1_g HW E[x] - m2_g sum_p xhat_c x),   m1_g = sum_{k in g} gamma_k S_k / N,  m2_g = sum_{k in g} gamma_k T_k / N
+// (the GroupNorm input gradient r_g (gamma_c g_c - m1_g - xhat_c m2_g) contracted with x).  So one streaming pass over dy and the image
+// (partials kernel: S_c and G_c per (image, slab), 4 sums per channel) and a small finish kernel that reduces them in fixed order and
+// applies the chain rule in double.
+static constexpr int kC3BwdSlabs = 128;  // partial sums per image: [B][128][C][4]
+
+__global__ void __launch_bounds__(256) c3_gn_bwd_partials_kernel(const uint16_t* __restrict__ dy16, const float4* __restrict__ img4,
+                                                                 const float4* __restrict__ coef, int HW, int C, int relu, int fp16,
+                                                                 float4* __restrict__ partial) {
+  pdl_trigger();  // programmatic dependent launch (launch.cuh): no global access before pdl_wait()
+  pdl_wait();
+  extern __shared__ float4 red[];  // [256 / (C/8)][C]
+  const int b = blockIdx.y, slab = blockIdx.x;
+  const int Q = C >> 3, q = threadIdx.x % Q, pl = threadIdx.x / Q, P = 256 / Q;
+  float4 cf[8], acc[8];
+#pragma unroll
+  for (int t = 0; t < 8; ++t) {
+    cf[t] = __ldg(coef + size_t(b) * C + q * 8 + t);
+    acc[t] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  const int per = (HW + kC3BwdSlabs - 1) / kC3BwdSlabs;
+  const int p0 = slab * per, p1 = min(HW, p0 + per);
+  for (int p = p0 + pl; p < p1; p += P) {
+    const float4 x = __ldg(img4 + size_t(b) * HW + p);
+    const uint4 raw = __ldg(reinterpret_cast<const uint4*>(dy16 + (size_t(b) * HW + p) * C + q * 8));
+    const uint32_t w4[4] = {raw.x, raw.y, raw.z, raw.w};
+#pragma unroll
+    for (int t2 = 0; t2 < 4; ++t2) {
+      float2 d;
+      if (fp16) d = __half22float2(*reinterpret_cast<const __half2*>(&w4[t2]));
+      else d = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w4[t2]));
+      const float dd[2] = {d.x, d.y};
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int t = 2 * t2 + h;
+        float g = dd[h];
+        // the forward's expression (c3_conv_gn_relu_kernel), so the ReLU mask is the forward's
+        if (relu && !(fmaf(cf[t].x, x.x, fmaf(cf[t].y, x.y, fmaf(cf[t].z, x.z, cf[t].w))) > 0.f)) g = 0.f;
+        acc[t].x += g;
+        acc[t].y = fmaf(g, x.x, acc[t].y);
+        acc[t].z = fmaf(g, x.y, acc[t].z);
+        acc[t].w = fmaf(g, x.z, acc[t].w);
+      }
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < 8; ++t) red[pl * C + q * 8 + t] = acc[t];
+  __syncthreads();
+  for (int c = threadIdx.x; c < C; c += 256) {  // fixed order over the pixel lanes
+    float4 s = red[c];
+    for (int l = 1; l < P; ++l) {
+      const float4 v = red[l * C + c];
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    partial[(size_t(b) * kC3BwdSlabs + slab) * C + c] = s;
+  }
+}
+
+// One CTA of C threads (thread = channel) walks the images in order; outputs are written (not accumulated), multiplied by `scale`.
+__global__ void c3_gn_bwd_finish_kernel(const float4* __restrict__ partial, const float* __restrict__ mom_partial, const float* __restrict__ w,
+                                        const float* __restrict__ gamma, float eps, int B, int HW, int C, float scale, float* __restrict__ dw,
+                                        float* __restrict__ dgamma, float* __restrict__ dbeta) {
+  pdl_trigger();  // programmatic dependent launch (launch.cuh): no global access before pdl_wait()
+  pdl_wait();
+  __shared__ double mom[9];
+  __shared__ double gs[1024], gt[1024];
+  const int c = threadIdx.x;
+  const int cpg = C / 32, g0 = (c / cpg) * cpg;
+  const double wc[3] = {w[c * 3], w[c * 3 + 1], w[c * 3 + 2]};
+  const double gam = gamma[c];
+  const double invN = 1.0 / (double(HW) * cpg);
+  double aw[3] = {0.0, 0.0, 0.0}, ag = 0.0, ab = 0.0;
+  for (int b = 0; b < B; ++b) {
+    if (c < 9) {  // the image's moments, reduced as c3_gn_coeffs_kernel does
+      double m = 0.0;
+      for (int sl = 0; sl < kMomSlabs; ++sl) m += double(mom_partial[(size_t(b) * kMomSlabs + sl) * 12 + c]);
+      mom[c] = m / double(HW);
+    }
+    double S = 0.0, G[3] = {0.0, 0.0, 0.0};
+    const float4* pp = partial + size_t(b) * kC3BwdSlabs * C + c;
+#pragma unroll 4
+    for (int sl = 0; sl < kC3BwdSlabs; ++sl) {
+      const float4 v = pp[size_t(sl) * C];
+      S += v.x; G[0] += v.y; G[1] += v.z; G[2] += v.w;
+    }
+    __syncthreads();
+    const double* mu = mom;     // E[x]
+    const double* Sx = mom + 3;  // E[x x^T]: xx xy xz yy yz zz
+    double m1 = 0.0, m2 = 0.0;
+    for (int k = g0; k < g0 + cpg; ++k) {
+      const double wx = w[k * 3], wy = w[k * 3 + 1], wz = w[k * 3 + 2];
+      m1 += wx * mu[0] + wy * mu[1] + wz * mu[2];
+      m2 += wx * wx * Sx[0] + 2.0 * wx * wy * Sx[1] + 2.0 * wx * wz * Sx[2] + wy * wy * Sx[3] + 2.0 * wy * wz * Sx[4] + wz * wz * Sx[5];
+    }
+    const double mean = m1 / cpg;
+    const double r = 1.0 / sqrt(fmax(m2 / cpg - mean * mean, 0.0) + double(eps));
+    const double T = r * (wc[0] * G[0] + wc[1] * G[1] + wc[2] * G[2] - mean * S);
+    gs[c] = gam * S;
+    gt[c] = gam * T;
+    __syncthreads();
+    double s1 = 0.0, s2 = 0.0;
+    for (int k = g0; k < g0 + cpg; ++k) { s1 += gs[k]; s2 += gt[k]; }
+    s1 *= invN; s2 *= invN;
+    const double Sw[3] = {Sx[0] * wc[0] + Sx[1] * wc[1] + Sx[2] * wc[2], Sx[1] * wc[0] + Sx[3] * wc[1] + Sx[4] * wc[2],
+                          Sx[2] * wc[0] + Sx[4] * wc[1] + Sx[5] * wc[2]};
+#pragma unroll
+    for (int j = 0; j < 3; ++j) aw[j] += r * (gam * G[j] - s1 * HW * mu[j] - s2 * r * HW * (Sw[j] - mean * mu[j]));
+    ag += T;
+    ab += S;
+    __syncthreads();  // mom / gs / gt are rewritten for the next image
+  }
+  if (dw) { dw[c * 3] = float(aw[0] * scale); dw[c * 3 + 1] = float(aw[1] * scale); dw[c * 3 + 2] = float(aw[2] * scale); }
+  if (dgamma) dgamma[c] = float(ag * scale);
+  if (dbeta) dbeta[c] = float(ab * scale);
+}
+
+size_t c3_gn_bwd_scratch_floats(int B, int C) { return size_t(B) * kC3BwdSlabs * C * 4; }
+
+const char* c3_gn_bwd(const float* img4, const float* mom, const float* coef, const float* w, const float* gamma, float eps, int relu, int B, int HW,
+                      int C, const void* dy16, int fp16, float scale, float* dw, float* dgamma, float* dbeta, float* partial, cudaStream_t st) {
+  if (C % 32 != 0 || C > 1024 || 256 % (C / 8) != 0) return "c3_gn_bwd: C must be a multiple of 32 with C/8 dividing 256";
+  const size_t smem = size_t(256 / (C / 8)) * C * sizeof(float4);
+  if (launch_k(c3_gn_bwd_partials_kernel, dim3(kC3BwdSlabs, B), dim3(256), smem, st, static_cast<const uint16_t*>(dy16),
+               reinterpret_cast<const float4*>(img4), reinterpret_cast<const float4*>(coef), HW, C, relu, fp16,
+               reinterpret_cast<float4*>(partial)) != cudaSuccess)
+    return "c3_gn_bwd partials launch failed";
+  if (launch_k(c3_gn_bwd_finish_kernel, dim3(1), dim3(C), 0, st, reinterpret_cast<const float4*>(partial), mom, w, gamma, eps, B, HW, C, scale, dw,
+               dgamma, dbeta) != cudaSuccess)
+    return "c3_gn_bwd finish launch failed";
+  return nullptr;
+}
+
 }  // namespace madm

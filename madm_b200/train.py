@@ -10,6 +10,11 @@ feature maps that carry a ``grad_fn``; ``loss.backward()`` then runs the CUDA en
 * ``cond_inputs`` / ``cond_emb`` — from which autograd itself reaches the learned prompt / time parameters through the tiny
   ``tanh(alpha) * embed`` arithmetic that stays in PyTorch (``ldm_base.py:675-717``).
 
+In the ``vae_decoder_loss`` / s0 variant the VAE decoder runs under ``no_grad`` and its image is detached before it becomes the first
+feature (``ldm_diffusers.py:191-201``): ``s0`` back-propagates into ``feature_projections.0`` only.  With ``return_unet_final_output=True``
+the UNet's final output ``before_vae.decoder`` carries grad (the meta-arch's ``vae_decoder_loss`` differentiates it) and
+``after_vae.decoder`` does not.
+
 Everything else must be frozen: BASELINE.json narrows the training configuration to LoRA gradients, so a call under grad with trainable
 BASE UNet weights (``finetune_unet='all'`` without freezing them) raises instead of silently dropping their gradients.  Several forwards
 may be in flight before one ``backward()`` (source pass + mixed pass, different adapters): each holds its own training workspace and
@@ -124,7 +129,7 @@ def trainable_sets(backbone, grad_inputs: Sequence[Tuple[str, torch.Tensor]]):
 
 class _ExtractFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, backbone, slot, eng, adapter, scaling, loss_scale, names, img, cond_inputs, cond_emb, timesteps, *params):
+    def forward(ctx, backbone, slot, eng, adapter, scaling, loss_scale, names, want_final, img, cond_inputs, cond_emb, timesteps, *params):
         dev = eng.device
         B = img.shape[0]
         lib = eng.lib
@@ -153,9 +158,9 @@ class _ExtractFn(torch.autograd.Function):
         ce = cond_emb.detach().to(torch.float32).reshape(-1, 1280).expand(B, 1280).contiguous()
         ts = timesteps.to(device=dev, dtype=torch.int64).contiguous()
         noise = backbone.feature_extractor.ldm_extractor.shared_noise
-        outs = [torch.empty(B, ch, side, side, dtype=torch.float32, device=dev) for ch, side in OUT_SHAPES["base"]]
+        outs = [torch.empty(B, ch, side, side, dtype=torch.float32, device=dev) for ch, side in OUT_SHAPES[eng.variant]]
         a = MadmExtractArgs()
-        a.B, a.stages, a.ema, a.flags = B, _lib.STAGE_ALL, 0, _lib.FLAG_TRAIN
+        a.B, a.stages, a.ema, a.flags = B, eng.stage_all, 0, _lib.FLAG_TRAIN
         a.img, a.cond_inputs, a.cond_emb, a.timesteps = img.data_ptr(), ci.data_ptr(), ce.data_ptr(), ts.data_ptr()
         a.shared_noise = noise.data_ptr()
         for i, t in enumerate(outs):
@@ -165,6 +170,11 @@ class _ExtractFn(torch.autograd.Function):
         a.range_flag = eng.range_flag.data_ptr()
         a.packed_dgrad = slot.dgrad.data_ptr()
         a.train_adapter, a.train_lora_scale, a.train_loss_scale = ad, float(scaling), float(loss_scale)
+        final = ()
+        if want_final:  # 'before_vae.decoder' (differentiable), 'after_vae.decoder' (not: the decoder runs under no_grad)
+            final = (torch.empty(B, 4, 64, 64, dtype=torch.float32, device=dev), torch.empty(B, 3, 512, 512, dtype=torch.float32, device=dev))
+            a.unet_sample, a.decoded = final[0].data_ptr(), final[1].data_ptr()
+            ctx.mark_non_differentiable(final[1])
         eng._range_poll()
         _lib.check(lib.madm_extract(eng.ctx, C.byref(a), st), eng.ctx, "madm_extract(train)")
         eng._range_publish()
@@ -175,7 +185,7 @@ class _ExtractFn(torch.autograd.Function):
         ctx.cond_shapes = (tuple(cond_inputs.shape), tuple(cond_emb.shape))
         ctx.save_for_backward(ce, *outs)
         ctx.set_materialize_grads(False)
-        return tuple(outs)
+        return tuple(outs) + final
 
     @staticmethod
     def backward(ctx, *douts):
@@ -196,6 +206,10 @@ class _ExtractFn(torch.autograd.Function):
                 g = g.to(torch.float32).contiguous()
                 keep.append(g)
                 b.dout[i], b.out[i] = g.data_ptr(), outs[i].data_ptr()
+            if len(douts) > 4 and douts[4] is not None:  # gradient of 'before_vae.decoder'; none: the UNet-output backward does no work
+                g = douts[4].to(torch.float32).contiguous()
+                keep.append(g)
+                b.d_unet_sample = g.data_ptr()
             b.cond_emb, b.d_cond_inputs, b.d_cond_emb = ce.data_ptr(), d_ci.data_ptr(), d_ce.data_ptr()
             b.adapter, b.lora_alpha_over_r, b.loss_scale = ctx.adapter, ctx.scaling, ctx.loss_scale
             b.packed, b.packed_dgrad = ctx.packed_ptr, slot.dgrad.data_ptr()
@@ -214,19 +228,21 @@ class _ExtractFn(torch.autograd.Function):
         ci_shape, ce_shape = ctx.cond_shapes
         g_ci = d_ci if ci_shape[0] == B else d_ci.sum(0, keepdim=True)
         g_ce = d_ce.reshape(B, *ce_shape[1:]) if ce_shape[0] == B else d_ce.sum(0, keepdim=True).reshape(1, *ce_shape[1:])
-        return (None,) * 7 + (None, g_ci, g_ce, None) + tuple(grads)
+        return (None,) * 8 + (None, g_ci, g_ce, None) + tuple(grads)
 
 
 def extract_with_grad(backbone, img, input_modal, ema_forward, timestep, grad_inputs, want_taps=False, timesteps=None, **kwargs):
-    """``AttentionFeatureExtractorBackbone._extract`` under grad: returns ``{'features': [s2, s3, s4, s5]}`` with a grad_fn."""
+    """``AttentionFeatureExtractorBackbone._extract`` under grad: returns ``{'features': [s2, s3, s4, s5]}`` (s0 variant: s0, s3, s4, s5)
+    with a grad_fn, plus ``unet_sample`` / ``decoded`` under ``return_unet_final_output`` (s0 variant)."""
     gen = backbone.feature_extractor
     ldm = gen.ldm_extractor
     if ema_forward:
         raise NotImplementedError(_UNSUPPORTED.format("ema_forward=True under grad (the teacher runs under no_grad, mtmadise.py:335-349)."))
-    if backbone.variant != "base":
-        raise NotImplementedError(_UNSUPPORTED.format("The vae_decoder_loss / s0 variant has no backward pass yet."))
-    if want_taps or kwargs.get("return_unet_final_output") or "modality_mask" in kwargs:
-        raise NotImplementedError(_UNSUPPORTED.format("Taps / return_unet_final_output / modality_mask are not available under grad."))
+    want_final = bool(kwargs.get("return_unet_final_output"))
+    if want_final and backbone.variant != "s0":
+        raise NotImplementedError("return_unet_final_output needs vae_decoder_loss=True (the reference raises on decoder_output too)")
+    if want_taps or "modality_mask" in kwargs:
+        raise NotImplementedError(_UNSUPPORTED.format("Taps / modality_mask are not available under grad."))
     if tuple(img.shape[1:]) != (3, 512, 512):
         raise ValueError(f"the training path expects [B,3,512,512] images, got {tuple(img.shape)}")
     if img.shape[0] > 8:
@@ -245,14 +261,17 @@ def extract_with_grad(backbone, img, input_modal, ema_forward, timestep, grad_in
     loss_scale = float(getattr(ldm, "train_loss_scale", None) or (1.0 if ldm.compute_dtype == "bf16" else 4096.0))
     names = [n for n, _ in engine_side]
     try:
-        outs = _ExtractFn.apply(backbone, slot, eng, adapter, scaling, loss_scale, names, img, batched["cond_inputs"], batched["cond_emb"],
-                                timesteps, *[p for _, p in engine_side])
+        outs = _ExtractFn.apply(backbone, slot, eng, adapter, scaling, loss_scale, names, want_final, img, batched["cond_inputs"],
+                                batched["cond_emb"], timesteps, *[p for _, p in engine_side])
     except Exception:
         slot.busy = False
         raise
     if not any(o.requires_grad for o in outs):  # nothing to back-propagate (e.g. only frozen inputs): release the slot now
         slot.busy = False
-    return {"features": list(outs)}
+    res = {"features": list(outs[:4])}
+    if want_final:
+        res["unet_sample"], res["decoded"] = outs[4], outs[5]
+    return res
 
 
 def _all_engine_trainables(backbone):
